@@ -26,6 +26,7 @@ Sub-records (other BASELINE.json configs, measured in the same run):
                                  all-gather of the per-rank top-k per query batch behind the C ABI
 
 `--impl reference` times the CPU path alone (the reference itself cannot be built here, see DESIGN.md).
+`--dump-outputs DIR` writes the pose the last timed step computed to DIR/pose.npy (both arms; the inputs are seeded).
 N > 1 (torchrun): the headline is independent replicas, one per GPU, no data-path collective ("scaling": "weak").
 """
 from __future__ import annotations
@@ -683,6 +684,8 @@ def run_reference(args, rank, world):
         x, sums, nf = oracle.register_aloam(*a, tree=tree)
     wall = time.perf_counter() - t0
     assert float(np.linalg.norm(x[4:] - c["t_true"])) < 0.05
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, pose=x)
     value = args.steps / wall
     sample = f"{args.steps} registrations of the config-1 frame in {wall:.2f} s"
     line = {
@@ -771,6 +774,8 @@ def run_gpu(args, rank, world, local_rank):
         ctx.sync()
         barrier()
         launches = ilsm.launch_count() - launches0
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, pose=d_pose.cpu().numpy())
         ms_steps = [a.elapsed_time(b) for a, b in evs]
         dev_ms = float(np.sum(ms_steps))
 
@@ -943,6 +948,15 @@ def emit(line):
     out.flush()
 
 
+def dump_outputs(out_dir, **arrays):
+    """--dump-outputs: what the timed path returned in its last step, one out_dir/<name>.npy per array, so that two builds
+    can be compared output for output on the same (seeded) workload.  pose = 7 doubles, q (x, y, z, w) then t, the
+    pose ilsm_register_dev leaves in place of the initial guess."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, np.float64))
+
+
 def main():
     claim_stdout()
     ap = argparse.ArgumentParser()
@@ -962,7 +976,11 @@ def main():
     ap.add_argument("--sc-keyframes", type=int, default=100_000)
     ap.add_argument("--sc-queries", type=int, default=512)
     ap.add_argument("--sc-batch", type=int, default=64)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

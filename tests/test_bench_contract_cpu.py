@@ -23,12 +23,21 @@ def _check_line(out, n_gpus):
     assert d["vs_baseline"] is None and d["higher_is_better"] is True
 
 
-def test_reference_arm_single_process(oracle_mod):
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "3", "--warmup", "1"],
-                       capture_output=True, text=True, timeout=300, cwd=ROOT)
+def test_reference_arm_single_process(oracle_mod, tmp_path):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "3", "--warmup", "1",
+                        "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=300, cwd=ROOT)
     assert r.returncode == 0, r.stderr
     assert len(r.stdout.strip().splitlines()) == 1, r.stdout  # ONE line on stdout: native prints go to stderr
     _check_line(r.stdout, 1)
+    # the dumped pose is the registration of the seeded config-1 workload
+    import numpy as np
+    import ilsm_b200
+    c = ilsm_b200.synth.config1(n_map=100_000)
+    tree = "nanoflann" if oracle_mod.lib_nanoflann() is not None else "own"
+    x, _, _ = oracle_mod.register_aloam(c["map_corner"], c["map_surf"], c["corner"], c["surf"], np.concatenate([c["q0"], c["t0"]]),
+                                        tree=tree)
+    pose = np.load(tmp_path / "pose.npy")
+    assert pose.dtype == np.float64 and np.array_equal(pose, x)
 
 
 def test_reference_arm_under_torchrun_world2(oracle_mod):

@@ -11,9 +11,9 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 @pytest.mark.gpu
-def test_bench_prints_one_json_line():
+def test_bench_prints_one_json_line(tmp_path, oracle_mod):
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "20", "--warmup", "3", "--cpu-seconds", "1",
-                        "--no-frontend", "--no-sweep", "--no-sequence", "--no-sharded"],
+                        "--no-frontend", "--no-sweep", "--no-sequence", "--no-sharded", "--dump-outputs", str(tmp_path)],
                        capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert r.returncode == 0, r.stderr[-2000:]
     lines = r.stdout.strip().splitlines()
@@ -26,3 +26,11 @@ def test_bench_prints_one_json_line():
     assert d["e2e"]["h2d_bytes_per_step"] > 0 and d["e2e"]["d2h_bytes_per_step"] > 0 and d["e2e"]["value"] > 100
     assert 0 < d["roofline"]["frac"] < 1 and d["roofline"]["bound"] == "hbm"
     assert d["cpu_baseline"]["kind"] in ("port", "reference") and d["cpu_baseline"]["value"] > 1
+    # the dumped pose of the last timed step is the oracle's registration of the same seeded workload
+    import numpy as np
+    import ilsm_b200
+    c = ilsm_b200.synth.config1(n_map=100_000)
+    x, _, _ = oracle_mod.register_aloam(c["map_corner"], c["map_surf"], c["corner"], c["surf"], np.concatenate([c["q0"], c["t0"]]))
+    pose = np.load(tmp_path / "pose.npy")
+    assert pose.dtype == np.float64 and pose.shape == (7,)
+    assert np.linalg.norm(pose[4:] - x[4:]) < 1e-4 and ilsm_b200.synth.quat_angle(pose[:4], x[:4]) < 1e-4

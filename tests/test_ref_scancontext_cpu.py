@@ -17,9 +17,20 @@ NUM_EXCLUDE_RECENT = 50  # Scancontext.h:86
 
 
 def oracle_detect(oracle_mod, db, q):
-    """detectLoopClosureID as the node runs it: the query is saved first, the tree holds all but the 50 most recent."""
+    """detectLoopClosureID as the node runs it: the query is saved first, the tree holds all but the 50 most recent.
+    The 10 ring-key candidates are the float 10-NN by brute force (the reference's nanoflann tree returns the same set on
+    the database of test_golden_cpu.py::test_oracle_ringkey_candidates_match_reference_golden; on this database the
+    stored detect_id / detect_yaw are what catches a different set), then the best candidate by distanceBtnScanContext."""
     n_search = len(db) + 1 - NUM_EXCLUDE_RECENT
-    arg, best, align, _ = oracle_mod.sc_detect_loop_reference(db[:n_search].astype(np.float64), q.astype(np.float64))
+    qd = q.astype(np.float64)
+    rk_db = np.stack([oracle_mod.sc_keys(d.astype(np.float64))[0] for d in db[:n_search]]).astype(np.float32)
+    rk_q = oracle_mod.sc_keys(qd)[0].astype(np.float32)
+    d2 = ((rk_db.astype(np.float64) - rk_q.astype(np.float64)) ** 2).sum(axis=1)
+    best, arg, align = 10000000.0, 0, 0
+    for c in np.argsort(d2, kind="stable")[:10]:
+        d, s = oracle_mod.sc_distance(qd, db[c].astype(np.float64))
+        if d < best:
+            best, arg, align = d, int(c), s
     return (arg, align) if best < 0.13 else (-1, align)
 
 

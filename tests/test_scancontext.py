@@ -16,19 +16,24 @@ def test_oracle_sc_recovers_known_shift(oracle_mod, ilsm):
 
 
 def test_oracle_sc_superset_of_reference_candidates(oracle_mod, ilsm):
-    """detectLoopClosureID scores 10 ring-key candidates (reference nanoflann); brute-force scoring of every entry is
-    a superset: same distance/shift for those ids, and a top-1 at least as good."""
-    if oracle_mod.ref() is None:
-        pytest.skip("oracle/_ref not built")
-    db = ilsm.synth.sc_database(400).astype(np.float64)
-    q, ids, _ = ilsm.synth.sc_queries(db.astype(np.float32), 6)
+    """detectLoopClosureID scores 10 ring-key candidates (reference nanoflann, the committed candidate sets of
+    tests/golden/ringkey_nanoflann.npz); brute-force scoring of every entry is a superset: same distance/shift for those
+    ids, and a top-1 at least as good."""
+    import hashlib
+    g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ringkey_nanoflann.npz"))
+    n, s0, nq, s1 = [int(v) for v in g["seeds"]]
+    db32 = ilsm.synth.sc_database(n, seed=s0)
+    q, _, _ = ilsm.synth.sc_queries(db32, nq, seed=s1)
+    assert np.array_equal(np.frombuffer(hashlib.sha256(db32.tobytes() + q.tobytes()).digest(), np.uint8), g["sha256"])
+    db = db32.astype(np.float64)
     for j in range(len(q)):
-        nn, best, align, cands = oracle_mod.sc_detect_loop_reference(db, q[j].astype(np.float64))
         dist, idx, sh = oracle_mod.sc_topk(db, q[j].astype(np.float64), len(db))
         lut = {int(i): (d, s) for d, i, s in zip(dist, idx, sh)}
-        for c in cands:
+        best = 10000000.0
+        for c in g["candidates"][j]:
             d, s = oracle_mod.sc_distance(q[j].astype(np.float64), db[int(c)])
             assert lut[int(c)] == (d, s)
+            best = min(best, d)
         assert dist[0] <= best
 
 
