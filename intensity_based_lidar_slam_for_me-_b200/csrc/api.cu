@@ -437,18 +437,10 @@ ILSM_API int ilsm_register(ilsm_ctx* ctx, ilsm_map* mc, ilsm_map* ms, const floa
   for (int i = 0; i < 3; ++i) src.v[4 + i] = t[i];
   if (o.outer_iterations < 1) return ILSM_OK;
   if ((rc = c.register_dev(&mc->m, &ms->m, d_corner, nc, d_surf, ns, stride_bytes, o, &src, nullptr))) return rc;
-  // pose (7 doubles, xq/xt are adjacent) and the report come back through pinned memory
-  unsigned char* pin = c.pinned.p;
-  ILSM_CUDA(cudaMemcpyAsync(pin, c.lm.p->xq, 7 * sizeof(double), cudaMemcpyDeviceToHost, c.stream));
-  ILSM_CUDA(cudaMemcpyAsync(pin + 64, &c.lm.p->report, sizeof(ilsm_reg_report), cudaMemcpyDeviceToHost, c.stream));
+  if ((rc = c.read_back_lm(c.stream))) return rc;
   ILSM_CUDA(cudaStreamSynchronize(c.stream));
-  const double* out = reinterpret_cast<const double*>(pin);
-  for (int i = 0; i < 4; ++i) q[i] = out[i];
-  for (int i = 0; i < 3; ++i) t[i] = out[4 + i];
-  if (report) {
-    memcpy(report, pin + 64, sizeof(*report));
-    report->passes = o.outer_iterations;
-  }
+  c.lm_result(q, t, report);
+  if (report) report->passes = o.outer_iterations;
   return ILSM_OK;
 }
 
@@ -510,22 +502,15 @@ ILSM_API int ilsm_register_frame(ilsm_ctx* ctx, ilsm_map* mc, ilsm_map* ms, cons
   if ((rc = register_frame_core(c, &mc->m, &ms->m, c.fe.raw.p, n, stride_bytes, min_range > 0.f ? min_range : 0.3f, line_res, plane_res, o,
                                 &src, nullptr, counts)))
     return rc;
-  unsigned char* pin = c.pinned.p;
-  ILSM_CUDA(cudaMemcpyAsync(pin, c.lm.p->xq, 7 * sizeof(double), cudaMemcpyDeviceToHost, c.stream));
-  ILSM_CUDA(cudaMemcpyAsync(pin + 64, &c.lm.p->report, sizeof(ilsm_reg_report), cudaMemcpyDeviceToHost, c.stream));
-  ILSM_CUDA(cudaMemcpyAsync(pin + 64 + sizeof(ilsm_reg_report), c.rf_stack_n.p, 2 * sizeof(int), cudaMemcpyDeviceToHost, c.stream));
+  int* sn = reinterpret_cast<int*>(c.pinned.p + Ctx::kPinSite);  // the down-sampled stack sizes
+  if ((rc = c.read_back_lm(c.stream))) return rc;
+  ILSM_CUDA(cudaMemcpyAsync(sn, c.rf_stack_n.p, 2 * sizeof(int), cudaMemcpyDeviceToHost, c.stream));
   ILSM_CUDA(cudaStreamSynchronize(c.stream));
   if (o.outer_iterations >= 1) {
-    const double* out = reinterpret_cast<const double*>(pin);
-    for (int i = 0; i < 4; ++i) q[i] = out[i];
-    for (int i = 0; i < 3; ++i) t[i] = out[4 + i];
-    if (report) {
-      memcpy(report, pin + 64, sizeof(*report));
-      report->passes = o.outer_iterations;
-    }
+    c.lm_result(q, t, report);
+    if (report) report->passes = o.outer_iterations;
   }
   if (sizes_out) {
-    const int* sn = reinterpret_cast<const int*>(pin + 64 + sizeof(ilsm_reg_report));
     sizes_out[0] = counts[2], sizes_out[1] = counts[4], sizes_out[2] = sn[0], sizes_out[3] = sn[1];
   }
   return ILSM_OK;
@@ -620,17 +605,10 @@ ILSM_API int ilsm_odometry(ilsm_ctx* ctx, ilsm_map* last_corner, ilsm_map* last_
     return ILSM_OK;
   }
   if ((rc = c.odometry_dev(&last_corner->m, &last_surf->m, d_sharp, nsh, d_flat, nfl, stride_bytes, o))) return rc;
-  unsigned char* pin = c.pinned.p;
-  ILSM_CUDA(cudaMemcpyAsync(pin, c.lm.p->xq, 7 * sizeof(double), cudaMemcpyDeviceToHost, c.stream));
-  ILSM_CUDA(cudaMemcpyAsync(pin + 64, &c.lm.p->report, sizeof(ilsm_reg_report), cudaMemcpyDeviceToHost, c.stream));
+  if ((rc = c.read_back_lm(c.stream))) return rc;
   ILSM_CUDA(cudaStreamSynchronize(c.stream));
-  const double* out = reinterpret_cast<const double*>(pin);
-  for (int i = 0; i < 4; ++i) q[i] = out[i];
-  for (int i = 0; i < 3; ++i) t[i] = out[4 + i];
-  if (report) {
-    memcpy(report, pin + 64, sizeof(*report));
-    report->passes = o.outer_iterations;
-  }
+  c.lm_result(q, t, report);
+  if (report) report->passes = o.outer_iterations;
   return ILSM_OK;
 }
 
@@ -1062,14 +1040,11 @@ ILSM_API int ilsm_solve(ilsm_ctx* ctx, double q[4], double t[3], int max_num_ite
   count_launches(1);
   int rc;
   if ((rc = c.solve_launch(max_num_iterations, huber_a, 0))) return rc;
-  unsigned char* pin = c.pinned.p;
-  ILSM_CUDA(cudaMemcpyAsync(pin, c.lm.p->xq, 7 * sizeof(double), cudaMemcpyDeviceToHost, c.stream));
-  ILSM_CUDA(cudaMemcpyAsync(pin + 64, &c.lm.p->report, sizeof(ilsm_reg_report), cudaMemcpyDeviceToHost, c.stream));
+  if ((rc = c.read_back_lm(c.stream))) return rc;
   ILSM_CUDA(cudaStreamSynchronize(c.stream));
-  const double* out = reinterpret_cast<const double*>(pin);
-  for (int i = 0; i < 4; ++i) q[i] = out[i];
-  for (int i = 0; i < 3; ++i) t[i] = out[4 + i];
-  if (summary) memcpy(summary, pin + 64 + offsetof(ilsm_reg_report, pass), sizeof(*summary));
+  ilsm_reg_report rep;
+  c.lm_result(q, t, &rep);
+  if (summary) *summary = rep.pass[0];
   return ILSM_OK;
 }
 

@@ -19,8 +19,6 @@
 
 namespace ilsm {
 
-constexpr size_t kLmHostBytes = offsetof(LmState, report) + sizeof(ilsm_reg_report);  // what a frame reads back of the LM state
-
 // grid (8, n_valid, 2): z = cloud kind
 __global__ void cube_gather_kernel(const float4* __restrict__ slabs_c, const float4* __restrict__ slabs_s, int cap,
                                    const __grid_constant__ GatherItems items, float4* __restrict__ out_c, float4* __restrict__ out_s) {
@@ -412,10 +410,8 @@ int cubemap_frame_enqueue(CubeMapH& m, const float* d_c, int nc, const float* d_
       return rc;
   }
   // pose in
-  double pose[7] = {qw.x, qw.y, qw.z, qw.w, tw[0], tw[1], tw[2]};
-  double* pin_pose = reinterpret_cast<double*>(c.pinned.p + 1024);
-  for (int i = 0; i < 7; ++i) pin_pose[i] = pose[i];
-  ILSM_CUDA(cudaMemcpyAsync(c.lm.p->xq, pin_pose, 7 * sizeof(double), cudaMemcpyHostToDevice, c.stream));
+  const double qw4[4] = {qw.x, qw.y, qw.z, qw.w};
+  if ((rc = c.upload_pose(qw4, tw, c.stream))) return rc;
   const bool optimise = n_mc > o.min_corner_map && n_ms > o.min_surf_map;  // laserMapping.cpp:624
   if (optimise) {
     if ((rc = build_pair_dev(&m.map_c, reinterpret_cast<const float*>(m.from_c.p), n_mc, &m.map_s, reinterpret_cast<const float*>(m.from_s.p),
@@ -435,11 +431,8 @@ int cubemap_frame_enqueue(CubeMapH& m, const float* d_c, int nc, const float* d_
   // pose, report and stack sizes come back first; the insertion with the optimised pose (still on the device) and the
   // per-cube VoxelGrid of the valid cubes follow -- on the side stream when the caller defers them (full-loop
   // pipeline: they overlap the next frame's upload and front end, wait_tail() joins them)
-  unsigned char* pin = c.pinned.p;
   int* pin_i = m.pin.p + kCNum + 2048;
-  // pose and report in ONE copy: the LM state up to the end of the report is contiguous (xq first)
-  static_assert(offsetof(LmState, xq) == 0 && kLmHostBytes <= 1024, "the pose-in staging area starts at pinned + 1024");
-  ILSM_CUDA(cudaMemcpyAsync(pin, c.lm.p, kLmHostBytes, cudaMemcpyDeviceToHost, c.stream));
+  if ((rc = c.read_back_lm(c.stream))) return rc;
   ILSM_CUDA(cudaMemcpyAsync(pin_i + 1, m.cur_stack_n(), 2 * sizeof(int), cudaMemcpyDeviceToHost, c.stream));
   cudaStream_t ts = defer_tail ? c.aux : c.stream;
   if (defer_tail) {
@@ -465,20 +458,14 @@ int cubemap_frame_collect(CubeMapH& m, double q_w[4], double t_w[3], ilsm_reg_re
   const double* t_wodom = m.pend.t_wodom;
   const bool optimise = m.pend.optimise, defer_tail = m.pend.defer_tail;
   const int n_mc = m.pend.n_mc, n_ms = m.pend.n_ms;
-  unsigned char* pin = c.pinned.p;
   int* pin_i = m.pin.p + kCNum + 2048;
   double r[3];
   ILSM_CUDA(cudaStreamSynchronize(c.stream));
   pin_i[0] = m.tail_flags;  // capacity flags: of this frame when synchronous, up to the previous frame when deferred
   if (!defer_tail) pin_i[0] |= m.adopt_counts();
   m.tail_flags = 0;
-  const double* out = reinterpret_cast<const double*>(pin);
-  for (int i = 0; i < 4; ++i) q_w[i] = out[i];
-  for (int i = 0; i < 3; ++i) t_w[i] = out[4 + i];
-  if (report && optimise) {
-    memcpy(report, pin + offsetof(LmState, report), sizeof(*report));
-    report->passes = m.pend.outer;
-  }
+  c.lm_result(q_w, t_w, optimise ? report : nullptr);
+  if (report && optimise) report->passes = m.pend.outer;
   // transformUpdate (laserMapping.cpp:145-149)
   const QuatH qwf{q_w[0], q_w[1], q_w[2], q_w[3]};
   const double n2 = qo.x * qo.x + qo.y * qo.y + qo.z * qo.z + qo.w * qo.w;

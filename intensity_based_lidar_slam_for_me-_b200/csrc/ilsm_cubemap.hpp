@@ -58,8 +58,8 @@ struct CubeMapH {
   // [2 kCNum, 4 kCNum) how many leading points of the cube are the output of its last pass (merge precondition)
   DevBuf<int> clean;
   bool vg_merge = true;
-  // stacks produced outside (staged full-loop pipeline: two sets, alternating by frame, written on the odometry stage's
-  // side stream): when set, the frame being enqueued -- solve and deferred insertion -- reads these instead of stack_*
+  // stacks produced outside (full loop: two sets, alternating by frame, written on the odometry stage's side stream):
+  // when set, the frame being enqueued -- solve and deferred insertion -- reads these instead of stack_*
   const float4 *ext_c = nullptr, *ext_s = nullptr;
   const int* ext_n = nullptr;
   const float4* cur_stack_c() const { return ext_c ? ext_c : stack_c.p; }

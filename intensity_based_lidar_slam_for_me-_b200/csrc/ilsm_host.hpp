@@ -2,7 +2,9 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <limits.h>
+#include <stddef.h>
 #include <stdint.h>
+#include <string.h>
 
 #include <mutex>
 #include <string>
@@ -109,6 +111,7 @@ struct LmState {
   ilsm_reg_report report;
   long long dbg[64];  // clock64() phase stamps written when ILSM_DEBUG_TIMING is compiled in (profiling aid)
 };
+constexpr size_t kLmHostBytes = offsetof(LmState, report) + sizeof(ilsm_reg_report);  // what a solve reads back of the LM state
 
 // Where the association kernel of the FIRST pass takes the pose from, and where the solve kernel of the LAST pass
 // leaves the result: folding these into the two kernels removes the 1-warp pose upload / download launches.
@@ -244,6 +247,29 @@ struct Ctx {
 
   int init(int dev);
   void release();
+  // LM pose staging in `pinned`: the LM state prefix (pose and report, xq first) comes back to offset 0 in one copy, a
+  // pose goes up from kPinPoseIn.  [kPinSite, kPinPoseIn) is left to a call site's own read-back in the same synchronise.
+  static constexpr size_t kPinSite = 1024, kPinPoseIn = 2048;
+  static_assert(offsetof(LmState, xq) == 0 && offsetof(LmState, xt) == 4 * sizeof(double) && kLmHostBytes <= kPinSite,
+                "the LM read-back overlaps the call sites' area");
+  int upload_pose(const double q[4], const double t[3], cudaStream_t s) {  // -> lm.p->xq, xt
+    double* p = reinterpret_cast<double*>(pinned.p + kPinPoseIn);
+    for (int i = 0; i < 4; ++i) p[i] = q[i];
+    for (int i = 0; i < 3; ++i) p[4 + i] = t[i];
+    ILSM_CUDA(cudaMemcpyAsync(lm.p->xq, p, 7 * sizeof(double), cudaMemcpyHostToDevice, s));
+    return ILSM_OK;
+  }
+  int read_back_lm(cudaStream_t s) {
+    ILSM_CUDA(cudaMemcpyAsync(pinned.p, lm.p, kLmHostBytes, cudaMemcpyDeviceToHost, s));
+    return ILSM_OK;
+  }
+  // after the caller has synchronised with read_back_lm's stream: the accepted pose and the report
+  void lm_result(double q[4], double t[3], ilsm_reg_report* report) const {
+    const double* x = reinterpret_cast<const double*>(pinned.p);
+    for (int i = 0; i < 4; ++i) q[i] = x[i];
+    for (int i = 0; i < 3; ++i) t[i] = x[4 + i];
+    if (report) memcpy(report, pinned.p + offsetof(LmState, report), sizeof(*report));
+  }
   bool async_build = false;  // ilsm_set_async: host-pointer map builds return without synchronising
   int associate_dev(Map* mc, Map* ms, const float* d_corner, int nc, const float* d_surf, int ns, int stride_bytes,
                     const ilsm_reg_opts& o, bool want_knn, const PoseSrc* src = nullptr);

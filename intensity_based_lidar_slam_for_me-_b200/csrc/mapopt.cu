@@ -216,10 +216,8 @@ int mapopt_frame_core(ilsm_mapopt* mo, const float* frame_xyz, int n, int stride
     if (rc) return rc;
   }
   // association (5-NN in the ground map, plane fit) + ceres::Solve (planes only, one pass, 10 iterations)
-  double* pin_pose = reinterpret_cast<double*>(c.pinned.p + 2048);
-  pin_pose[0] = qw.x, pin_pose[1] = qw.y, pin_pose[2] = qw.z, pin_pose[3] = qw.w;
-  for (int i = 0; i < 3; ++i) pin_pose[4 + i] = tw[i];
-  ILSM_CUDA(cudaMemcpyAsync(c.lm.p->xq, pin_pose, 7 * sizeof(double), cudaMemcpyHostToDevice, s));
+  const double qw4[4] = {qw.x, qw.y, qw.z, qw.w};
+  if ((rc = c.upload_pose(qw4, tw, s))) return rc;
   ilsm_reg_opts o;
   ilsm_reg_opts_default(&o);
   o.outer_iterations = 1, o.max_num_iterations = 10, o.min_corner_map = 0, o.min_surf_map = 0;
@@ -227,15 +225,14 @@ int mapopt_frame_core(ilsm_mapopt* mo, const float* frame_xyz, int n, int stride
   rc = c.register_dev(&m.empty, &m.map, nullptr, 0, reinterpret_cast<const float*>(m.stack.p), n_all, 16, o);
   c.d_stack_counts = nullptr;
   if (rc) return rc;
-  unsigned char* pin = c.pinned.p;
-  ILSM_CUDA(cudaMemcpyAsync(pin, c.lm.p->xq, 7 * sizeof(double), cudaMemcpyDeviceToHost, s));
-  ILSM_CUDA(cudaMemcpyAsync(pin + 64, &c.lm.p->report, sizeof(ilsm_reg_report), cudaMemcpyDeviceToHost, s));
-  ILSM_CUDA(cudaMemcpyAsync(pin + 1024, m.counts.p, 2 * sizeof(int), cudaMemcpyDeviceToHost, s));
+  int* pin_counts = reinterpret_cast<int*>(c.pinned.p + Ctx::kPinSite);
+  if ((rc = c.read_back_lm(s))) return rc;
+  ILSM_CUDA(cudaMemcpyAsync(pin_counts, m.counts.p, 2 * sizeof(int), cudaMemcpyDeviceToHost, s));
   ILSM_CUDA(cudaStreamSynchronize(s));
-  const double* out = reinterpret_cast<const double*>(pin);
+  double out[7];
   ilsm_reg_report rep;
-  memcpy(&rep, pin + 64, sizeof(rep));
-  const int n_stack = reinterpret_cast<const int*>(pin + 1024)[1];
+  c.lm_result(out, out + 4, &rep);
+  const int n_stack = pin_counts[1];
   const bool converged = rep.pass[0].termination == ILSM_CONVERGENCE;  // mapOptimization.cpp:448
   QuatH qk = qw;       // cur_keyframe.q_map_cur_k_ / t_map_cur_k_: the predicted pose unless the solve converged
   double tk[3] = {tw[0], tw[1], tw[2]};

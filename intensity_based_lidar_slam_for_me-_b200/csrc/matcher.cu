@@ -199,19 +199,12 @@ ILSM_API int ilsm_align_points(ilsm_ctx* ctx, const float* src_xyz, const float*
     ILSM_CUDA(launch_pdl(align_factors_kernel, dim3((n + 255) / 256), dim3(256), 0, c.stream, d_src, d_dst, n, stride_bytes / 4, f.type.p, f.p.p, f.a.p, f.b.p));
     count_launches(1);
   }
-  double* pin_pose = reinterpret_cast<double*>(c.pinned.p + 2048);
-  for (int i = 0; i < 4; ++i) pin_pose[i] = q[i];
-  for (int i = 0; i < 3; ++i) pin_pose[4 + i] = t[i];
-  ILSM_CUDA(cudaMemcpyAsync(c.lm.p->xq, pin_pose, 7 * sizeof(double), cudaMemcpyHostToDevice, c.stream));
-  if ((rc = c.solve_launch(max_num_iterations, huber_a, 0))) return rc;
-  unsigned char* pin = c.pinned.p;
-  ILSM_CUDA(cudaMemcpyAsync(pin, c.lm.p->xq, 7 * sizeof(double), cudaMemcpyDeviceToHost, c.stream));
-  ILSM_CUDA(cudaMemcpyAsync(pin + 64, &c.lm.p->report, sizeof(ilsm_reg_report), cudaMemcpyDeviceToHost, c.stream));
+  if ((rc = c.upload_pose(q, t, c.stream)) || (rc = c.solve_launch(max_num_iterations, huber_a, 0)) || (rc = c.read_back_lm(c.stream)))
+    return rc;
   ILSM_CUDA(cudaStreamSynchronize(c.stream));
-  const double* out = reinterpret_cast<const double*>(pin);
-  for (int i = 0; i < 4; ++i) q[i] = out[i];
-  for (int i = 0; i < 3; ++i) t[i] = out[4 + i];
-  if (summary) memcpy(summary, pin + 64 + offsetof(ilsm_reg_report, pass), sizeof(*summary));
+  ilsm_reg_report rep;
+  c.lm_result(q, t, &rep);
+  if (summary) *summary = rep.pass[0];
   return ILSM_OK;
 }
 

@@ -144,33 +144,37 @@ def test_pipeline_survives_degenerate_frames(ctx, ilsm, mapping):
 def test_pipelined_mapping_stage_gives_the_same_poses(ctx, ilsm):
     """ilsm_slam_create_async: laserMapping as its own stage on a second context (frame k's mapping overlaps frame k+1's
     front end + odometry).  Odometry poses frame for frame and mapped poses one call later are bit-identical to the
-    synchronous loop; misuse of the two handle kinds is rejected."""
+    synchronous loop -- also when some frames skip the odometry solve (use_aloam = 0); misuse of the two handle kinds is
+    rejected."""
     import os, sys
     sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tools"))
     from sequence_bench import corridor_sequence
     clouds, _ = corridor_sequence(ilsm.synth, 14, 0x5EED0100, 40.0)
-    a = ilsm.Slam(ctx, 0.4, 0.8, 0.3, 4096)
-    b = ilsm.Slam(ctx, 0.4, 0.8, 0.3, 4096, pipelined=True)
-    sync = [a.frame(c) for c in clouds]
-    mapped = []
-    for k, c in enumerate(clouds):
-        qo, to, qm, tm, st = b.frame_async(c)
-        assert np.array_equal(qo, sync[k][0]) and np.array_equal(to, sync[k][1])
-        assert (qm is None) == (k == 0)
-        if qm is not None:
-            mapped.append((qm, tm, st.mapping.pass_[1].num_plane_factors))
-    qm, tm, st = b.flush()
-    mapped.append((qm, tm, st.mapping.pass_[1].num_plane_factors))
-    assert b.flush()[0] is None
-    assert len(mapped) == len(clouds)
-    for k in range(len(clouds)):
-        assert np.array_equal(mapped[k][0], sync[k][2]) and np.array_equal(mapped[k][1], sync[k][3]), k
-        assert mapped[k][2] == sync[k][4].mapping.pass_[1].num_plane_factors
-    with pytest.raises(ilsm.IlsmError):
-        b.frame(clouds[0])
-    with pytest.raises(ilsm.IlsmError):
-        a.frame_async(clouds[0])
-    a.close(), b.close()
+    for use in (None, [k % 5 != 3 for k in range(len(clouds))]):
+        ua = [True if use is None else use[k] for k in range(len(clouds))]
+        a = ilsm.Slam(ctx, 0.4, 0.8, 0.3, 4096)
+        b = ilsm.Slam(ctx, 0.4, 0.8, 0.3, 4096, pipelined=True)
+        sync = [a.frame(c, use_aloam=ua[k]) for k, c in enumerate(clouds)]
+        mapped = []
+        for k, c in enumerate(clouds):
+            qo, to, qm, tm, st = b.frame_async(c, use_aloam=ua[k])
+            assert np.array_equal(qo, sync[k][0]) and np.array_equal(to, sync[k][1])
+            assert st.ran_odometry == sync[k][4].ran_odometry
+            assert (qm is None) == (k == 0)
+            if qm is not None:
+                mapped.append((qm, tm, st.mapping.pass_[1].num_plane_factors))
+        qm, tm, st = b.flush()
+        mapped.append((qm, tm, st.mapping.pass_[1].num_plane_factors))
+        assert b.flush()[0] is None
+        assert len(mapped) == len(clouds)
+        for k in range(len(clouds)):
+            assert np.array_equal(mapped[k][0], sync[k][2]) and np.array_equal(mapped[k][1], sync[k][3]), k
+            assert mapped[k][2] == sync[k][4].mapping.pass_[1].num_plane_factors
+        with pytest.raises(ilsm.IlsmError):
+            b.frame(clouds[0])
+        with pytest.raises(ilsm.IlsmError):
+            a.frame_async(clouds[0])
+        a.close(), b.close()
 
 
 def test_cube_merge_voxelgrid_is_bit_identical_to_the_general_pass(ctx, ilsm, monkeypatch):
@@ -267,12 +271,12 @@ def test_three_stage_loop_destroyed_with_frames_in_flight(ctx, ilsm):
     b.close()
 
 
-@pytest.mark.parametrize("pipelined", [False, True])
-def test_feature_clouds_above_16384_points(ctx, oracle_mod, ilsm, pipelined):
+@pytest.mark.parametrize("mode", ["synchronous", "pipelined", "staged"])
+def test_feature_clouds_above_16384_points(ctx, oracle_mod, ilsm, mode):
     """A 64-ring sensor whose beams all fall inside the reference's +-22.5 degree ring formula keeps every return
     (scanRegistration.cpp:308-316, 570-589): ~17.7 k less-flat points per frame in the open scene -- more than one block's
     VoxelGrid sorts.  The full loop routes such clouds through the tiled multi-block VoxelGrid and must still match the
-    chained oracle, in the synchronous loop and with the mapping stage pipelined."""
+    chained oracle, in the synchronous loop, with the mapping stage pipelined and as three stages."""
     S = ilsm.synth
     scene = S.Scene()
     q0, t0 = S.default_pose()
@@ -281,26 +285,27 @@ def test_feature_clouds_above_16384_points(ctx, oracle_mod, ilsm, pipelined):
         q = S.quat_mul(q0, S.quat_from_rotvec([0.0, 0.0, 0.01 * k]))
         t = np.asarray(t0) + [0.15 * k, 0.02 * k, 0.0]
         frames.append(S.make_frame(scene, q, t, seed=0x5EED0700 + k, fov_deg=22.0)[0])
-    slam = ilsm.Slam(ctx, 0.4, 0.8, 0.3, 16384, pipelined=pipelined)
+    slam = ilsm.Slam(ctx, 0.4, 0.8, 0.3, 16384, pipelined=mode == "pipelined", staged=mode == "staged")
     oslam = oracle_mod.Slam(0.4, 0.8, 0.3)
-    want, got = [], []
-    for k, cloud in enumerate(frames):
-        wodom, wmap, info = oslam.frame(cloud)
-        want.append(wmap)
-        if pipelined:
-            r = slam.frame_async(cloud)
-            st = r[4]
-            if r[2] is not None:
-                got.append((r[2], r[3]))
-        else:
-            gqo, gto, gqm, gtm, st = slam.frame(cloud)
-            got.append((gqm, gtm))
+    want = [oslam.frame(cloud) for cloud in frames]
+    if mode == "staged":
+        _, mapped, st = _run_staged(slam, frames)
+        got, stats = [mapped[k][:2] for k in range(len(frames))], [st[k] for k in range(len(frames))]
+    elif mode == "pipelined":
+        got, stats = [], []
+        for cloud in frames:
+            qo, to, qm, tm, st = slam.frame_async(cloud)
+            stats.append(st)
+            if qm is not None:
+                got.append((qm, tm))
+        got.append(slam.flush()[:2])
+    else:
+        runs = [slam.frame(cloud) for cloud in frames]
+        got, stats = [r[2:4] for r in runs], [r[4] for r in runs]
+    assert len(got) == len(want)
+    for k, ((gq, gt), (_, w, info), st) in enumerate(zip(got, want, stats)):
         assert st.n_less_flat == len(info["features"]["less_flat"]) and st.n_less_flat > 16384, (k, st.n_less_flat)
         assert st.n_less_sharp == len(info["features"]["less_sharp_idx"])
-    if pipelined:
-        got.append(slam.flush()[:2])
-    assert len(got) == len(want)
-    for k, ((gq, gt), w) in enumerate(zip(got, want)):
         assert np.linalg.norm(gt - w[4:]) < 1e-4 and S.quat_angle(gq, w[:4]) < 1e-4, k
     slam.close()
 
