@@ -199,6 +199,7 @@ def load_library(path: str | None = None):
         "ilsm_align_points": (i32, [vp, vp, vp, i32, i32, vp, vp, i32, f64, C.POINTER(SolveSummary)]),
         "ilsm_associate_dev": (i32, [vp, vp, vp, vp, i32, vp, i32, i32, vp, C.POINTER(RegOpts)]),
         "ilsm_launch_count": (C.c_longlong, []),
+        "ilsm_debug_live_bytes": (None, [C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]),
         "ilsm_eval_normal_eq": (i32, [vp, vp, vp, f64, C.POINTER(f64), vp, vp]),
         "ilsm_eval_normal_eq_dev": (i32, [vp, vp, f64, vp]),
         "ilsm_solve_dev": (i32, [vp, vp, i32, f64]),
@@ -213,6 +214,13 @@ def load_library(path: str | None = None):
 
 def launch_count() -> int:
     return int(load_library().ilsm_launch_count())
+
+
+def live_bytes() -> tuple[int, int]:
+    """(device, pinned) bytes the library's buffers hold, all handles of the process together.  Makes no CUDA call."""
+    dev, pin = C.c_longlong(0), C.c_longlong(0)
+    load_library().ilsm_debug_live_bytes(C.byref(dev), C.byref(pin))
+    return dev.value, pin.value
 
 
 def _check(rc):

@@ -23,6 +23,7 @@ int fail_cuda(cudaError_t e, const char* where) {
 }
 static std::atomic<long long> g_launches{0};
 void count_launches(int k) { g_launches.fetch_add(k, std::memory_order_relaxed); }
+std::atomic<long long> g_live_bytes[2] = {{0}, {0}};
 
 int check_launch(const char* where) {
   cudaError_t e = cudaGetLastError();
@@ -99,37 +100,22 @@ int Ctx::init(int dev) {
   return ILSM_OK;
 }
 
-void Ctx::release() {
-  if (fe_graph_exec) cudaGraphExecDestroy(fe_graph_exec), fe_graph_exec = nullptr;
+Ctx::~Ctx() {
+  if (fe_graph_exec) cudaGraphExecDestroy(fe_graph_exec);
   if (stream) cudaStreamSynchronize(stream);
-  fe.vg_hash.release(), fe.vg_keys.release(), fe.vg_state.release(), fe.vg_chunk.release(), fe.chunk_hist.release(), fe.chunk_base.release(), fe.scanid.release(), fe.picked.release(), fe.ori.release(), fe.curv.release(), fe.stats.release();
-  fe.src_index.release(), fe.label.release(), fe.sort_ind.release(), fe.ring_sharp.release(), fe.ring_lsharp.release();
-  fe.ring_flat.release(), fe.sharp.release(), fe.lsharp.release(), fe.flat.release(), fe.counts.release();
-  fe.cloud.release(), fe.ring_pts.release(), fe.ring_out.release(), fe.lflat.release(), fe.vox_packed.release();
-  fe.pc2.release(), fe.raw.release(), fe.img.release(), fe.track.release(), fe.vox_out.release(), fe.vox_n.release();
-  lm.release(), partials.release(), stack_raw.release(), out_idx.release(), out_d2.release(), pinned.release();
-  rf_lsharp.release(), rf_stack_c.release(), rf_stack_s.release(), rf_stack_n.release();
-  if (qbin) qbin->release(), delete qbin, qbin = nullptr;
-  qwork.release();
-  fac.type.release(), fac.p.release(), fac.a.release(), fac.b.release(), fac.knn_idx.release(), fac.knn_d2.release();
-  if (aux) cudaStreamSynchronize(aux), cudaStreamDestroy(aux);
+  if (aux) cudaStreamSynchronize(aux);
+  delete qbin;
   if (ev_fork) cudaEventDestroy(ev_fork);
   if (ev_join) cudaEventDestroy(ev_join);
+  if (aux) cudaStreamDestroy(aux);
   if (stream) cudaStreamDestroy(stream);
-  stream = nullptr, aux = nullptr, ev_fork = nullptr, ev_join = nullptr;
 }
 
-void Map::release() {
+Map::~Map() {
   if (stream) cudaStreamSynchronize(stream);
   if (ready) cudaEventDestroy(ready);
   if (ctx_done) cudaEventDestroy(ctx_done);
   if (stream) cudaStreamDestroy(stream);
-  stream = nullptr, ready = nullptr, ctx_done = nullptr;
-  cells.release(), sorted.release(), orig.release(), slot_of.release(), rank_of.release(), counters.release(), occ.release();
-  gen = 0, cur = 0, table_cap = 0, occ_cap = 0, clean_size[0] = clean_size[1] = 0, filled_n[0] = filled_n[1] = 0;
-  bbox.release(), raw.release();
-  vox_table.release(), ins_new.release(), ins_out.release(), ins_slot_new.release(), ins_slot_old.release();
-  ins_keep.release(), ins_pos.release(), ins_bsum.release();
 }
 
 static bool valid_stride(int s) { return s >= 12 && (s % 4) == 0; }
@@ -179,7 +165,6 @@ ILSM_API int ilsm_create(int device, ilsm_ctx** out) {
   if (!h) return fail(ILSM_ERR_OUT_OF_MEMORY, "host allocation failed");
   int rc = h->c.init(device);
   if (rc) {
-    h->c.release();
     delete h;
     return rc;
   }
@@ -190,7 +175,6 @@ ILSM_API int ilsm_create(int device, ilsm_ctx** out) {
 ILSM_API void ilsm_destroy(ilsm_ctx* ctx) {
   if (!ctx) return;
   cudaSetDevice(ctx->c.device);
-  ctx->c.release();
   delete ctx;
 }
 
@@ -211,6 +195,13 @@ ILSM_API int ilsm_debug_stamps(ilsm_ctx* ctx, long long* out64) {
   return ILSM_OK;
 }
 
+// testing aid (not in include/ilsm.h): bytes held by the device and the pinned buffers of every handle of the process;
+// makes no CUDA call
+ILSM_API void ilsm_debug_live_bytes(long long* device, long long* pinned) {
+  if (device) *device = g_live_bytes[0].load();
+  if (pinned) *pinned = g_live_bytes[1].load();
+}
+
 ILSM_API int ilsm_set_async(ilsm_ctx* ctx, int on) {
   if (!ctx) return fail(ILSM_ERR_INVALID_ARG, "null ctx");
   std::lock_guard<std::mutex> lk(ctx->c.mu);
@@ -227,7 +218,6 @@ ILSM_API int ilsm_map_create(ilsm_ctx* ctx, ilsm_map** out) {
     cudaSetDevice(ctx->c.device);
     int rc = m->m.init(&ctx->c);
     if (rc) {
-      m->m.release();
       delete m;
       return rc;
     }
@@ -238,12 +228,9 @@ ILSM_API int ilsm_map_create(ilsm_ctx* ctx, ilsm_map** out) {
 
 ILSM_API void ilsm_map_destroy(ilsm_map* map) {
   if (!map) return;
-  {
-    std::lock_guard<std::mutex> lk(map->m.ctx->mu);
-    cudaSetDevice(map->m.ctx->device);
-    cudaStreamSynchronize(map->m.ctx->stream);
-    map->m.release();
-  }
+  std::lock_guard<std::mutex> lk(map->m.ctx->mu);
+  cudaSetDevice(map->m.ctx->device);
+  cudaStreamSynchronize(map->m.ctx->stream);
   delete map;
 }
 
@@ -852,18 +839,10 @@ ILSM_API int ilsm_sc_create(ilsm_ctx* ctx, ilsm_sc** out) {
 
 ILSM_API void ilsm_sc_destroy(ilsm_sc* sc) {
   if (!sc) return;
-  {
-    std::lock_guard<std::mutex> lk(sc->d.ctx->mu);
-    cudaSetDevice(sc->d.ctx->device);
-    cudaStreamSynchronize(sc->d.ctx->stream);
-    ScDb& d = sc->d;
-    d.db.release(), d.bins.release(), d.query.release(), d.out_dist.release(), d.part_d.release(), d.part_id.release(), d.part_sh.release();
-    d.out_id.release(), d.out_shift.release(), d.stage.release();
-    d.ringkey.release(), d.rk_part.release(), d.cand_out.release(), d.pk_local.release(), d.pk_all.release(), d.pk_out.release();
-    d.qbatch.release();
-    d.pf_query.release(), d.pf_dist.release(), d.pf_thr.release(), d.pf_part.release(), d.pf_list.release(), d.pf_list_n.release();
-    sc_nccl_release(d);
-  }
+  std::lock_guard<std::mutex> lk(sc->d.ctx->mu);
+  cudaSetDevice(sc->d.ctx->device);
+  cudaStreamSynchronize(sc->d.ctx->stream);
+  sc_nccl_release(sc->d);
   delete sc;
 }
 

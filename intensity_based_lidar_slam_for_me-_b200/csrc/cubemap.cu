@@ -209,8 +209,8 @@ int CubeMapH::init(Ctx* c, float lres, float pres, int cube_cap) {
       (rc = pin_counts.reserve(2 * kCNum + 16)))
     return rc;
   // the two count arrays and the error word sit back to back (cnt_all): the host mirror is refreshed with ONE copy per frame;
-  // cnt_c / cnt_s / err are views into it (cap 0: not owned)
-  cnt_c.p = cnt_all.p, cnt_s.p = cnt_all.p + kCNum, err.p = cnt_all.p + 2 * kCNum;
+  // cnt_c / cnt_s / err are views into it
+  cnt_c = cnt_all.p, cnt_s = cnt_all.p + kCNum, err = cnt_all.p + 2 * kCNum;
   ILSM_CUDA(cudaEventCreateWithFlags(&ev_tail, cudaEventDisableTiming));
   slab_of.resize(kCNum);
   for (int i = 0; i < kCNum; ++i) slab_of[i] = i;
@@ -226,17 +226,10 @@ int CubeMapH::init(Ctx* c, float lres, float pres, int cube_cap) {
   return ILSM_OK;
 }
 
-void CubeMapH::release() {
+CubeMapH::~CubeMapH() {
   if (ctx && ctx->stream) cudaStreamSynchronize(ctx->stream);
   if (ctx && ctx->aux) cudaStreamSynchronize(ctx->aux);
   if (ev_tail) cudaEventDestroy(ev_tail);
-  ev_tail = nullptr;
-  pin_counts.release();
-  map_c.release(), map_s.release();
-  slabs_c.release(), slabs_s.release(), from_c.release(), from_s.release(), stack_c.release(), stack_s.release();
-  cnt_c.p = cnt_s.p = err.p = nullptr;  // views into cnt_all
-  scratch.release(), hscratch.release(), world_tmp.release(), cnt_all.release(), slab_of_d.release(), stack_n.release(), clean.release();
-  zero_list.release(), raw.release(), pin.release();
 }
 
 static int cube_coord_h(double v, int cen) {
@@ -293,7 +286,7 @@ int CubeMapH::roll(const double t[3]) {
     const int n = (int)recycled.size() < kCNum ? (int)recycled.size() : kCNum;
     for (int i = 0; i < n; ++i) p[i] = recycled[i];
     ILSM_CUDA(cudaMemcpyAsync(zero_list.p, p, n * sizeof(int), cudaMemcpyHostToDevice, s));
-    ILSM_CUDA(launch_pdl(cube_zero_counts_kernel, dim3((n + 255) / 256), dim3(256), 0, s, cnt_c.p, cnt_s.p, clean.p + 2 * kCNum, zero_list.p, n));
+    ILSM_CUDA(launch_pdl(cube_zero_counts_kernel, dim3((n + 255) / 256), dim3(256), 0, s, cnt_c, cnt_s, clean.p + 2 * kCNum, zero_list.p, n));
     ILSM_CUDA(cudaMemcpyAsync(slab_of_d.p, slab_of.data(), kCNum * sizeof(int), cudaMemcpyHostToDevice, s));
     ILSM_CUDA(cudaStreamSynchronize(s));
     count_launches(1);
@@ -326,7 +319,7 @@ int CubeMapH::gather(int* n_mc, int* n_ms) {
 
 int CubeMapH::insert(const int* d_counts, int nc_host, int ns_host, int world_frame, cudaStream_t s) {
   if (!s) s = ctx->stream;
-  ILSM_CUDA(launch_pdl(cube_insert_kernel, dim3(2), dim3(1024), kVoxelBlockMax * sizeof(u64), s, cur_stack_c(), cur_stack_s(), d_counts, nc_host, ns_host, ctx->lm.p, world_frame, cenW, cenH, cenD, slab_of_d.p, slabs_c.p, slabs_s.p, cnt_c.p, cnt_s.p, cap, world_tmp.p, kVoxelBlockMax, err.p, clean.p));
+  ILSM_CUDA(launch_pdl(cube_insert_kernel, dim3(2), dim3(1024), kVoxelBlockMax * sizeof(u64), s, cur_stack_c(), cur_stack_s(), d_counts, nc_host, ns_host, ctx->lm.p, world_frame, cenW, cenH, cenD, slab_of_d.p, slabs_c.p, slabs_s.p, cnt_c, cnt_s, cap, world_tmp.p, kVoxelBlockMax, err, clean.p));
   count_launches(1);
   return check_launch("cube_insert");
 }
@@ -338,7 +331,7 @@ int CubeMapH::filter_valid(cudaStream_t s) {
   for (int v = 0; v < 125; ++v) vs.slab[v] = v < n_valid ? slab_of[valid[v]] : 0;
   // shared memory: the hash-based path's 192 KB only when a cube can be large enough to take it
   const size_t smem = cap > 2048 ? kVgHashSmemBytes : (size_t)kVoxelBlockMax * sizeof(u64);
-  ILSM_CUDA(launch_pdl(cube_filter_kernel, dim3(2 * n_valid), dim3(1024), smem, s, vs, slabs_c.p, slabs_s.p, cnt_c.p, cnt_s.p, cap, line_res, plane_res, scratch.p, err.p, hscratch.p, clean.p, vg_merge ? 1 : 0));
+  ILSM_CUDA(launch_pdl(cube_filter_kernel, dim3(2 * n_valid), dim3(1024), smem, s, vs, slabs_c.p, slabs_s.p, cnt_c, cnt_s, cap, line_res, plane_res, scratch.p, err, hscratch.p, clean.p, vg_merge ? 1 : 0));
   count_launches(1);
   return check_launch("cube_filter");
 }
@@ -406,7 +399,7 @@ int cubemap_frame_enqueue(CubeMapH& m, const float* d_c, int nc, const float* d_
     const int ioff = stride_bytes >= 32 ? 4 : 3;
     ILSM_CUDA(cudaMemsetAsync(m.stack_n.p, 0, 4 * sizeof(int), c.stream));
     if ((rc = c.voxelgrid_pair_dev(d_c, nc, m.line_res, m.stack_c.p, d_s, ns, m.plane_res, m.stack_s.p, stride_bytes, ioff,
-                                   m.stack_n.p, c.stream, m.err.p)))
+                                   m.stack_n.p, c.stream, m.err)))
       return rc;
   }
   // pose in
@@ -484,7 +477,7 @@ int cubemap_frame_collect(CubeMapH& m, double q_w[4], double t_w[3], ilsm_reg_re
   if (pin_i[0]) {
     char msg[160];
     snprintf(msg, sizeof(msg), "cube map: capacity exceeded (flags 0x%x: 16 down-sampled stack>16384, 32 cube slab full, 64 cube>16384, 2 leaf too small)", pin_i[0]);
-    cudaMemsetAsync(m.err.p, 0, sizeof(int), c.stream);
+    cudaMemsetAsync(m.err, 0, sizeof(int), c.stream);
     return fail(ILSM_ERR_OUT_OF_MEMORY, msg);
   }
   return ILSM_OK;
@@ -514,7 +507,6 @@ ILSM_API int ilsm_cubemap_create(ilsm_ctx* ctx_, float line_res, float plane_res
   cudaSetDevice(c->device);
   int rc = h->m.init(c, line_res, plane_res, cube_capacity);
   if (rc) {
-    h->m.release();
     delete h;
     return rc;
   }
@@ -524,11 +516,8 @@ ILSM_API int ilsm_cubemap_create(ilsm_ctx* ctx_, float line_res, float plane_res
 
 ILSM_API void ilsm_cubemap_destroy(ilsm_cubemap* cm) {
   if (!cm) return;
-  {
-    std::lock_guard<std::mutex> lk(cm->m.ctx->mu);
-    cudaSetDevice(cm->m.ctx->device);
-    cm->m.release();
-  }
+  std::lock_guard<std::mutex> lk(cm->m.ctx->mu);
+  cudaSetDevice(cm->m.ctx->device);
   delete cm;
 }
 
@@ -587,7 +576,7 @@ ILSM_API int ilsm_cubemap_insert_world(ilsm_cubemap* cm, const float* corner, in
   const int flags = m.adopt_counts() | m.tail_flags;
   m.tail_flags = 0;
   if (flags) {
-    cudaMemsetAsync(m.err.p, 0, sizeof(int), c.stream);
+    cudaMemsetAsync(m.err, 0, sizeof(int), c.stream);
     return fail(ILSM_ERR_OUT_OF_MEMORY, "cube map: a cube exceeded its slab capacity");
   }
   return ILSM_OK;

@@ -305,14 +305,9 @@ ILSM_API int ilsm_ground_create(ilsm_ctx* ctx, ilsm_ground** out) {
 
 ILSM_API void ilsm_ground_destroy(ilsm_ground* g) {
   if (!g) return;
-  {
-    std::lock_guard<std::mutex> lk(g->ctx->mu);
-    cudaSetDevice(g->ctx->device);
-    cudaStreamSynchronize(g->ctx->stream);
-    GroundBufs& b = g->b;
-    b.raw.release(), b.coeff.release(), b.scr.release(), b.out.release(), b.chunk_cnt.release(), b.chunk_base.release();
-    b.totals.release(), b.triples.release(), b.counts.release(), b.models.release(), b.partial.release();
-  }
+  std::lock_guard<std::mutex> lk(g->ctx->mu);
+  cudaSetDevice(g->ctx->device);
+  cudaStreamSynchronize(g->ctx->stream);
   delete g;
 }
 

@@ -52,7 +52,7 @@ struct CubeMapH {
   DevBuf<float4> slabs_c, slabs_s, from_c, from_s, stack_c, stack_s, scratch, world_tmp;
   DevBuf<uint32_t> hscratch;  // hash-based VoxelGrid scratch, one slice per cube_filter block
   DevBuf<int> cnt_all;              // cnt_c | cnt_s | err, contiguous
-  DevBuf<int> cnt_c, cnt_s, err;    // views into cnt_all (not owned)
+  int *cnt_c = nullptr, *cnt_s = nullptr, *err = nullptr;  // views into cnt_all
   DevBuf<int> slab_of_d, stack_n, zero_list;
   // per slab and cloud kind: [0, 2 kCNum) the last VoxelGrid pass left the cube unchanged and nothing was inserted since;
   // [2 kCNum, 4 kCNum) how many leading points of the cube are the output of its last pass (merge precondition)
@@ -69,7 +69,7 @@ struct CubeMapH {
   PinnedBuf<int> pin;
 
   int init(Ctx* c, float lres, float pres, int cube_cap);
-  void release();
+  ~CubeMapH();  // synchronises the context's streams, then destroys ev_tail
   int roll(const double t[3]);
   int gather(int* n_mc, int* n_ms);
   int insert(const int* d_counts, int nc_host, int ns_host, int world_frame, cudaStream_t s = nullptr);

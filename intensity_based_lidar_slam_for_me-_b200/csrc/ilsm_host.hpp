@@ -6,6 +6,7 @@
 #include <stdint.h>
 #include <string.h>
 
+#include <atomic>
 #include <mutex>
 #include <string>
 
@@ -38,55 +39,66 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 
-// Grow-only device buffer (HBM is plentiful: 180 GB; reallocation would serialise the stream).
-template <typename T>
-struct DevBuf {
-  T* p = nullptr;
-  size_t cap = 0;
-  int reserve(size_t n) {
-    if (n <= cap) return ILSM_OK;
-    size_t want = n + n / 2 + 64;
-    T* np = nullptr;
-    cudaError_t e = cudaMalloc(&np, want * sizeof(T));
-    if (e != cudaSuccess) {
-      cudaGetLastError();
-      return fail(ILSM_ERR_OUT_OF_MEMORY, "cudaMalloc failed");
-    }
-    if (p) cudaFree(p);  // implicit device sync: only on growth
-    p = np;
-    cap = want;
-    return ILSM_OK;
-  }
-  void release() {
-    if (p) cudaFree(p);
-    p = nullptr;
-    cap = 0;
-  }
+// Bytes held by all device [0] and pinned [1] buffers of the process (ilsm_debug_live_bytes): a test can check that
+// closing a handle frees everything it allocated, which cudaMemGetInfo cannot show on a GPU other processes use too.
+extern std::atomic<long long> g_live_bytes[2];
+
+struct DeviceMem {
+  static constexpr int kind = 0;
+  static constexpr const char* what = "cudaMalloc failed";
+  static cudaError_t alloc(void** p, size_t bytes) { return cudaMalloc(p, bytes); }
+  static void dealloc(void* p) { cudaFree(p); }  // implicit device sync
+};
+struct PinnedMem {
+  static constexpr int kind = 1;
+  static constexpr const char* what = "cudaMallocHost failed";
+  static cudaError_t alloc(void** p, size_t bytes) { return cudaMallocHost(p, bytes); }
+  static void dealloc(void* p) { cudaFreeHost(p); }
 };
 
-template <typename T>
-struct PinnedBuf {
+// Grow-only buffer that owns its memory (HBM is plentiful: 180 GB; reallocation would serialise the stream).  Freed
+// when the buffer is destroyed: its owner's teardown must have synchronised every stream that still reads it.
+template <typename T, typename Mem>
+struct Buf {
   T* p = nullptr;
   size_t cap = 0;
+  Buf() = default;
+  Buf(const Buf&) = delete;
+  Buf& operator=(const Buf&) = delete;
+  Buf(Buf&& o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr, o.cap = 0; }
+  Buf& operator=(Buf&& o) noexcept {
+    if (this != &o) release(), p = o.p, cap = o.cap, o.p = nullptr, o.cap = 0;
+    return *this;
+  }
+  ~Buf() { release(); }
   int reserve(size_t n) {
     if (n <= cap) return ILSM_OK;
     size_t want = n + n / 2 + 64;
-    T* np = nullptr;
-    if (cudaMallocHost(&np, want * sizeof(T)) != cudaSuccess) {
+    void* np = nullptr;
+    if (Mem::alloc(&np, want * sizeof(T)) != cudaSuccess) {
       cudaGetLastError();
-      return fail(ILSM_ERR_OUT_OF_MEMORY, "cudaMallocHost failed");
+      return fail(ILSM_ERR_OUT_OF_MEMORY, Mem::what);
     }
-    if (p) cudaFreeHost(p);
-    p = np;
+    release();  // only on growth
+    p = static_cast<T*>(np);
     cap = want;
+    g_live_bytes[Mem::kind].fetch_add((long long)(cap * sizeof(T)), std::memory_order_relaxed);
     return ILSM_OK;
   }
+
+ private:
   void release() {
-    if (p) cudaFreeHost(p);
+    if (!p) return;
+    Mem::dealloc(p);
+    g_live_bytes[Mem::kind].fetch_sub((long long)(cap * sizeof(T)), std::memory_order_relaxed);
     p = nullptr;
     cap = 0;
   }
 };
+template <typename T>
+using DevBuf = Buf<T, DeviceMem>;
+template <typename T>
+using PinnedBuf = Buf<T, PinnedMem>;
 
 // Levenberg-Marquardt state that lives in HBM for the duration of a registration: the trust-region loop of
 // ceres::Solve runs on the device, one evaluation kernel per iteration, no host round trip.
@@ -179,7 +191,7 @@ struct Map {
   const uint32_t* cur_counters() const { return counters.p + 8 * cur; }
   int knn_dev(const float* d_q, int nq, int stride_bytes, int k, float max_dist, int32_t* d_idx, float* d_d2);
   GridView view() const;
-  void release();
+  ~Map();  // synchronises the map's stream, then destroys it and the events
 };
 
 // Device-side factor storage (SoA), one slot per stack point (corner slots first).
@@ -246,7 +258,7 @@ struct Ctx {
   bool bulk_attr_set = false;  // normal_eq_bulk_kernel's dynamic shared-memory opt-in done on this device
 
   int init(int dev);
-  void release();
+  ~Ctx();  // the caller has made `device` current
   // LM pose staging in `pinned`: the LM state prefix (pose and report, xq first) comes back to offset 0 in one copy, a
   // pose goes up from kPinPoseIn.  [kPinSite, kPinPoseIn) is left to a call site's own read-back in the same synchronise.
   static constexpr size_t kPinSite = 1024, kPinPoseIn = 2048;
@@ -332,6 +344,8 @@ struct ScDb {
   int candidates_dev(const float* d_qdesc, int n_search, int num_cand, int* d_id, float* d_key_d2, double* d_dist, int* d_shift);
   int make_dev(const float* d_pts, int n, int stride_bytes, float* d_desc);
   int query_dev(const float* d_qdesc, int n_search, int id_offset, int k, double* d_dist, int* d_id, int* d_shift);
+  ScDb();  // both in scancontext.cu, where ScQuery is complete
+  ~ScDb();
 };
 
 }  // namespace ilsm

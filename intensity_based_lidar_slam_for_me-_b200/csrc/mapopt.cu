@@ -112,16 +112,15 @@ ILSM_API int ilsm_mapopt_create(ilsm_ctx* ctx, float voxel_leaf, float downsampl
 
 ILSM_API void ilsm_mapopt_destroy(ilsm_mapopt* mo) {
   if (!mo) return;
-  MapOptH& m = mo->m;
+  ilsm_ground* ground = mo->m.ground;
   {
-    std::lock_guard<std::mutex> lk(m.ctx->mu);
-    cudaSetDevice(m.ctx->device);
-    cudaStreamSynchronize(m.ctx->stream);
-    m.map.release(), m.empty.release();
-    m.merged.release(), m.stack.release(), m.world.release(), m.plane_raw.release(), m.counts.release();
+    Ctx& c = *mo->m.ctx;
+    std::lock_guard<std::mutex> lk(c.mu);
+    cudaSetDevice(c.device);
+    cudaStreamSynchronize(c.stream);
+    delete mo;
   }
-  ilsm_ground_destroy(m.ground);
-  delete mo;
+  ilsm_ground_destroy(ground);  // takes the context's mutex itself
 }
 
 ILSM_API int ilsm_mapopt_map_size(const ilsm_mapopt* mo) { return mo ? mo->m.map.n : 0; }

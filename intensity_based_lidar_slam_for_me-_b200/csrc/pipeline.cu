@@ -205,7 +205,7 @@ static int stack_voxelgrid(Ctx& c, const CubeMapH& cm, const SlamH::FeSlot& o, c
   ILSM_CUDA(cudaMemsetAsync(set.n.p, 0, 4 * sizeof(int), c.aux));
   if ((rc = c.voxelgrid_pair_dev(reinterpret_cast<const float*>(o.lsharp.p), n_lsharp, cm.line_res, set.c.p,
                                  reinterpret_cast<const float*>(o.lf), n_lflat, cm.plane_res, set.s.p, 16, 3, set.n.p, c.aux,
-                                 cm.err.p)))
+                                 cm.err)))
     return rc;
   ILSM_CUDA(cudaEventRecord(set.ev_ready, c.aux));
   return ILSM_OK;
@@ -566,13 +566,9 @@ ILSM_API void ilsm_slam_destroy(ilsm_slam* slam) {
     std::lock_guard<std::mutex> lk(s.ctx->mu);
     cudaSetDevice(s.ctx->device);
     cudaStreamSynchronize(s.ctx->stream);
-    s.last_corner.release(), s.last_surf.release();
-    for (SlamH::FeSlot& o : s.fslot) {
-      o.sharp.release(), o.flat.release(), o.lsharp.release(), o.lflat.release();
+    for (SlamH::FeSlot& o : s.fslot)
       if (o.ev) cudaEventDestroy(o.ev);
-    }
     for (SlamH::StackSet& set : s.stk) {
-      set.c.release(), set.s.release(), set.n.release();
       if (set.ev_ready) cudaEventDestroy(set.ev_ready);
       if (set.ev_free) cudaEventDestroy(set.ev_free);
     }
@@ -581,7 +577,8 @@ ILSM_API void ilsm_slam_destroy(ilsm_slam* slam) {
   if (s.mapopt) ilsm_mapopt_destroy(s.mapopt);
   if (s.ctx2) ilsm_destroy(s.ctx2);
   if (s.ctx0) ilsm_destroy(s.ctx0);
-  delete slam;
+  cudaSetDevice(s.ctx->device);
+  delete slam;  // frees the slots, stack sets and last-frame maps: no stage reads them any more
 }
 
 ILSM_API ilsm_cubemap* ilsm_slam_cubemap(ilsm_slam* slam) { return slam ? slam->s.cube : nullptr; }

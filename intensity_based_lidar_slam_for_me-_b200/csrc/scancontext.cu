@@ -11,6 +11,8 @@
 // is stored as float32 [20][60] row-major = 4800 B per keyframe without loss; all arithmetic is fp64 like Eigen's.
 // The kernel is HBM-bound for one query (4800 B per candidate, ~12 kFLOP fp64); no tensor cores: the 7-shift
 // column-cosine search after sector-key alignment is not a dense contraction at batch size 1.
+#include <utility>
+
 #include "ilsm_host.hpp"
 
 namespace ilsm {
@@ -581,6 +583,9 @@ int sc_merge_dev(Ctx* ctx, const void* d_packed, int shards, int k, void* d_out,
 // ---------------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------------
+ScDb::ScDb() = default;
+ScDb::~ScDb() = default;
+
 int ScDb::append_dev(const float* d_desc, int n_add, bool from_host) {
   if (n_add <= 0) return ILSM_OK;
   const size_t need = (size_t)(count + n_add) * kDesc;
@@ -591,8 +596,7 @@ int ScDb::append_dev(const float* d_desc, int n_add, bool from_host) {
     if (count > 0)
       ILSM_CUDA(cudaMemcpyAsync(bigger.p, db.p, (size_t)count * kDesc * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
     ILSM_CUDA(cudaStreamSynchronize(ctx->stream));
-    db.release();
-    db = bigger;
+    db = std::move(bigger);
   }
   ILSM_CUDA(cudaMemcpyAsync(db.p + (size_t)count * kDesc, d_desc, (size_t)n_add * kDesc * sizeof(float),
                             from_host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, ctx->stream));
@@ -605,8 +609,7 @@ int ScDb::append_dev(const float* d_desc, int n_add, bool from_host) {
     if (count > 0)
       ILSM_CUDA(cudaMemcpyAsync(bigger.p, ringkey.p, (size_t)count * kNR * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
     ILSM_CUDA(cudaStreamSynchronize(ctx->stream));
-    ringkey.release();
-    ringkey = bigger;
+    ringkey = std::move(bigger);
   }
   ILSM_CUDA(launch_pdl(sc_ringkey_kernel, dim3((n_add * kNR + 255) / 256), dim3(256), 0, ctx->stream, (const float*)db.p, count, n_add,
                        ringkey.p));

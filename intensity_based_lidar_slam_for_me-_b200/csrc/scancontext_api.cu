@@ -176,7 +176,6 @@ ILSM_API int ilsm_sc_prefilter_debug(ilsm_sc* sc, const float* desc_20x60, int n
     ILSM_CUDA(cudaMemcpyAsync(aligned_shift, sh.p, (size_t)n_queries * n_search, cudaMemcpyDeviceToHost, c.stream));
     ILSM_CUDA(cudaStreamSynchronize(c.stream));
   }
-  sh.release();
   return rc;
 }
 
