@@ -645,6 +645,59 @@ ILSM_API int ilsm_sc_query_topk_sharded(ilsm_sc* sc, const float* desc_20x60, in
 ILSM_API int ilsm_sc_query_topk_sharded_dev(ilsm_sc* sc, const float* d_desc_20x60, int n_queries, int n_search, int id_offset, int k,
                                             void* d_packed_out);
 
+/* ------------------------------------------------ K6: loop-closure verification, point-to-point ICP ---- */
+/* pcl::IterativeClosestPoint<PointXYZI, PointXYZI> (PCL 1.10) for a batch of (source, target) pairs.  Per pair, starting
+ * from the guess P: every iteration maps the ORIGINAL source points by P (double math, float store), takes the exact 1-NN
+ * of each in the target (ties by (d2, index)), keeps the pairs with d2 <= max_correspondence_distance^2, fits the rigid
+ * transform of those pairs in closed form (fp64 sums, Horn's quaternion method) and composes it onto P, until
+ * DefaultConvergenceCriteria stops it.  The fitness is getFitnessScore(fitness_max_range) of the final pose: the mean 1-NN
+ * d2 over the points with d2 <= fitness_max_range -- PCL compares the SQUARED distance with the range; kept.
+ * Replaces: the pcl::IterativeClosestPoint of loopClosureThread  intensity_feature_tracker.cpp:195-393. */
+typedef enum ilsm_icp_state { /* pcl::registration::DefaultConvergenceCriteria::ConvergenceState, same order */
+  ILSM_ICP_NOT_CONVERGED = 0,
+  ILSM_ICP_ITERATIONS = 1,
+  ILSM_ICP_TRANSFORM = 2,
+  ILSM_ICP_ABS_MSE = 3,
+  ILSM_ICP_REL_MSE = 4,
+  ILSM_ICP_NO_CORRESPONDENCES = 5
+} ilsm_icp_state;
+
+typedef struct ilsm_icp_opts {
+  double max_correspondence_distance; /* metres; sqrt(DBL_MAX) = no gate */
+  int max_iterations;                 /* the loop is a do-while: 0 still runs one iteration */
+  int pad;
+  double transformation_epsilon;          /* on |t|^2 of one iteration's increment */
+  double transformation_rotation_epsilon; /* on cos(angle) of the increment; <= 0: 1 - transformation_epsilon */
+  double euclidean_fitness_epsilon;       /* on the relative change of the correspondence MSE */
+  double fitness_max_range;               /* compared with the 1-NN d2 of the fitness score */
+} ilsm_icp_opts;
+
+/* PCL 1.10's defaults: sqrt(DBL_MAX), 10, 0, 0, -DBL_MAX, DBL_MAX. */
+ILSM_API void ilsm_icp_opts_default(ilsm_icp_opts* o);
+
+typedef struct ilsm_icp_result {
+  double q_xyzw[4], t[3]; /* final transformation, source -> target */
+  double fitness;         /* getFitnessScore(fitness_max_range); DBL_MAX when no point is in range */
+  double mse;             /* the last correspondence search's mean d2; DBL_MAX when it found none */
+  int iterations;         /* nr_iterations_ */
+  int state;              /* ilsm_icp_state */
+  int converged;          /* hasConverged(): every state but NOT_CONVERGED and NO_CORRESPONDENCES */
+  int n_correspondences;  /* of the last correspondence search */
+} ilsm_icp_result;
+
+/* Pair p aligns source points [src_offsets[p], src_offsets[p+1]) (3 floats with a byte stride) to targets[p] (a built
+ * ilsm_map of this context), starting from guess7[7p..7p+6] = (qx,qy,qz,qw,tx,ty,tz), a unit quaternion, or the identity
+ * when guess7 is NULL.  opts NULL: the defaults.  One kernel launch for the whole batch; returns when results[0..n_pairs)
+ * are filled.  A pair with fewer than 3 source points or an empty target ends in ILSM_ICP_NO_CORRESPONDENCES with 0
+ * iterations and the guess as its pose.  The _dev form reads the points from device memory (offsets, guesses and results
+ * stay on the host). */
+ILSM_API int ilsm_icp_align_batch(ilsm_ctx* ctx, ilsm_map* const* targets, int n_pairs, const float* src_xyz,
+                                  const int* src_offsets, int stride_bytes, const double* guess7,
+                                  const ilsm_icp_opts* opts, ilsm_icp_result* results);
+ILSM_API int ilsm_icp_align_batch_dev(ilsm_ctx* ctx, ilsm_map* const* targets, int n_pairs, const float* d_src_xyz,
+                                      const int* src_offsets, int stride_bytes, const double* guess7,
+                                      const ilsm_icp_opts* opts, ilsm_icp_result* results);
+
 #ifdef __cplusplus
 }
 #endif

@@ -378,6 +378,124 @@ class SCManager {
   double last_dist_ = 0;
 };
 
+// ------------------------------------------------------------------------------------------------ pcl::IterativeClosestPoint
+// Eigen::Matrix4f's layout without Eigen: 16 floats, column-major, m(r, c).
+struct Matrix4f {
+  float m[16] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1};
+  static Matrix4f Identity() { return Matrix4f(); }
+  float& operator()(int r, int c) { return m[c * 4 + r]; }
+  float operator()(int r, int c) const { return m[c * 4 + r]; }
+};
+
+// Rigid transform (rotation block + translation column) -> (qx, qy, qz, qw, tx, ty, tz), in double.
+inline void matrix_to_pose7(const Matrix4f& T, double out[7]) {
+  double R[3][3];
+  for (int r = 0; r < 3; ++r)
+    for (int c = 0; c < 3; ++c) R[r][c] = T(r, c);
+  const double tr = R[0][0] + R[1][1] + R[2][2];
+  double x, y, z, w;
+  if (tr > 0) {
+    const double s = std::sqrt(tr + 1.0) * 2;
+    w = 0.25 * s, x = (R[2][1] - R[1][2]) / s, y = (R[0][2] - R[2][0]) / s, z = (R[1][0] - R[0][1]) / s;
+  } else if (R[0][0] > R[1][1] && R[0][0] > R[2][2]) {
+    const double s = std::sqrt(1.0 + R[0][0] - R[1][1] - R[2][2]) * 2;
+    w = (R[2][1] - R[1][2]) / s, x = 0.25 * s, y = (R[0][1] + R[1][0]) / s, z = (R[0][2] + R[2][0]) / s;
+  } else if (R[1][1] > R[2][2]) {
+    const double s = std::sqrt(1.0 + R[1][1] - R[0][0] - R[2][2]) * 2;
+    w = (R[0][2] - R[2][0]) / s, x = (R[0][1] + R[1][0]) / s, y = 0.25 * s, z = (R[1][2] + R[2][1]) / s;
+  } else {
+    const double s = std::sqrt(1.0 + R[2][2] - R[0][0] - R[1][1]) * 2;
+    w = (R[1][0] - R[0][1]) / s, x = (R[0][2] + R[2][0]) / s, y = (R[1][2] + R[2][1]) / s, z = 0.25 * s;
+  }
+  const double n = std::sqrt(x * x + y * y + z * z + w * w);
+  out[0] = x / n, out[1] = y / n, out[2] = z / n, out[3] = w / n;
+  out[4] = T(0, 3), out[5] = T(1, 3), out[6] = T(2, 3);
+}
+
+inline Matrix4f pose7_to_matrix(const double q[4], const double t[3]) {
+  const double x = q[0], y = q[1], z = q[2], w = q[3];
+  Matrix4f T;
+  T(0, 0) = (float)(1 - 2 * (y * y + z * z)), T(0, 1) = (float)(2 * (x * y - w * z)), T(0, 2) = (float)(2 * (x * z + w * y));
+  T(1, 0) = (float)(2 * (x * y + w * z)), T(1, 1) = (float)(1 - 2 * (x * x + z * z)), T(1, 2) = (float)(2 * (y * z - w * x));
+  T(2, 0) = (float)(2 * (x * z - w * y)), T(2, 1) = (float)(2 * (y * z + w * x)), T(2, 2) = (float)(1 - 2 * (x * x + y * y));
+  T(0, 3) = (float)t[0], T(1, 3) = (float)t[1], T(2, 3) = (float)t[2];
+  return T;
+}
+
+// icp.setInputSource(cur); icp.setInputTarget(submap); icp.align(result, guess);
+// if (icp.hasConverged() && icp.getFitnessScore() < threshold) ...   loopClosureThread, intensity_feature_tracker.cpp:195-393
+// One align() is a batch of one of ilsm_icp_align_batch; the pose is kept in double (lastResult()) and rounded into the
+// Matrix4f of getFinalTransformation().
+template <typename PointSource, typename PointTarget>
+class IterativeClosestPoint {
+ public:
+  typedef PointCloud<PointSource> SourceCloud;
+  explicit IterativeClosestPoint(ContextPtr ctx = Context::shared()) : ctx_(std::move(ctx)) {
+    check(ilsm_map_create(ctx_->get(), &target_), "ilsm_map_create");
+    ilsm_icp_opts_default(&opts_);
+    res_ = ilsm_icp_result();
+  }
+  ~IterativeClosestPoint() { ilsm_map_destroy(target_); }
+  IterativeClosestPoint(const IterativeClosestPoint&) = delete;
+  IterativeClosestPoint& operator=(const IterativeClosestPoint&) = delete;
+
+  template <typename CloudT>
+  void setInputSource(const std::shared_ptr<CloudT>& cloud) { setInputSource(*cloud); }
+  template <typename CloudT>
+  void setInputSource(const CloudT& cloud) {
+    src_.resize(cloud.points.size() * 3);
+    for (size_t i = 0; i < cloud.points.size(); ++i)
+      src_[3 * i] = cloud.points[i].x, src_[3 * i + 1] = cloud.points[i].y, src_[3 * i + 2] = cloud.points[i].z;
+  }
+  // the target's search structure is built here, once, like PCL's k-d tree
+  template <typename CloudT>
+  void setInputTarget(const std::shared_ptr<CloudT>& cloud) { setInputTarget(*cloud); }
+  template <typename CloudT>
+  void setInputTarget(const CloudT& cloud) {
+    typedef typename std::remove_reference<decltype(cloud.points[0])>::type P;
+    check(ilsm_map_build(target_, cloud_ptr(cloud), (int)cloud.points.size(), stride_of<P>(), 0.f), "setInputTarget");
+  }
+  void setMaxCorrespondenceDistance(double d) { opts_.max_correspondence_distance = d; }
+  void setMaximumIterations(int n) { opts_.max_iterations = n; }
+  void setTransformationEpsilon(double e) { opts_.transformation_epsilon = e; }
+  void setTransformationRotationEpsilon(double e) { opts_.transformation_rotation_epsilon = e; }
+  void setEuclideanFitnessEpsilon(double e) { opts_.euclidean_fitness_epsilon = e; }
+  void setRANSACIterations(int n) {  // no correspondence rejector is implemented: only PCL's "none" (0) is honoured
+    if (n != 0) std::fprintf(stderr, "[ilsm] IterativeClosestPoint::setRANSACIterations(%d) ignored: no rejector\n", n);
+  }
+
+  void align(SourceCloud& output) { align(output, Matrix4f::Identity()); }
+  void align(SourceCloud& output, const Matrix4f& guess) {
+    double g[7];
+    matrix_to_pose7(guess, g);
+    const int offs[2] = {0, (int)(src_.size() / 3)};
+    ilsm_map* tg = target_;
+    check(ilsm_icp_align_batch(ctx_->get(), &tg, 1, src_.empty() ? nullptr : src_.data(), offs, 12, g, &opts_, &res_),
+          "IterativeClosestPoint::align");
+    final_ = pose7_to_matrix(res_.q_xyzw, res_.t);
+    output.resize(src_.size() / 3);
+    for (size_t i = 0; i < output.points.size(); ++i) {  // the source under the final transformation
+      const float* p = &src_[3 * i];
+      PointSource& o = output.points[i];
+      o.x = final_(0, 0) * p[0] + final_(0, 1) * p[1] + final_(0, 2) * p[2] + final_(0, 3);
+      o.y = final_(1, 0) * p[0] + final_(1, 1) * p[1] + final_(1, 2) * p[2] + final_(1, 3);
+      o.z = final_(2, 0) * p[0] + final_(2, 1) * p[1] + final_(2, 2) * p[2] + final_(2, 3);
+    }
+  }
+  bool hasConverged() const { return res_.converged != 0; }
+  double getFitnessScore() const { return res_.fitness; }  // PCL's default range: every point
+  Matrix4f getFinalTransformation() const { return final_; }
+  const ilsm_icp_result& lastResult() const { return res_; }
+
+ private:
+  ContextPtr ctx_;
+  ilsm_map* target_ = nullptr;
+  std::vector<float> src_;
+  ilsm_icp_opts opts_;
+  ilsm_icp_result res_;
+  Matrix4f final_;
+};
+
 // ------------------------------------------------------------------------------------------------ ImageHandler
 class ImageHandler {
  public:

@@ -88,6 +88,36 @@ class MapOptStats(C.Structure):
                 ("solve", SolveSummary), ("q_key", C.c_double * 4), ("t_key", C.c_double * 3), ("reserved", C.c_double)]
 
 
+class IcpOpts(C.Structure):
+    """ilsm_icp_opts (pcl::IterativeClosestPoint's settings); IcpOpts() holds PCL 1.10's defaults."""
+    _fields_ = [("max_correspondence_distance", C.c_double), ("max_iterations", C.c_int32), ("pad", C.c_int32),
+                ("transformation_epsilon", C.c_double), ("transformation_rotation_epsilon", C.c_double),
+                ("euclidean_fitness_epsilon", C.c_double), ("fitness_max_range", C.c_double)]
+
+    def __init__(self, **kw):
+        super().__init__()
+        load_library().ilsm_icp_opts_default(C.byref(self))
+        for k, v in kw.items():
+            setattr(self, k, v)
+
+
+ICP_NOT_CONVERGED, ICP_ITERATIONS, ICP_TRANSFORM, ICP_ABS_MSE, ICP_REL_MSE, ICP_NO_CORRESPONDENCES = range(6)
+
+
+class IcpResult(C.Structure):
+    """ilsm_icp_result: final transformation (source -> target), getFitnessScore, convergence state."""
+    _fields_ = [("q_xyzw", C.c_double * 4), ("t", C.c_double * 3), ("fitness", C.c_double), ("mse", C.c_double),
+                ("iterations", C.c_int32), ("state", C.c_int32), ("converged", C.c_int32), ("n_correspondences", C.c_int32)]
+
+    @property
+    def q(self):
+        return np.array(self.q_xyzw[:], np.float64)
+
+    @property
+    def tv(self):
+        return np.array(self.t[:], np.float64)
+
+
 DMATCH_DTYPE = np.dtype([("queryIdx", "<i4"), ("trainIdx", "<i4"), ("imgIdx", "<i4"), ("distance", "<f4")])
 FACTOR_DTYPE = np.dtype([("type", "<i4"), ("src", "<i4"), ("p", "<f8", 3), ("a", "<f8", 3), ("b", "<f8", 3)])
 
@@ -204,6 +234,9 @@ def load_library(path: str | None = None):
         "ilsm_eval_normal_eq_dev": (i32, [vp, vp, f64, vp]),
         "ilsm_solve_dev": (i32, [vp, vp, i32, f64]),
         "ilsm_solve": (i32, [vp, vp, vp, i32, f64, C.POINTER(SolveSummary)]),
+        "ilsm_icp_opts_default": (None, [C.POINTER(IcpOpts)]),
+        "ilsm_icp_align_batch": (i32, [vp, vp, i32, vp, vp, i32, vp, C.POINTER(IcpOpts), vp]),
+        "ilsm_icp_align_batch_dev": (i32, [vp, vp, i32, vp, vp, i32, vp, C.POINTER(IcpOpts), vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
@@ -461,6 +494,33 @@ class Context:
         s = SolveSummary()
         _check(self._lib.ilsm_solve(self._h, _ptr(qq), _ptr(tt), max_num_iterations, huber_a, C.byref(s)))
         return qq, tt, s
+
+
+    # -- loopClosureThread's pcl::IterativeClosestPoint (intensity_feature_tracker.cpp:195-393) ------
+    def icp_align(self, target: "LocalMap", source, q=(0.0, 0.0, 0.0, 1.0), t=(0.0, 0.0, 0.0), **opts) -> IcpResult:
+        """align(output, guess) of `source` ((n, >=3) points) to `target`, plus getFitnessScore; opts: IcpOpts fields."""
+        return self.icp_align_batch([target], [source], [(q, t)], **opts)[0]
+
+    def icp_align_batch(self, targets, sources, guesses=None, **opts) -> list:
+        """One launch for every (target, source) pair; guesses: None (identity) or one (q_xyzw, t) per pair.  Returns a
+        list of IcpResult."""
+        n = len(targets)
+        if len(sources) != n or (guesses is not None and len(guesses) != n):
+            raise ValueError("one source (and guess) per target")
+        pts = [np.asarray(s, np.float32)[:, :3] for s in sources]
+        offs = np.zeros(n + 1, np.int32)
+        offs[1:] = np.cumsum([len(p) for p in pts])
+        src = np.ascontiguousarray(np.concatenate(pts) if n else np.zeros((0, 3), np.float32))
+        g = None
+        if guesses is not None:
+            g = np.ascontiguousarray([np.concatenate([np.asarray(q, np.float64), np.asarray(t, np.float64)])
+                                      for q, t in guesses], np.float64).reshape(n, 7)
+        hs = (C.c_void_p * max(n, 1))(*[m._h.value for m in targets])
+        res = (IcpResult * max(n, 1))()
+        o = IcpOpts(**opts)
+        _check(self._lib.ilsm_icp_align_batch(self._h, hs, n, _ptr(src), _ptr(offs), 12, _ptr(g) if g is not None else None,
+                                              C.byref(o), res))
+        return [res[i] for i in range(n)]
 
 
 class LocalMap:

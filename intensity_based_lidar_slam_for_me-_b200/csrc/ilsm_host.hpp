@@ -4,6 +4,7 @@
 #include <limits.h>
 #include <stddef.h>
 #include <stdint.h>
+#include <stdlib.h>
 #include <string.h>
 
 #include <atomic>
@@ -37,6 +38,30 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr, cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
+}
+
+// Cluster size of the kernels that run a whole iterative solve in one thread-block cluster (the LM solve, ICP): `wide`
+// CTAs, a non-portable size, where the device can place one cluster of `kernel` with `threads` threads per CTA, else the
+// portable 8; ILSM_SOLVE_CLUSTER=8 forces 8.  Probed once per context and kernel: `cached` is -1 until then, then 1 or 0.
+template <typename... KArgs>
+bool wide_cluster(int& cached, void (*kernel)(KArgs...), int wide, int threads) {
+  if (cached < 0) {
+    cached = 0;
+    if (cudaFuncSetAttribute(kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess) {
+      cudaLaunchConfig_t cfg = {};
+      cfg.gridDim = dim3(wide), cfg.blockDim = dim3(threads);
+      cudaLaunchAttribute at;
+      at.id = cudaLaunchAttributeClusterDimension;
+      at.val.clusterDim.x = wide, at.val.clusterDim.y = 1, at.val.clusterDim.z = 1;
+      cfg.attrs = &at, cfg.numAttrs = 1;
+      int n_clusters = 0;
+      if (cudaOccupancyMaxActiveClusters(&n_clusters, kernel, &cfg) == cudaSuccess && n_clusters >= 1) cached = 1;
+    }
+    (void)cudaGetLastError();
+    if (const char* e = getenv("ILSM_SOLVE_CLUSTER"))
+      if (atoi(e) == 8) cached = 0;
+  }
+  return cached != 0;
 }
 
 // Bytes held by all device [0] and pinned [1] buffers of the process (ilsm_debug_live_bytes): a test can check that
@@ -255,7 +280,14 @@ struct Ctx {
   int knn_group = 8;          // queries per group of the binned search (ILSM_KNN_GROUP: 1, 2, 4, 8, 16 or 32)
   int knn_binned_min = 8192;  // query sets at least this large take the binned path (ILSM_KNN_BINNED_MIN overrides)
   size_t partial_blocks = 0;
-  bool bulk_attr_set = false;  // normal_eq_bulk_kernel's dynamic shared-memory opt-in done on this device
+  bool bulk_attr_set = false;
+  // ICP verification batches (icp.cu): staged source points, per-pair records, tile partials, results
+  DevBuf<float> icp_src;
+  DevBuf<unsigned char> icp_pairs;
+  DevBuf<double> icp_part;
+  DevBuf<ilsm_icp_result> icp_res;
+  PinnedBuf<unsigned char> icp_pin;
+  int icp_wide = -1;  // ICP as 16-CTA clusters (1) or 8 (0); -1: not probed yet  // normal_eq_bulk_kernel's dynamic shared-memory opt-in done on this device
 
   int init(int dev);
   ~Ctx();  // the caller has made `device` current

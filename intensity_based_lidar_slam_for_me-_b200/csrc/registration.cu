@@ -1441,24 +1441,7 @@ int Ctx::solve_launch(int max_iter, double huber_a, int pass, const PoseDst* dst
   prm.d_pose7_out = dst ? dst->d_pose7 : nullptr;
   prm.d_report_out = dst ? dst->d_report : nullptr;
   FactorView fv = factor_view(fac, false);
-  if (solve_wide < 0) {  // first solve of this context: can the device place a 16-CTA cluster?
-    solve_wide = 0;
-    auto* k16 = solve_cluster_kernel<kClusterSizeWide, kSolveThreadsWide>;
-    if (cudaFuncSetAttribute(k16, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess) {
-      cudaLaunchConfig_t cfg = {};
-      cfg.gridDim = dim3(kClusterSizeWide), cfg.blockDim = dim3(kSolveThreadsWide);
-      cudaLaunchAttribute at;
-      at.id = cudaLaunchAttributeClusterDimension;
-      at.val.clusterDim.x = kClusterSizeWide, at.val.clusterDim.y = 1, at.val.clusterDim.z = 1;
-      cfg.attrs = &at, cfg.numAttrs = 1;
-      int n_clusters = 0;
-      if (cudaOccupancyMaxActiveClusters(&n_clusters, k16, &cfg) == cudaSuccess && n_clusters >= 1) solve_wide = 1;
-    }
-    (void)cudaGetLastError();
-    if (const char* e = getenv("ILSM_SOLVE_CLUSTER"))
-      if (atoi(e) == 8) solve_wide = 0;
-  }
-  if (solve_wide)
+  if (wide_cluster(solve_wide, solve_cluster_kernel<kClusterSizeWide, kSolveThreadsWide>, kClusterSizeWide, kSolveThreadsWide))
     ILSM_CUDA(launch_pdl(solve_cluster_kernel<kClusterSizeWide, kSolveThreadsWide>, dim3(kClusterSizeWide), dim3(kSolveThreadsWide), 0,
                          stream, fv, fac.n, lm.p, prm, d_stack_counts));
   else

@@ -411,3 +411,31 @@ def sc_queries(db, n_q, seed=SEED_SC + 1, noise=0.05):
         d = d + (rng.normal(0.0, noise, d.shape).astype(np.float32) * occ)
         q[j] = d
     return q, ids.astype(np.int32), shifts.astype(np.int32)
+
+
+def loop_keyframes(n_per_lap=12, laps=2, radius=8.0, leaf=0.4, seed=0x5EED1C00, scene=None):
+    """Keyframes of a closed path through the box scene (Scene()): `laps` times around a circle of `radius` m, every lap
+    0.1 m further out and 3 degrees more yaw than the one before, so that keyframe k of a lap revisits keyframe k of the
+    first.  Per keyframe: true pose (q, t), `src` = its OS0-64 frame thinned by VoxelGrid(leaf) in the sensor frame,
+    `world` = the same points in the world frame.  Loop-closure verification workload (tools/icp_bench.py, ICP tests)."""
+    scene = scene or Scene()
+    out = []
+    for lap in range(laps):
+        for k in range(n_per_lap):
+            a = 2 * np.pi * k / n_per_lap
+            r = radius + 0.1 * lap
+            q = quat_from_rotvec([0.0, 0.0, a + np.pi / 2 + np.deg2rad(3.0 * lap)])
+            t = np.array([r * np.cos(a), r * np.sin(a), 1.5])
+            cloud, _ = make_frame(scene, q, t, seed=seed + lap * n_per_lap + k)
+            pts = cloud[np.any(cloud[:, :3] != 0, axis=1), :3]
+            src = voxel_centroid_np(pts, leaf)
+            world = (src.astype(np.float64) @ quat_to_mat(q).T + t).astype(np.float32)
+            out.append(dict(q=q, t=t, src=src, world=world, lap=lap, k=k))
+    return out
+
+
+def loop_submap(kfs, c, n_per_lap, half=2, leaf=0.4):
+    """World-frame submap around keyframe c: keyframes c-half .. c+half of c's lap (cyclic), VoxelGrid(leaf)."""
+    lap0 = (c // n_per_lap) * n_per_lap
+    ids = [lap0 + (c - lap0 + d) % n_per_lap for d in range(-half, half + 1)]
+    return voxel_centroid_np(np.concatenate([kfs[i]["world"] for i in ids]), leaf)
