@@ -31,44 +31,10 @@ int check_launch(const char* where) {
   return ILSM_OK;
 }
 
-int eval_only_launch(Ctx* c, double* d_out, const double* d_pose7 = nullptr, double huber_a = 0.0);
+int eval_only_launch(Ctx* c, double* d_out, const double* d_pose7, double huber_a);
 int factors_export(Ctx* c, ilsm_factor* d_out);
 int sc_merge_dev(Ctx* ctx, const void* d_packed, int shards, int k, void* d_out, int batch = 1, size_t shard_stride = 0);
 void sc_nccl_release(ScDb& d);  // scancontext_api.cu
-
-struct Pose7 {
-  double v[7];
-};
-
-__global__ void set_pose_kernel(LmState* st, Pose7 p, int also_candidate, double huber_a) {
-  pdl_entry();
-  for (int i = 0; i < 4; ++i) st->xq[i] = p.v[i];
-  for (int i = 0; i < 3; ++i) st->xt[i] = p.v[4 + i];
-  if (also_candidate) {
-    for (int i = 0; i < 4; ++i) st->cq[i] = p.v[i];
-    for (int i = 0; i < 3; ++i) st->ct[i] = p.v[4 + i];
-    st->huber_a = huber_a;
-  }
-}
-
-__global__ void pose_io_kernel(LmState* st, double* pose7, ilsm_reg_report* report, int direction) {
-  pdl_entry();
-  // direction 0: pose7 -> state ; 1: state -> pose7 (+ report)
-  int t = threadIdx.x;
-  if (direction == 0) {
-    if (t < 4) st->xq[t] = pose7[t];
-    else if (t < 7) st->xt[t - 4] = pose7[t];
-  } else {
-    if (t < 4) pose7[t] = st->xq[t];
-    else if (t < 7) pose7[t] = st->xt[t - 4];
-    if (report) {
-      const int words = (int)(sizeof(ilsm_reg_report) / 4);
-      const int32_t* src = reinterpret_cast<const int32_t*>(&st->report);
-      int32_t* dst = reinterpret_cast<int32_t*>(report);
-      for (int w = t; w < words; w += blockDim.x) dst[w] = src[w];
-    }
-  }
-}
 
 int Ctx::init(int dev) {
   int count = 0;
@@ -117,8 +83,6 @@ Map::~Map() {
   if (ctx_done) cudaEventDestroy(ctx_done);
   if (stream) cudaStreamDestroy(stream);
 }
-
-static bool valid_stride(int s) { return s >= 12 && (s % 4) == 0; }
 
 static ilsm_reg_opts sanitize(const ilsm_reg_opts* o) {
   ilsm_reg_opts r;
@@ -353,6 +317,35 @@ static int check_reg_args(ilsm_ctx* ctx, ilsm_map* mc, ilsm_map* ms, const float
   return ILSM_OK;
 }
 
+static int check_map_size(const ilsm_reg_opts& o, const ilsm_map* mc, const ilsm_map* ms) {
+  if ((o.min_corner_map > 0 && !(mc->m.n > o.min_corner_map)) || (o.min_surf_map > 0 && !(ms->m.n > o.min_surf_map)))
+    return fail(ILSM_ERR_NOT_ENOUGH_MAP, "time Map corner and surf num are not enough");
+  return ILSM_OK;
+}
+
+// the initial guess of a host-pointer entry point, carried by the first association launch
+static PoseSrc host_pose(const double q[4], const double t[3]) {
+  PoseSrc src;
+  src.mode = 1;
+  for (int i = 0; i < 4; ++i) src.v[i] = q[i];
+  for (int i = 0; i < 3; ++i) src.v[4 + i] = t[i];
+  return src;
+}
+
+// the factor records of the last association to the caller's host buffer (nullptr: none wanted), through the out_idx
+// scratch (reinterpreted) to keep allocations few; the caller synchronises
+static int export_factors(Ctx& c, ilsm_factor* factors) {
+  const int n = c.fac.n;
+  if (!factors || n == 0) return ILSM_OK;
+  size_t words = ((size_t)n * sizeof(ilsm_factor) + 3) / 4;
+  int rc;
+  if ((rc = c.out_idx.reserve(words + 8))) return rc;
+  ilsm_factor* d_f = reinterpret_cast<ilsm_factor*>(c.out_idx.p);
+  if ((rc = factors_export(&c, d_f))) return rc;
+  ILSM_CUDA(cudaMemcpyAsync(factors, d_f, (size_t)n * sizeof(ilsm_factor), cudaMemcpyDeviceToHost, c.stream));
+  return ILSM_OK;
+}
+
 // stage both stacks into ctx.stack_raw; returns device pointers
 static int stage_stacks(Ctx& c, const float* corner, int nc, const float* surf, int ns, int stride_bytes,
                         const float** d_corner, const float** d_surf) {
@@ -377,8 +370,7 @@ ILSM_API int ilsm_register_dev(ilsm_ctx* ctx, ilsm_map* mc, ilsm_map* ms, const 
   Ctx& c = ctx->c;
   std::lock_guard<std::mutex> lk(c.mu);
   ILSM_CUDA(cudaSetDevice(c.device));
-  if ((o.min_corner_map > 0 && !(mc->m.n > o.min_corner_map)) || (o.min_surf_map > 0 && !(ms->m.n > o.min_surf_map)))
-    return fail(ILSM_ERR_NOT_ENOUGH_MAP, "time Map corner and surf num are not enough");
+  if ((rc = check_map_size(o, mc, ms))) return rc;
   // the first association reads the pose straight from d_pose7 (and seeds the LM state), the last solve writes the
   // result and the report back: no separate pose upload / download launches
   PoseSrc src;
@@ -414,21 +406,13 @@ ILSM_API int ilsm_register(ilsm_ctx* ctx, ilsm_map* mc, ilsm_map* ms, const floa
   std::lock_guard<std::mutex> lk(c.mu);
   ILSM_CUDA(cudaSetDevice(c.device));
   if (report) memset(report, 0, sizeof(*report));
-  if ((o.min_corner_map > 0 && !(mc->m.n > o.min_corner_map)) || (o.min_surf_map > 0 && !(ms->m.n > o.min_surf_map)))
-    return fail(ILSM_ERR_NOT_ENOUGH_MAP, "time Map corner and surf num are not enough");
+  if ((rc = check_map_size(o, mc, ms))) return rc;
   const float *d_corner, *d_surf;
   if ((rc = stage_stacks(c, corner, nc, surf, ns, stride_bytes, &d_corner, &d_surf))) return rc;
-  PoseSrc src;  // the initial guess travels with the first association launch
-  src.mode = 1;
-  for (int i = 0; i < 4; ++i) src.v[i] = q[i];
-  for (int i = 0; i < 3; ++i) src.v[4 + i] = t[i];
+  const PoseSrc src = host_pose(q, t);
   if (o.outer_iterations < 1) return ILSM_OK;
   if ((rc = c.register_dev(&mc->m, &ms->m, d_corner, nc, d_surf, ns, stride_bytes, o, &src, nullptr))) return rc;
-  if ((rc = c.read_back_lm(c.stream))) return rc;
-  ILSM_CUDA(cudaStreamSynchronize(c.stream));
-  c.lm_result(q, t, report);
-  if (report) report->passes = o.outer_iterations;
-  return ILSM_OK;
+  return c.lm_finish(q, t, report, o.outer_iterations);
 }
 
 // Front end + stacks + registration of one organised frame against two prebuilt maps, the frame already on the device.
@@ -450,10 +434,9 @@ static int register_frame_core(Ctx& c, Map* mc, Map* ms, const float* d_frame, i
   if ((rc = c.gather_dev(c.fe.cloud.p, c.fe.lsharp.p, c.fe.counts.p, 2, n_lsharp, c.rf_lsharp.p))) return rc;
   // downSizeFilterCorner / downSizeFilterSurf (laserMapping.cpp:608-616)
   ILSM_CUDA(cudaMemsetAsync(c.rf_stack_n.p, 0, 4 * sizeof(int), c.stream));
-  if ((rc = c.voxelgrid_pair_dev(reinterpret_cast<const float*>(c.rf_lsharp.p), n_lsharp, line_res, c.rf_stack_c.p,
-                                 reinterpret_cast<const float*>(c.fe.lflat.p), n_lflat, plane_res, c.rf_stack_s.p, 16, 3, c.rf_stack_n.p,
-                                 c.stream)))
-    return rc;
+  const Ctx::VgCloud vc[2] = {{reinterpret_cast<const float*>(c.rf_lsharp.p), n_lsharp, line_res, c.rf_stack_c.p, c.rf_stack_n.p},
+                              {reinterpret_cast<const float*>(c.fe.lflat.p), n_lflat, plane_res, c.rf_stack_s.p, c.rf_stack_n.p + 1}};
+  if ((rc = c.voxelgrid(vc, 2, 16, 3, c.stream))) return rc;
   if (o.outer_iterations < 1) return ILSM_OK;
   // the association / solve block with the stack sizes read on the device (laserMapping.cpp:640-861)
   c.d_stack_counts = c.rf_stack_n.p;
@@ -463,28 +446,34 @@ static int register_frame_core(Ctx& c, Map* mc, Map* ms, const float* d_frame, i
   return rc;
 }
 
+// the argument checks of ilsm_register_frame[_dev]; `who` names the entry point in the message
+static int check_frame_args(ilsm_ctx* ctx, ilsm_map* mc, ilsm_map* ms, const float* xyzi, int n, bool has_pose, int stride_bytes,
+                            float line_res, float plane_res, const char* who) {
+  char msg[160];
+  if (!ctx || !mc || !ms || (n > 0 && !xyzi) || !has_pose)
+    return snprintf(msg, sizeof(msg), "%s: null argument", who), fail(ILSM_ERR_INVALID_ARG, msg);
+  if (mc->m.ctx != &ctx->c || ms->m.ctx != &ctx->c)
+    return snprintf(msg, sizeof(msg), "%s: map belongs to another context", who), fail(ILSM_ERR_INVALID_ARG, msg);
+  if (n < 0 || !valid_stride(stride_bytes) || stride_bytes < 16 || !(line_res > 0.f) || !(plane_res > 0.f))
+    return snprintf(msg, sizeof(msg), "%s: bad n/stride/resolution", who), fail(ILSM_ERR_INVALID_ARG, msg);
+  return ILSM_OK;
+}
+
 ILSM_API int ilsm_register_frame(ilsm_ctx* ctx, ilsm_map* mc, ilsm_map* ms, const float* xyzi, int n, int stride_bytes, float min_range,
                                  float line_res, float plane_res, double q[4], double t[3], const ilsm_reg_opts* opts,
                                  ilsm_reg_report* report, int32_t sizes_out[4]) {
-  if (!ctx || !mc || !ms || (n > 0 && !xyzi) || !q || !t) return fail(ILSM_ERR_INVALID_ARG, "register_frame: null argument");
-  if (mc->m.ctx != &ctx->c || ms->m.ctx != &ctx->c) return fail(ILSM_ERR_INVALID_ARG, "register_frame: map belongs to another context");
-  if (n < 0 || !valid_stride(stride_bytes) || stride_bytes < 16 || !(line_res > 0.f) || !(plane_res > 0.f))
-    return fail(ILSM_ERR_INVALID_ARG, "register_frame: bad n/stride/resolution");
+  int rc = check_frame_args(ctx, mc, ms, xyzi, n, q && t, stride_bytes, line_res, plane_res, "register_frame");
+  if (rc) return rc;
   ilsm_reg_opts o = sanitize(opts);
   Ctx& c = ctx->c;
   std::lock_guard<std::mutex> lk(c.mu);
   ILSM_CUDA(cudaSetDevice(c.device));
   if (report) memset(report, 0, sizeof(*report));
-  if ((o.min_corner_map > 0 && !(mc->m.n > o.min_corner_map)) || (o.min_surf_map > 0 && !(ms->m.n > o.min_surf_map)))
-    return fail(ILSM_ERR_NOT_ENOUGH_MAP, "time Map corner and surf num are not enough");
+  if ((rc = check_map_size(o, mc, ms))) return rc;
   const size_t bytes = (size_t)n * stride_bytes;
-  int rc;
   if ((rc = c.fe.raw.reserve(bytes / 4 + 4))) return rc;
   if (bytes) ILSM_CUDA(cudaMemcpyAsync(c.fe.raw.p, xyzi, bytes, cudaMemcpyHostToDevice, c.stream));
-  PoseSrc src;
-  src.mode = 1;
-  for (int i = 0; i < 4; ++i) src.v[i] = q[i];
-  for (int i = 0; i < 3; ++i) src.v[4 + i] = t[i];
+  const PoseSrc src = host_pose(q, t);
   int counts[8];
   if ((rc = register_frame_core(c, &mc->m, &ms->m, c.fe.raw.p, n, stride_bytes, min_range > 0.f ? min_range : 0.3f, line_res, plane_res, o,
                                 &src, nullptr, counts)))
@@ -505,10 +494,8 @@ ILSM_API int ilsm_register_frame(ilsm_ctx* ctx, ilsm_map* mc, ilsm_map* ms, cons
 
 ILSM_API int ilsm_register_frame_dev(ilsm_ctx* ctx, ilsm_map* mc, ilsm_map* ms, const float* d_xyzi, int n, int stride_bytes,
                                      float min_range, float line_res, float plane_res, double* d_pose7, const ilsm_reg_opts* opts) {
-  if (!ctx || !mc || !ms || (n > 0 && !d_xyzi) || !d_pose7) return fail(ILSM_ERR_INVALID_ARG, "register_frame_dev: null argument");
-  if (mc->m.ctx != &ctx->c || ms->m.ctx != &ctx->c) return fail(ILSM_ERR_INVALID_ARG, "register_frame_dev: map belongs to another context");
-  if (n < 0 || !valid_stride(stride_bytes) || stride_bytes < 16 || !(line_res > 0.f) || !(plane_res > 0.f))
-    return fail(ILSM_ERR_INVALID_ARG, "register_frame_dev: bad n/stride/resolution");
+  int rc = check_frame_args(ctx, mc, ms, d_xyzi, n, d_pose7 != nullptr, stride_bytes, line_res, plane_res, "register_frame_dev");
+  if (rc) return rc;
   ilsm_reg_opts o = sanitize(opts);
   Ctx& c = ctx->c;
   std::lock_guard<std::mutex> lk(c.mu);
@@ -534,22 +521,11 @@ ILSM_API int ilsm_associate(ilsm_ctx* ctx, ilsm_map* mc, ilsm_map* ms, const flo
   ILSM_CUDA(cudaSetDevice(c.device));
   const float *d_corner, *d_surf;
   if ((rc = stage_stacks(c, corner, nc, surf, ns, stride_bytes, &d_corner, &d_surf))) return rc;
-  Pose7 p;
-  for (int i = 0; i < 4; ++i) p.v[i] = q[i];
-  for (int i = 0; i < 3; ++i) p.v[4 + i] = t[i];
-  ILSM_CUDA(launch_pdl(set_pose_kernel, dim3(1), dim3(1), 0, c.stream, c.lm.p, p, 1, o.huber_a));
-  count_launches(1);
+  if ((rc = c.upload_pose(q, t, c.stream))) return rc;
   const bool want_knn = knn_idx != nullptr && knn_d2 != nullptr;
-  if ((rc = c.associate_dev(&mc->m, &ms->m, d_corner, nc, d_surf, ns, stride_bytes, o, want_knn))) return rc;
+  if ((rc = c.associate_dev(&mc->m, &ms->m, d_corner, nc, d_surf, ns, stride_bytes, o, want_knn)) || (rc = export_factors(c, factors)))
+    return rc;
   const int n = nc + ns;
-  if (factors && n > 0) {
-    // export through out_idx scratch (reinterpreted) to keep allocations few
-    size_t words = ((size_t)n * sizeof(ilsm_factor) + 3) / 4;
-    if ((rc = c.out_idx.reserve(words + 8))) return rc;
-    ilsm_factor* d_f = reinterpret_cast<ilsm_factor*>(c.out_idx.p);
-    if ((rc = factors_export(&c, d_f))) return rc;
-    ILSM_CUDA(cudaMemcpyAsync(factors, d_f, (size_t)n * sizeof(ilsm_factor), cudaMemcpyDeviceToHost, c.stream));
-  }
   if (want_knn && n > 0) {
     ILSM_CUDA(cudaMemcpyAsync(knn_idx, c.fac.knn_idx.p, (size_t)n * 5 * 4, cudaMemcpyDeviceToHost, c.stream));
     ILSM_CUDA(cudaMemcpyAsync(knn_d2, c.fac.knn_d2.p, (size_t)n * 5 * 4, cudaMemcpyDeviceToHost, c.stream));
@@ -572,31 +548,17 @@ ILSM_API int ilsm_odometry(ilsm_ctx* ctx, ilsm_map* last_corner, ilsm_map* last_
   if (report) memset(report, 0, sizeof(*report));
   const float *d_sharp, *d_flat;
   if ((rc = stage_stacks(c, sharp, nsh, flat, nfl, stride_bytes, &d_sharp, &d_flat))) return rc;
-  Pose7 p;
-  for (int i = 0; i < 4; ++i) p.v[i] = q[i];
-  for (int i = 0; i < 3; ++i) p.v[4 + i] = t[i];
-  ILSM_CUDA(launch_pdl(set_pose_kernel, dim3(1), dim3(1), 0, c.stream, c.lm.p, p, 1, o.huber_a));
-  count_launches(1);
-  const int n = nsh + nfl;
+  if ((rc = c.upload_pose(q, t, c.stream))) return rc;
   if (factors) {
     // association only at the given pose (parity aid): export the factor records, no solve
-    if ((rc = c.odom_associate_dev(&last_corner->m, &last_surf->m, d_sharp, nsh, d_flat, nfl, stride_bytes))) return rc;
-    if (n > 0) {
-      size_t words = ((size_t)n * sizeof(ilsm_factor) + 3) / 4;
-      if ((rc = c.out_idx.reserve(words + 8))) return rc;
-      ilsm_factor* d_f = reinterpret_cast<ilsm_factor*>(c.out_idx.p);
-      if ((rc = factors_export(&c, d_f))) return rc;
-      ILSM_CUDA(cudaMemcpyAsync(factors, d_f, (size_t)n * sizeof(ilsm_factor), cudaMemcpyDeviceToHost, c.stream));
-    }
+    if ((rc = c.odom_associate_dev(&last_corner->m, &last_surf->m, d_sharp, nsh, d_flat, nfl, stride_bytes)) ||
+        (rc = export_factors(c, factors)))
+      return rc;
     ILSM_CUDA(cudaStreamSynchronize(c.stream));
     return ILSM_OK;
   }
   if ((rc = c.odometry_dev(&last_corner->m, &last_surf->m, d_sharp, nsh, d_flat, nfl, stride_bytes, o))) return rc;
-  if ((rc = c.read_back_lm(c.stream))) return rc;
-  ILSM_CUDA(cudaStreamSynchronize(c.stream));
-  c.lm_result(q, t, report);
-  if (report) report->passes = o.outer_iterations;
-  return ILSM_OK;
+  return c.lm_finish(q, t, report, o.outer_iterations);
 }
 
 // ------------------------------------------------------------------------------------------------ front end
@@ -810,12 +772,8 @@ ILSM_API int ilsm_voxelgrid(ilsm_ctx* ctx, const float* xyzi, int n, int stride_
   int rc;
   if ((rc = c.fe.raw.reserve(bytes / 4 + 4)) || (rc = c.fe.vox_out.reserve(n + 4)) || (rc = c.fe.vox_n.reserve(4))) return rc;
   ILSM_CUDA(cudaMemcpyAsync(c.fe.raw.p, xyzi, bytes, cudaMemcpyHostToDevice, c.stream));
-  const int ioff = stride_bytes >= 32 ? 4 : 3;
-  if (n <= 16384)  // one block sorts in shared memory; larger clouds take the tiled multi-block path
-    rc = c.voxelgrid_dev(c.fe.raw.p, n, nullptr, 0, stride_bytes, ioff, leaf, c.fe.vox_out.p, c.fe.vox_n.p);
-  else
-    rc = c.voxelgrid_large_dev(c.fe.raw.p, n, stride_bytes, ioff, leaf, c.fe.vox_out.p, c.fe.vox_n.p);
-  if (rc) return rc;
+  const Ctx::VgCloud vc = {c.fe.raw.p, n, leaf, c.fe.vox_out.p, c.fe.vox_n.p};
+  if ((rc = c.voxelgrid(&vc, 1, stride_bytes, intensity_word(stride_bytes), c.stream))) return rc;
   int* pin = reinterpret_cast<int*>(c.pinned.p);
   ILSM_CUDA(cudaMemcpyAsync(pin, c.fe.vox_n.p, sizeof(int), cudaMemcpyDeviceToHost, c.stream));
   ILSM_CUDA(cudaStreamSynchronize(c.stream));
@@ -956,17 +914,11 @@ ILSM_API int ilsm_eval_normal_eq(ilsm_ctx* ctx, const double q[4], const double 
   Ctx& c = ctx->c;
   std::lock_guard<std::mutex> lk(c.mu);
   ILSM_CUDA(cudaSetDevice(c.device));
-  Pose7 p;
-  for (int i = 0; i < 4; ++i) p.v[i] = q[i];
-  for (int i = 0; i < 3; ++i) p.v[4 + i] = t[i];
-  ILSM_CUDA(launch_pdl(set_pose_kernel, dim3(1), dim3(1), 0, c.stream, c.lm.p, p, 1, huber_a));
-  count_launches(1);
   int rc;
-  if ((rc = c.partials.reserve(64))) return rc;
-  // eval_out lives at the tail of the partials buffer? keep it simple: dedicated 32 doubles in out_d2 scratch
-  if ((rc = c.out_d2.reserve(128))) return rc;
+  // the pose is evaluated where upload_pose leaves it (xq, xt: 7 contiguous doubles); the 32 sums go to out_d2 scratch
+  if ((rc = c.upload_pose(q, t, c.stream)) || (rc = c.out_d2.reserve(128))) return rc;
   double* d_out = reinterpret_cast<double*>(c.out_d2.p);
-  if ((rc = eval_only_launch(&c, d_out))) return rc;
+  if ((rc = eval_only_launch(&c, d_out, c.lm.p->xq, huber_a))) return rc;
   double* pin = reinterpret_cast<double*>(c.pinned.p);
   ILSM_CUDA(cudaMemcpyAsync(pin, d_out, 32 * sizeof(double), cudaMemcpyDeviceToHost, c.stream));
   ILSM_CUDA(cudaStreamSynchronize(c.stream));
@@ -998,8 +950,10 @@ ILSM_API int ilsm_solve_dev(ilsm_ctx* ctx, const double* d_pose7_in, int max_num
   std::lock_guard<std::mutex> lk(c.mu);
   ILSM_CUDA(cudaSetDevice(c.device));
   if (d_pose7_in) {
-    ILSM_CUDA(launch_pdl(pose_io_kernel, dim3(1), dim3(32), 0, c.stream, c.lm.p, const_cast<double*>(d_pose7_in), (ilsm_reg_report*)nullptr, 0));
-    count_launches(1);
+    PoseSrc src;
+    src.mode = 2, src.dptr = d_pose7_in;
+    int rc = c.seed_pose(src);
+    if (rc) return rc;
   }
   return c.solve_launch(max_num_iterations, huber_a, 0);
 }
@@ -1012,17 +966,10 @@ ILSM_API int ilsm_solve(ilsm_ctx* ctx, double q[4], double t[3], int max_num_ite
   Ctx& c = ctx->c;
   std::lock_guard<std::mutex> lk(c.mu);
   ILSM_CUDA(cudaSetDevice(c.device));
-  Pose7 p;
-  for (int i = 0; i < 4; ++i) p.v[i] = q[i];
-  for (int i = 0; i < 3; ++i) p.v[4 + i] = t[i];
-  ILSM_CUDA(launch_pdl(set_pose_kernel, dim3(1), dim3(1), 0, c.stream, c.lm.p, p, 0, 0.0));
-  count_launches(1);
   int rc;
-  if ((rc = c.solve_launch(max_num_iterations, huber_a, 0))) return rc;
-  if ((rc = c.read_back_lm(c.stream))) return rc;
-  ILSM_CUDA(cudaStreamSynchronize(c.stream));
   ilsm_reg_report rep;
-  c.lm_result(q, t, &rep);
+  if ((rc = c.upload_pose(q, t, c.stream)) || (rc = c.solve_launch(max_num_iterations, huber_a, 0)) || (rc = c.lm_finish(q, t, &rep, 1)))
+    return rc;
   if (summary) *summary = rep.pass[0];
   return ILSM_OK;
 }

@@ -396,11 +396,9 @@ int cubemap_frame_enqueue(CubeMapH& m, const float* d_c, int nc, const float* d_
   // device; the full-loop pipeline has already produced them on its side stream (stacks_ready)
   if (!stacks_ready) {
     if ((rc = m.stack_c.reserve(nc + 4)) || (rc = m.stack_s.reserve(ns + 4))) return rc;
-    const int ioff = stride_bytes >= 32 ? 4 : 3;
     ILSM_CUDA(cudaMemsetAsync(m.stack_n.p, 0, 4 * sizeof(int), c.stream));
-    if ((rc = c.voxelgrid_pair_dev(d_c, nc, m.line_res, m.stack_c.p, d_s, ns, m.plane_res, m.stack_s.p, stride_bytes, ioff,
-                                   m.stack_n.p, c.stream, m.err)))
-      return rc;
+    const Ctx::VgCloud vc[2] = {{d_c, nc, m.line_res, m.stack_c.p, m.stack_n.p}, {d_s, ns, m.plane_res, m.stack_s.p, m.stack_n.p + 1}};
+    if ((rc = c.voxelgrid(vc, 2, stride_bytes, intensity_word(stride_bytes), c.stream, m.err))) return rc;
   }
   // pose in
   const double qw4[4] = {qw.x, qw.y, qw.z, qw.w};
@@ -546,7 +544,7 @@ __global__ void pack_xyzi_kernel(const float* __restrict__ in, int n, int stride
 ILSM_API int ilsm_cubemap_insert_world(ilsm_cubemap* cm, const float* corner, int nc, const float* surf, int ns, int stride_bytes,
                                        const double centre[3]) {
   if (!cm || !centre || (nc > 0 && !corner) || (ns > 0 && !surf)) return fail(ILSM_ERR_INVALID_ARG, "cubemap_insert_world: null argument");
-  if (nc < 0 || ns < 0 || stride_bytes < 12 || stride_bytes % 4) return fail(ILSM_ERR_INVALID_ARG, "cubemap_insert_world: bad n/stride");
+  if (nc < 0 || ns < 0 || !valid_stride(stride_bytes)) return fail(ILSM_ERR_INVALID_ARG, "cubemap_insert_world: bad n/stride");
   CubeMapH& m = cm->m;
   Ctx& c = *m.ctx;
   std::lock_guard<std::mutex> lk(c.mu);
@@ -587,7 +585,7 @@ ILSM_API int ilsm_cubemap_frame(ilsm_cubemap* cm, const float* corner_last, int 
                                 const ilsm_reg_opts* opts, ilsm_reg_report* report, ilsm_cubemap_stats* stats) {
   if (!cm || !q_wodom || !t_wodom || !q_w || !t_w || (nc > 0 && !corner_last) || (ns > 0 && !surf_last))
     return fail(ILSM_ERR_INVALID_ARG, "cubemap_frame: null argument");
-  if (nc < 0 || ns < 0 || stride_bytes < 16 || stride_bytes % 4 || nc >= (1 << 24) || ns >= (1 << 24))
+  if (nc < 0 || ns < 0 || !valid_stride(stride_bytes) || stride_bytes < 16 || nc >= (1 << 24) || ns >= (1 << 24))
     return fail(ILSM_ERR_INVALID_ARG, "cubemap_frame: bad n/stride (fewer than 2^24 points per feature cloud)");
   CubeMapH& m = cm->m;
   Ctx& c = *m.ctx;

@@ -422,7 +422,7 @@ extern "C" {
 ILSM_API int ilsm_ground_extract(ilsm_ground* g, const float* xyz, int n, int stride_bytes, const ilsm_ground_opts* opts,
                                  float* out_xyz, int capacity, int* n_out, float coeff_abcd[4], ilsm_ground_info* info) {
   if (!g || !n_out || (n > 0 && !xyz)) return fail(ILSM_ERR_INVALID_ARG, "ground_extract: null argument");
-  if (n < 0 || stride_bytes < 12 || stride_bytes % 4) return fail(ILSM_ERR_INVALID_ARG, "ground_extract: bad n/stride");
+  if (n < 0 || !valid_stride(stride_bytes)) return fail(ILSM_ERR_INVALID_ARG, "ground_extract: bad n/stride");
   ilsm_ground_opts o;
   if (opts) o = *opts; else ilsm_ground_opts_default(&o);
   if (o.max_iterations < 1 || o.max_iterations > 62) return fail(ILSM_ERR_INVALID_ARG, "ground_extract: max_iterations must be in [1, 62]");

@@ -362,7 +362,7 @@ static int icp_check(ilsm_ctx* ctx, ilsm_map* const* targets, int n_pairs, const
   if (n_pairs == 0) return ILSM_OK;
   if (!targets || !offs || !results)
     return snprintf(msg, sizeof(msg), "%s: null targets / offsets / results", who), fail(ILSM_ERR_INVALID_ARG, msg);
-  if (stride_bytes < 12 || (stride_bytes % 4) != 0)
+  if (!valid_stride(stride_bytes))
     return snprintf(msg, sizeof(msg), "%s: bad stride", who), fail(ILSM_ERR_INVALID_ARG, msg);
   if (opts && opts->max_iterations < 0)
     return snprintf(msg, sizeof(msg), "%s: max_iterations < 0", who), fail(ILSM_ERR_INVALID_ARG, msg);

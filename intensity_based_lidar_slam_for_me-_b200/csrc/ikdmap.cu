@@ -227,7 +227,7 @@ __global__ void compact_points_kernel(const float4* __restrict__ old_pts, int n_
 
 // Add_Points(points, downsample_on): policy 1 = nearest-to-centre per `ds` voxel, 0 = plain append
 int Map::insert_dev(const float* d_src, int n_new, int stride_bytes, int policy, float ds) {
-  if (n_new < 0 || (stride_bytes % 4) != 0 || stride_bytes < 12) return fail(ILSM_ERR_INVALID_ARG, "map_insert: bad n/stride");
+  if (n_new < 0 || !valid_stride(stride_bytes)) return fail(ILSM_ERR_INVALID_ARG, "map_insert: bad n/stride");
   if (policy == 1 && !(ds > 0.f)) return fail(ILSM_ERR_INVALID_ARG, "map_insert: downsample size must be positive");
   if (n_new == 0) return ILSM_OK;
   const int n_old = n;

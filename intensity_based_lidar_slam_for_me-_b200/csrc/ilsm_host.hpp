@@ -21,6 +21,11 @@ int fail_cuda(cudaError_t e, const char* where);
 int check_launch(const char* where);
 void count_launches(int k);
 
+// A point stride the entry points accept: x, y, z as floats on 4-byte boundaries.
+inline bool valid_stride(int stride_bytes) { return stride_bytes >= 12 && (stride_bytes % 4) == 0; }
+// Float index of a point's intensity: the fifth word of a 32-byte-or-wider record (PCL's PointXYZI), else the fourth.
+inline int intensity_word(int stride_bytes) { return stride_bytes >= 32 ? 4 : 3; }
+
 #define ILSM_CUDA(call)                                        \
   do {                                                         \
     cudaError_t e__ = (call);                                  \
@@ -314,7 +319,18 @@ struct Ctx {
     for (int i = 0; i < 3; ++i) t[i] = x[4 + i];
     if (report) memcpy(report, pinned.p + offsetof(LmState, report), sizeof(*report));
   }
+  // the whole LM tail of a host-pointer entry point: read back, synchronise, then the pose and the report (`passes`:
+  // the outer passes that ran)
+  int lm_finish(double q[4], double t[3], ilsm_reg_report* report, int passes) {
+    int rc = read_back_lm(stream);
+    if (rc) return rc;
+    ILSM_CUDA(cudaStreamSynchronize(stream));
+    lm_result(q, t, report);
+    if (report) report->passes = passes;
+    return ILSM_OK;
+  }
   bool async_build = false;  // ilsm_set_async: host-pointer map builds return without synchronising
+  int seed_pose(const PoseSrc& src);  // src's pose -> lm.p->xq, xt, one 1-warp launch
   int associate_dev(Map* mc, Map* ms, const float* d_corner, int nc, const float* d_surf, int ns, int stride_bytes,
                     const ilsm_reg_opts& o, bool want_knn, const PoseSrc* src = nullptr);
   int solve_launch(int max_iter, double huber_a, int pass, const PoseDst* dst = nullptr);  // the whole LM solve, one cluster launch
@@ -331,12 +347,18 @@ struct Ctx {
   bool fe_graphs_ok = true;                 // false after a failed capture: plain launches from then on
   int pc2_unpack_dev(const unsigned char* d_data, int n, const ilsm_pc2_layout& l, float4* d_out);
   int pc2_pack_dev(const float4* d_in, int n, const ilsm_pc2_layout& l, unsigned char* d_out);
-  int voxelgrid_dev(const float* d_in, int n, const int* d_n, int n_slot, int stride_bytes, int ioff, float leaf,
-                    float4* d_out, int* d_n_out);
+  // VoxelGrid of 1 or 2 clouds on stream s; d_err: the error word the kernels OR their flags into (nullptr: the front
+  // end's)
+  struct VgCloud {
+    const float* in;
+    int n;
+    float leaf;
+    float4* out;
+    int* n_out;  // device slot of the voxel count
+  };
+  int voxelgrid(const VgCloud* clouds, int count, int stride_bytes, int ioff, cudaStream_t s, int* d_err = nullptr);
   int voxelgrid_large_dev(const float* d_in, int n, int stride_bytes, int ioff, float leaf, float4* d_out, int* d_n_out,
-                          cudaStream_t s = nullptr, int* d_err = nullptr);
-  int voxelgrid_pair_dev(const float* d_c, int nc, float leaf_c, float4* d_out_c, const float* d_s, int ns, float leaf_s,
-                         float4* d_out_s, int stride_bytes, int ioff, int* d_n_out2, cudaStream_t s, int* d_err = nullptr);
+                          cudaStream_t s, int* d_err);
   int gather_dev(const float4* d_cloud, const int* d_idx, const int* d_counts, int slot, int max_n, float4* d_out);
   int register_dev(Map* mc, Map* ms, const float* d_corner, int nc, const float* d_surf, int ns, int stride_bytes,
                    const ilsm_reg_opts& o, const PoseSrc* src = nullptr, const PoseDst* dst = nullptr);

@@ -300,7 +300,7 @@ int Map::wait_ready(cudaStream_t user) {
 // tables and alternates between them: build g fills table g & 1, which build g - 1 emptied while it scattered.
 int Map::prepare_build(const float* d_src, int n_pts, int stride_bytes, float cell_size, cudaStream_t s, void* job_out) {
   BuildJob& jb = *static_cast<BuildJob*>(job_out);
-  if (n_pts < 0 || (stride_bytes % 4) != 0 || stride_bytes < 12) return fail(ILSM_ERR_INVALID_ARG, "map_build: bad n/stride");
+  if (n_pts < 0 || !valid_stride(stride_bytes)) return fail(ILSM_ERR_INVALID_ARG, "map_build: bad n/stride");
   if (!(cell_size > 0.f)) cell_size = 1.0f;
   int want_log2 = ilog2_ceil((uint32_t)(n_pts > 0 ? 2u * (uint32_t)n_pts : 2u));
   if (want_log2 < 10) want_log2 = 10;
@@ -475,7 +475,7 @@ static int launch_knn(const GridView& g, const float* d_q, int nq, int stride_f,
 }
 
 int Map::knn_dev(const float* d_q, int nq, int stride_bytes, int k, float max_dist, int32_t* d_idx, float* d_d2) {
-  if (nq < 0 || k < 1 || k > 8 || (stride_bytes % 4) != 0 || stride_bytes < 12)
+  if (nq < 0 || k < 1 || k > 8 || !valid_stride(stride_bytes))
     return fail(ILSM_ERR_INVALID_ARG, "knn: bad nq/k/stride");
   if (table_size == 0) return fail(ILSM_ERR_STATE, "knn: map not built");
   if (nq == 0) return ILSM_OK;

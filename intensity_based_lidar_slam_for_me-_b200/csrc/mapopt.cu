@@ -5,7 +5,7 @@
 //   GroundPointOut += pc_plane ; removeNaN            :147-151                  -> pack kernel (non-finite points dropped
 //                                                                                  by the VoxelGrid / build kernels)
 //   first callback: ikdtree->Build(transformed cloud) :186-195                  -> Map::build_dev
-//   voxel_grid_(0.8).filter(GroundPointOut)           :368-370, 578             -> voxelgrid_dev / voxelgrid_large_dev
+//   voxel_grid_(0.8).filter(GroundPointOut)           :368-370, 578             -> Ctx::voxelgrid
 //   Nearest_Search(5) + plane fit + LidarPlaneNormFactor, Solve (10 it.)  :377-442  -> Ctx::register_dev (planes only)
 //   CONVERGENCE gate: transformUpdate / keyframe pose :448-457                  -> host (pose algebra)
 //   ikdtree->Add_Points(transformed cloud, true)      :471-475                  -> Map::insert_dev (0.4 m boxes)
@@ -210,9 +210,8 @@ int mapopt_frame_core(ilsm_mapopt* mo, const float* frame_xyz, int n, int stride
   // VoxelGrid(0.8) of the merged cloud; the stack size stays on the device (counts[1])
   ILSM_CUDA(cudaMemsetAsync(m.counts.p, 0, 4 * sizeof(int), s));
   if (n_all > 0) {
-    if (n_all <= 16384) rc = c.voxelgrid_dev(reinterpret_cast<const float*>(m.merged.p), n_all, nullptr, 0, 16, 3, m.leaf, m.stack.p, m.counts.p + 1);
-    else rc = c.voxelgrid_large_dev(reinterpret_cast<const float*>(m.merged.p), n_all, 16, 3, m.leaf, m.stack.p, m.counts.p + 1);
-    if (rc) return rc;
+    const Ctx::VgCloud vc = {reinterpret_cast<const float*>(m.merged.p), n_all, m.leaf, m.stack.p, m.counts.p + 1};
+    if ((rc = c.voxelgrid(&vc, 1, 16, 3, c.stream))) return rc;
   }
   // association (5-NN in the ground map, plane fit) + ceres::Solve (planes only, one pass, 10 iterations)
   const double qw4[4] = {qw.x, qw.y, qw.z, qw.w};
@@ -279,7 +278,7 @@ ILSM_API int ilsm_mapopt_frame(ilsm_mapopt* mo, const float* frame_xyz, int n, i
                                double t_w[3], const ilsm_ground_opts* gopts, ilsm_mapopt_stats* stats) {
   if (!mo || !q_wodom || !t_wodom || !q_w || !t_w || (n > 0 && !frame_xyz) || (n_plane > 0 && !plane_xyz))
     return fail(ILSM_ERR_INVALID_ARG, "mapopt_frame: null argument");
-  if (n < 0 || n_plane < 0 || stride_bytes < 12 || stride_bytes % 4 || plane_stride_bytes < 12 || plane_stride_bytes % 4)
+  if (n < 0 || n_plane < 0 || !valid_stride(stride_bytes) || !valid_stride(plane_stride_bytes))
     return fail(ILSM_ERR_INVALID_ARG, "mapopt_frame: bad n/stride");
   Ctx& c = *mo->m.ctx;
   std::lock_guard<std::mutex> lk(c.mu);

@@ -178,7 +178,7 @@ ILSM_API int ilsm_orb_match(ilsm_ctx* ctx, const uint8_t* cur_desc, int n_cur, c
 ILSM_API int ilsm_align_points(ilsm_ctx* ctx, const float* src_xyz, const float* dst_xyz, int n, int stride_bytes, double q[4],
                                double t[3], int max_num_iterations, double huber_a, ilsm_solve_summary* summary) {
   if (!ctx || !q || !t || (n > 0 && (!src_xyz || !dst_xyz))) return fail(ILSM_ERR_INVALID_ARG, "align_points: null argument");
-  if (n < 0 || stride_bytes < 12 || stride_bytes % 4) return fail(ILSM_ERR_INVALID_ARG, "align_points: bad n/stride");
+  if (n < 0 || !valid_stride(stride_bytes)) return fail(ILSM_ERR_INVALID_ARG, "align_points: bad n/stride");
   if (max_num_iterations < 0) max_num_iterations = 0;
   if (max_num_iterations > 200) max_num_iterations = 200;
   Ctx& c = ctx->c;
@@ -199,11 +199,9 @@ ILSM_API int ilsm_align_points(ilsm_ctx* ctx, const float* src_xyz, const float*
     ILSM_CUDA(launch_pdl(align_factors_kernel, dim3((n + 255) / 256), dim3(256), 0, c.stream, d_src, d_dst, n, stride_bytes / 4, f.type.p, f.p.p, f.a.p, f.b.p));
     count_launches(1);
   }
-  if ((rc = c.upload_pose(q, t, c.stream)) || (rc = c.solve_launch(max_num_iterations, huber_a, 0)) || (rc = c.read_back_lm(c.stream)))
-    return rc;
-  ILSM_CUDA(cudaStreamSynchronize(c.stream));
   ilsm_reg_report rep;
-  c.lm_result(q, t, &rep);
+  if ((rc = c.upload_pose(q, t, c.stream)) || (rc = c.solve_launch(max_num_iterations, huber_a, 0)) || (rc = c.lm_finish(q, t, &rep, 1)))
+    return rc;
   if (summary) *summary = rep.pass[0];
   return ILSM_OK;
 }

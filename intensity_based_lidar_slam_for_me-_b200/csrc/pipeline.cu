@@ -203,10 +203,9 @@ static int stack_voxelgrid(Ctx& c, const CubeMapH& cm, const SlamH::FeSlot& o, c
   ILSM_CUDA(cudaStreamWaitEvent(c.aux, o.ev, 0));
   if (set.free_recorded) ILSM_CUDA(cudaStreamWaitEvent(c.aux, set.ev_free, 0));  // frame - 2's insertion read this set
   ILSM_CUDA(cudaMemsetAsync(set.n.p, 0, 4 * sizeof(int), c.aux));
-  if ((rc = c.voxelgrid_pair_dev(reinterpret_cast<const float*>(o.lsharp.p), n_lsharp, cm.line_res, set.c.p,
-                                 reinterpret_cast<const float*>(o.lf), n_lflat, cm.plane_res, set.s.p, 16, 3, set.n.p, c.aux,
-                                 cm.err)))
-    return rc;
+  const Ctx::VgCloud vc[2] = {{reinterpret_cast<const float*>(o.lsharp.p), n_lsharp, cm.line_res, set.c.p, set.n.p},
+                              {reinterpret_cast<const float*>(o.lf), n_lflat, cm.plane_res, set.s.p, set.n.p + 1}};
+  if ((rc = c.voxelgrid(vc, 2, 16, 3, c.aux, cm.err))) return rc;
   ILSM_CUDA(cudaEventRecord(set.ev_ready, c.aux));
   return ILSM_OK;
 }
@@ -596,7 +595,7 @@ extern "C" {
 
 ILSM_API int ilsm_slam_frame(ilsm_slam* slam, const float* xyzi, int n, int stride_bytes, int use_aloam, double q_odom[4],
                              double t_odom[3], double q_map[4], double t_map[3], ilsm_slam_stats* stats) {
-  if (n < 0 || stride_bytes < 12 || stride_bytes % 4) return fail(ILSM_ERR_INVALID_ARG, "slam_frame: bad n/stride");
+  if (n < 0 || !valid_stride(stride_bytes)) return fail(ILSM_ERR_INVALID_ARG, "slam_frame: bad n/stride");
   return slam_frame_impl(slam, xyzi, n, stride_bytes, nullptr, use_aloam, q_odom, t_odom, q_map, t_map, stats);
 }
 
@@ -612,7 +611,7 @@ ILSM_API int ilsm_slam_frame_pc2(ilsm_slam* slam, const uint8_t* data, int n_poi
 ILSM_API int ilsm_slam_frame_async(ilsm_slam* slam, const float* xyzi, int n, int stride_bytes, int use_aloam, double q_odom[4],
                                    double t_odom[3], double q_map_prev[4], double t_map_prev[3], int* have_prev,
                                    ilsm_slam_stats* stats) {
-  if (n < 0 || stride_bytes < 12 || stride_bytes % 4) return fail(ILSM_ERR_INVALID_ARG, "slam_frame_async: bad n/stride");
+  if (n < 0 || !valid_stride(stride_bytes)) return fail(ILSM_ERR_INVALID_ARG, "slam_frame_async: bad n/stride");
   if (!have_prev) return fail(ILSM_ERR_INVALID_ARG, "slam_frame_async: null have_prev");
   return slam_frame_impl(slam, xyzi, n, stride_bytes, nullptr, use_aloam, q_odom, t_odom, q_map_prev, t_map_prev, stats, have_prev);
 }
@@ -711,7 +710,7 @@ extern "C" ILSM_API int ilsm_slam_frame_staged(ilsm_slam* slam, const float* xyz
                                                double t_map[3], int* map_frame, ilsm_slam_stats* stats) {
   if (!slam || (n > 0 && !xyzi) || !q_odom || !t_odom || !q_map || !t_map || !odom_frame || !map_frame)
     return fail(ILSM_ERR_INVALID_ARG, "slam_frame_staged: null argument");
-  if (n >= 0 && (stride_bytes < 12 || stride_bytes % 4)) return fail(ILSM_ERR_INVALID_ARG, "slam_frame_staged: bad stride");
+  if (n >= 0 && !valid_stride(stride_bytes)) return fail(ILSM_ERR_INVALID_ARG, "slam_frame_staged: bad stride");
   SlamH& s = slam->s;
   if (!s.staged) return fail(ILSM_ERR_STATE, "slam_frame_staged: not an ilsm_slam_create_staged handle");
   *odom_frame = *map_frame = -1;

@@ -1117,7 +1117,7 @@ __global__ void __cluster_dims__(kCS, 1, 1) __launch_bounds__(kThr, 1)
 constexpr int kEvalThreads = 384, kEvalBlocksPerSm = 1;
 
 __global__ void __launch_bounds__(kEvalThreads, kEvalBlocksPerSm)
-    normal_eq_kernel(FactorView fv, int n, LmState* st, const double* __restrict__ pose7, double huber_in,
+    normal_eq_kernel(FactorView fv, int n, LmState* st, const double* __restrict__ pose7, double huber_a,
                      double* __restrict__ partials, double* __restrict__ eval_out) {
   pdl_entry();
   __shared__ double red[kEvalThreads / 32][kSumStride];
@@ -1125,12 +1125,8 @@ __global__ void __launch_bounds__(kEvalThreads, kEvalBlocksPerSm)
   double acc[kSumStride];
 #pragma unroll
   for (int i = 0; i < kSumStride; ++i) acc[i] = 0.0;
-  // pose from the caller's device buffer when given, else the candidate pose of the LM state
-  const double* pq = pose7 ? pose7 : st->cq;
-  const double* pt = pose7 ? pose7 + 4 : st->ct;
-  const double q[4] = {pq[0], pq[1], pq[2], pq[3]};
-  const double t[3] = {pt[0], pt[1], pt[2]};
-  const double huber_a = pose7 ? huber_in : st->huber_a;
+  const double q[4] = {pose7[0], pose7[1], pose7[2], pose7[3]};
+  const double t[3] = {pose7[4], pose7[5], pose7[6]};
   // persistent grid-stride loop: the 32 running sums stay in registers across factors, so the reduction cost is paid
   // once per thread; the next factor's record is in flight while the current one is evaluated.  Only the bytes a
   // factor type needs are read: type 0 (gate / fit failed) 4 B, plane 52 B, edge 84 B.
@@ -1219,7 +1215,7 @@ constexpr size_t kBulkSmemBytes = (size_t)kBulkStages * kBulkStageBytes + 2 * kB
 // 12 warps and not 13: registers are allocated per SM sub-partition (4 x 16 K), so a 13th warp would cap the kernel at
 // 128 registers per thread (spills in the tile loop).
 __global__ void __launch_bounds__(kBulkThreads, 1)
-    normal_eq_bulk_kernel(FactorView fv, int n, int nc, LmState* st, const double* __restrict__ pose7, double huber_in,
+    normal_eq_bulk_kernel(FactorView fv, int n, int nc, LmState* st, const double* __restrict__ pose7, double huber_a,
                           double* __restrict__ partials, double* __restrict__ eval_out) {
   pdl_entry();
   extern __shared__ __align__(128) unsigned char bulk_smem[];
@@ -1264,12 +1260,9 @@ __global__ void __launch_bounds__(kBulkThreads, 1)
       }
     }
   } else {
-    // ---- consumers (pose from the caller's device buffer when given, else the candidate pose of the LM state)
-    const double* pq = pose7 ? pose7 : st->cq;
-    const double* pt = pose7 ? pose7 + 4 : st->ct;
-    const double q[4] = {pq[0], pq[1], pq[2], pq[3]};
-    const double t[3] = {pt[0], pt[1], pt[2]};
-    const double huber_a = pose7 ? huber_in : st->huber_a;
+    // ---- consumers
+    const double q[4] = {pose7[0], pose7[1], pose7[2], pose7[3]};
+    const double t[3] = {pose7[4], pose7[5], pose7[6]};
     // Eigen::Quaterniond::toRotationMatrix of the pose, once per thread (the pose is constant for the launch)
     const double tx = 2.0 * q[0], ty2 = 2.0 * q[1], tz = 2.0 * q[2];
     const double twx = tx * q[3], twy = ty2 * q[3], twz = tz * q[3], txx = tx * q[0], txy = ty2 * q[0], txz = tz * q[0];
@@ -1349,11 +1342,17 @@ static FactorView factor_view(FactorBufs& f, bool want_knn) {
   return v;
 }
 
-// empty stacks: nothing to associate, but a pose handed in with the launch must still reach the LM state
+// the pose of `src` into the LM state without an association launch to carry it (empty stacks, ilsm_solve_dev)
 __global__ void pose_seed_kernel(LmState* st, PoseSrc src) {
   pdl_entry();
   const double* p7 = src.mode == 2 ? src.dptr : src.v;
   if (threadIdx.x < 7) st->xq[threadIdx.x] = p7[threadIdx.x];
+}
+
+int Ctx::seed_pose(const PoseSrc& src) {
+  ILSM_CUDA(launch_pdl(pose_seed_kernel, dim3(1), dim3(32), 0, stream, lm.p, src));
+  count_launches(1);
+  return check_launch("pose_seed");
 }
 
 int Ctx::associate_dev(Map* mc, Map* ms, const float* d_corner, int nc, const float* d_surf, int ns, int stride_bytes,
@@ -1368,12 +1367,7 @@ int Ctx::associate_dev(Map* mc, Map* ms, const float* d_corner, int nc, const fl
   fac.n = n;
   fac.nc = nc;
   const PoseSrc ps = src ? *src : PoseSrc();
-  if (n == 0) {
-    if (ps.mode == 0) return ILSM_OK;
-    ILSM_CUDA(launch_pdl(pose_seed_kernel, dim3(1), dim3(32), 0, stream, lm.p, ps));
-    count_launches(1);
-    return check_launch("pose_seed");
-  }
+  if (n == 0) return ps.mode == 0 ? ILSM_OK : seed_pose(ps);
   if ((rc = mc->wait_ready(stream)) || (rc = ms->wait_ready(stream))) return rc;
   AssocParams prm;
   prm.gate_sq = o.knn_gate_sq;
@@ -1461,8 +1455,8 @@ int Ctx::register_dev(Map* mc, Map* ms, const float* d_corner, int nc, const flo
   return ILSM_OK;
 }
 
-// stand-alone evaluation (ilsm_eval_normal_eq): pose and Huber width from d_pose7 / huber_a, or (d_pose7 == nullptr)
-// the candidate pose lm->cq/ct and lm->huber_a
+// stand-alone evaluation (ilsm_eval_normal_eq[_dev]) at the 7 doubles d_pose7 (q then t, on the device) with Huber
+// width huber_a
 int eval_only_launch(Ctx* c, double* d_out, const double* d_pose7, double huber_a) {
   // bandwidth regime (at least one 352-factor tile per SM): the bulk-copy staged kernel, one persistent CTA per SM
   const long long ntiles = ((long long)c->fac.n + kBulkTile - 1) / kBulkTile;

@@ -94,10 +94,11 @@ def test_voxelgrid_bit_exact(ctx, oracle_mod, cfg_full, leaf):
     assert np.array_equal(ctx.voxelgrid(one, leaf), one)
 
 
-@pytest.mark.parametrize("n,leaf", [(16385, 0.4), (40000, 0.8), (65536, 0.2), (150000, 0.4)])
+@pytest.mark.parametrize("n,leaf", [(2049, 0.2), (16384, 0.4), (16385, 0.4), (40000, 0.8), (65536, 0.2), (150000, 0.4)])
 def test_voxelgrid_large_clouds_bit_exact(ctx, oracle_mod, ilsm, cfg_full, n, leaf):
     """More than 16384 points (mapOptimization filters ground + less-flat clouds of ~40k points, mapOptimization.cpp:
-    368-370): the tiled multi-block sort path gives the same voxels, order and float centroids as the oracle."""
+    368-370): the tiled multi-block sort path gives the same voxels, order and float centroids as the oracle.  2049 (the
+    first hash-based size) and 16384 (the largest single block) are the block path's boundaries."""
     rng = np.random.default_rng(n)
     base = cfg_full["map_surf"]
     pts = np.zeros((n, 4), np.float32)
