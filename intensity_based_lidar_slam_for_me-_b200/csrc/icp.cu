@@ -192,7 +192,9 @@ __device__ void icp_tile(const IcpPair& pp, const IcpParams& prm, const int (&bb
       nd2 = cand_d2(res.key[0]), nx = res.x[0], ny = res.y[0], nz = res.z[0];
     }
   }
-  const bool ok = found && (double)nd2 <= (fit ? prm.fit_range : prm.max_corr2);
+  // a transformed point with a non-finite coordinate (NaN / Inf input, or a float store that overflows) never takes
+  // part, whatever the gate: its d2 is NaN or +inf, and +inf would pass an infinite gate
+  const bool ok = found && isfinite(px) && isfinite(py) && isfinite(pz) && (double)nd2 <= (fit ? prm.fit_range : prm.max_corr2);
   double c[kIcpSums];
 #pragma unroll
   for (int k = 0; k < kIcpSums; ++k) c[k] = 0.0;

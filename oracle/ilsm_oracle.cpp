@@ -102,6 +102,7 @@ struct TopK {
 };
 
 inline const float* pt(const float* base, int stride_f, int i) { return base + (size_t)i * stride_f; }
+inline bool finite3(const float* p) { return std::isfinite(p[0]) && std::isfinite(p[1]) && std::isfinite(p[2]); }
 
 // Exact k-d tree (own implementation; median split on widest axis).  Pruning uses only the single-axis
 // bound fl((q-split)^2) which is <= the float distance of every point behind the split plane because
@@ -194,12 +195,16 @@ struct KdTree {
     nodes[me].right = r;
     return me;
   }
+  // A point with a non-finite coordinate is left out, as the library's map build leaves it out (mapOptimization.cpp:151
+  // strips such points before the tree is built); a NaN would otherwise break the median split and, offered first to a
+  // search, hold the result slot.
   void build(const float* b, int n_, int stride_f_) {
     base = b;
-    n = n_;
     stride_f = stride_f_;
-    ids.resize(n);
-    std::iota(ids.begin(), ids.end(), 0);
+    ids.clear();
+    for (int i = 0; i < n_; ++i)
+      if (finite3(pt(b, stride_f, i))) ids.push_back(i);
+    n = (int)ids.size();
     nodes.clear();
     nodes.reserve(2 * (n / LEAF + 2));
     if (n > 0) build_rec(0, n);
@@ -760,7 +765,8 @@ ORC_API void orc_knn_brute(const float* map, int n, int map_stride_bytes, const 
   for (int i = 0; i < nq; ++i) {
     TopK top(k);
     const float* qq = pt(q, qs, i);
-    for (int j = 0; j < n; ++j) top.offer(dist2f(qq, pt(map, ms, j)), j);
+    for (int j = 0; j < n; ++j)
+      if (finite3(pt(map, ms, j))) top.offer(dist2f(qq, pt(map, ms, j)), j);
     for (int j = 0; j < k; ++j) {
       idx[(size_t)i * k + j] = j < top.n ? top.c[j].i : -1;
       d2[(size_t)i * k + j] = j < top.n ? top.c[j].d : INFINITY;

@@ -25,7 +25,8 @@
 // Declared deviations from PCL (DESIGN section 2): P is kept in fp64 and applied to the original points (PCL composes a
 // Matrix4f and re-transforms the already transformed cloud); the sums are fp64 in a fixed order; the rotation is Horn's
 // closed form (largest eigenvector of the 4x4 quaternion matrix, cyclic Jacobi in fp64) instead of Eigen's float JacobiSVD;
-// correspondence ties are broken by (d2, index).
+// correspondence ties are broken by (d2, index); a point with a non-finite coordinate never takes part (a target point
+// is left out of the tree, a transformed source point has no correspondence and no fitness term).
 //
 // The fixed order, the same as the kernel's (csrc/icp.cu): the per-point terms count, d2, p - o, q - o, (p - o)(q - o)^T,
 // with o the guess translation, are summed per 256-point tile as a lane-pair butterfly over each 32-point group followed
@@ -143,10 +144,13 @@ void pass_sums(Pass& ps, const double q[4], const double t[3], const double o[3]
         double* c = lane[l];
         for (int k = 0; k < kSums; ++k) c[k] = 0.0;
         const int i = tile * kTile + g * kGroup + l;
-        if (i >= n || ps.idx[i] < 0 || !((double)ps.d2[i] <= gate)) continue;
+        if (i >= n) continue;
+        const float* p = &ps.moved[3 * (size_t)i];
+        // a transformed point with a non-finite coordinate never takes part, whatever the gate (even +inf)
+        if (!std::isfinite(p[0]) || !std::isfinite(p[1]) || !std::isfinite(p[2])) continue;
+        if (ps.idx[i] < 0 || !((double)ps.d2[i] <= gate)) continue;
         c[0] = 1.0, c[1] = (double)ps.d2[i];
         if (nsum == 2) continue;
-        const float* p = &ps.moved[3 * (size_t)i];
         const float* r = ps.tgt + (size_t)ps.idx[i] * ps.tstride_f;
         const double dp[3] = {(double)p[0] - o[0], (double)p[1] - o[1], (double)p[2] - o[2]};
         const double dq[3] = {(double)r[0] - o[0], (double)r[1] - o[1], (double)r[2] - o[2]};

@@ -1,4 +1,4 @@
-"""K6 ICP loop verification on the GPU (ilsm_icp_align_batch): against the oracle, batch == singles bit for bit,
+"""K6 ICP loop verification on the GPU (ilsm_icp_align_batch): equal to the oracle byte for byte, batch == singles,
 determinism across runs and cluster sizes, one launch per call, stress paths, the end-to-end loop check in the box scene,
 and teardown."""
 import os
@@ -37,7 +37,7 @@ def rot_angle(q1, q2):
 def test_gpu_matches_oracle(ilsm, icp_oracle, ctx, loop):
     kfs, n = loop
     S = ilsm.synth
-    worst = [0.0, 0.0, 0.0]
+    worst, mismatches = [0.0, 0.0, 0.0], 0
     for c in (0, 4, 9):
         tg = S.loop_submap(kfs, c, n)
         m = ctx.new_map().set_input_cloud(tg, 1.0)
@@ -52,9 +52,12 @@ def test_gpu_matches_oracle(ilsm, icp_oracle, ctx, loop):
                 worst[0] = max(worst[0], float(np.abs(g.tv - w.tv).max()))
                 worst[1] = max(worst[1], rot_angle(g.q, w.q))
                 worst[2] = max(worst[2], abs(g.fitness - w.fitness) / max(abs(w.fitness), 1e-300))
+                mismatches += bytes(g) != bytes(w)
         m.close()
-    print(f"GPU vs oracle: max |dt| {worst[0]:.3e} m, max rotation {worst[1]:.3e} rad, max fitness rel {worst[2]:.3e}")
-    assert worst[0] <= 1e-6 and worst[1] <= 1e-6 and worst[2] <= 1e-6
+    print(f"GPU vs oracle: {mismatches} results not byte-equal; max |dt| {worst[0]:.3e} m, max rotation {worst[1]:.3e} rad, "
+          f"max fitness rel {worst[2]:.3e}")
+    # the kernel and the oracle share every arithmetic step (DESIGN section 2): equal bytes, not a tolerance
+    assert mismatches == 0
 
 
 def test_batch_equals_singles_bit_for_bit(ilsm, ctx, loop):
@@ -126,8 +129,7 @@ def test_stress_large_source_and_outside_box(ilsm, icp_oracle, ctx, loop, gated)
         g = ctx.icp_align(m, src, q0, t0, **opts)
         w = icp_oracle.icp_align(tg, src, q0, t0, **opts)
         assert (g.iterations, g.state, g.converged, g.n_correspondences) == (w.iterations, w.state, w.converged, w.n_correspondences)
-        assert np.abs(g.tv - w.tv).max() <= 1e-6 and rot_angle(g.q, w.q) <= 1e-6
-        assert abs(g.fitness - w.fitness) <= 1e-6 * abs(w.fitness)
+        assert bytes(g) == bytes(w), (g.tv, w.tv, g.q, w.q, g.fitness, w.fitness)
     m.close()
 
 

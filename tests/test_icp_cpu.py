@@ -1,6 +1,6 @@
 """K6 ICP loop verification without a GPU: the oracle (oracle/ilsm_oracle_icp.cpp) against an independent numpy
-restatement of pcl::IterativeClosestPoint (float32 brute-force 1-NN, Kabsch by SVD, the state machine in Python), one
-case per terminal state; ground-truth recovery; the ABI surface (struct layouts, argument errors)."""
+restatement of pcl::IterativeClosestPoint (exact float32 1-NN, Kabsch by SVD, the state machine in Python), one
+case per terminal state; non-finite points; ground-truth recovery; the ABI surface (struct layouts, argument errors)."""
 import ctypes as C
 import os
 import subprocess
@@ -41,12 +41,45 @@ def rotate(q, v):
     return (v + q[3] * uv) + np.cross(np.broadcast_to(u, v.shape), uv)
 
 
+def transform(q, t, v):
+    """pointAssociateToMap: double math, float store (a non-finite point stays non-finite)."""
+    with np.errstate(invalid="ignore", over="ignore"):
+        return (rotate(q, v) + t).astype(np.float32)
+
+
+def flann_d2(a, b):
+    """The 1-NN distance expression of FLANN's L2_Simple in float32, ((dx*dx)+(dy*dy))+(dz*dz), row by row."""
+    with np.errstate(invalid="ignore", over="ignore"):
+        d = [a[:, k] - b[:, k] for k in range(3)]
+        return (d[0] * d[0] + d[1] * d[1]) + d[2] * d[2]
+
+
 def nn1(target, moved):
-    """Exact 1-NN in float32, ((dx*dx)+(dy*dy))+(dz*dz); ties by (d2, index)."""
-    d = [(moved[:, None, a] - target[None, :, a]) for a in range(3)]
-    d2 = (d[0] * d[0] + d[1] * d[1]) + d[2] * d[2]
-    j = np.lexsort((np.broadcast_to(np.arange(len(target)), d2.shape), d2), axis=1)[:, 0] if len(target) else None
-    return j, d2[np.arange(len(moved)), j]
+    """Exact 1-NN under flann_d2, ties by (d2, index).  A fp64 k-d tree (scipy's cKDTree) gives each query its exact
+    nearest distance dmin; every target point within dmin (1 + 1e-5) is a candidate (the float expression is within a
+    few 1e-7 of the exact squared distance), and the candidates are ranked by (float d2, index).  A point with a
+    non-finite coordinate, target or query, never takes part: j = -1 and d2 = inf where no target point does."""
+    from scipy.spatial import cKDTree
+    T = np.asarray(target, np.float32)[:, :3]
+    live = np.flatnonzero(np.isfinite(T).all(axis=1))
+    T = T[live]
+    j = np.full(len(moved), -1, np.int64)
+    d2 = np.full(len(moved), np.inf, np.float32)
+    qs = np.flatnonzero(np.isfinite(moved).all(axis=1))
+    if not len(T) or not len(qs):
+        return j, d2
+    tree = cKDTree(T.astype(np.float64))
+    q = moved[qs].astype(np.float64)
+    dmin, _ = tree.query(q, k=1)
+    cand = tree.query_ball_point(q, dmin * (1 + 1e-5) + 1e-20)
+    qi = np.repeat(np.arange(len(qs)), [len(c) for c in cand])
+    ti = np.concatenate([np.asarray(c, np.int64) for c in cand])
+    dd = flann_d2(moved[qs][qi], T[ti])
+    order = np.lexsort((ti, dd, qi))
+    first = order[np.r_[True, qi[order][1:] != qi[order][:-1]]]
+    assert len(first) == len(qs)  # every finite query has at least its exact nearest point as a candidate
+    j[qs], d2[qs] = live[ti[first]], dd[first]
+    return j, d2
 
 
 def np_icp(target, source, q, t, max_correspondence_distance=np.sqrt(FMAX), max_iterations=10, transformation_epsilon=0.0,
@@ -58,9 +91,9 @@ def np_icp(target, source, q, t, max_correspondence_distance=np.sqrt(FMAX), max_
     gate = max_correspondence_distance * max_correspondence_distance
     prev_mse, it = FMAX, 0
     while True:
-        moved = (rotate(q, S) + t).astype(np.float32)
+        moved = transform(q, t, S)
         j, d2 = nn1(T, moved)
-        keep = d2.astype(np.float64) <= gate
+        keep = (j >= 0) & (d2.astype(np.float64) <= gate)
         n = int(keep.sum())
         mse = float(np.sum(d2[keep].astype(np.float64)) / n) if n else FMAX
         if n < 3:
@@ -89,9 +122,8 @@ def np_icp(target, source, q, t, max_correspondence_distance=np.sqrt(FMAX), max_
             state = REL_MSE
             break
         prev_mse = mse
-    moved = (rotate(q, S) + t).astype(np.float32)
-    _, d2 = nn1(T, moved)
-    inr = d2.astype(np.float64) <= fitness_max_range
+    j, d2 = nn1(T, transform(q, t, S))
+    inr = (j >= 0) & (d2.astype(np.float64) <= fitness_max_range)
     fitness = float(np.sum(d2[inr].astype(np.float64)) / inr.sum()) if inr.any() else FMAX
     return dict(q=q, t=t, iterations=it, state=state, converged=state not in (NOT_CONVERGED, NO_CORRESPONDENCES),
                 n_correspondences=n, fitness=fitness, mse=mse)
@@ -177,6 +209,25 @@ def test_too_few_points_and_empty_target(icp_oracle):
         r = icp_oracle.icp_align(tgt, src, (0, 0, 0, 1), (0.5, 0, 0))
         assert (r.state, r.iterations, r.converged) == (NO_CORRESPONDENCES, 0, 0)
         assert np.array_equal(r.tv, [0.5, 0, 0])
+
+
+def test_non_finite_points_never_take_part(icp_oracle):
+    """NaN / Inf target points are left out (the result equals the run without them: the finite points keep their
+    order); a source point whose transform is non-finite has no correspondence, even with no gate and no range."""
+    T, S, _, _ = pair()
+    Tb, Sb = T.copy(), S.copy()
+    bad = np.arange(3, len(T), 41)
+    for k, i in enumerate(bad):
+        Tb[i, k % 3] = (np.nan, np.inf, -np.inf)[k % 3]
+        Sb[i + 1, (k + 1) % 3] = (np.nan, np.inf, -np.inf)[k % 3]
+    Sb[7] = np.finfo(np.float32).max  # finite, but any yaw near the true one overflows its float store
+    q0, t0 = np.array([0.0, 0.0, np.sin(0.03), np.cos(0.03)]), np.array([0.2, -0.1, 0.0])
+    for opts in (dict(max_iterations=30, transformation_epsilon=1e-8),
+                 dict(max_iterations=30, transformation_epsilon=1e-8, max_correspondence_distance=np.inf, fitness_max_range=np.inf)):
+        r = icp_oracle.icp_align(Tb, Sb, q0, t0, **opts)
+        agree(r, np_icp(Tb, Sb, q0, t0, **opts))
+        assert bytes(r) == bytes(icp_oracle.icp_align(np.delete(Tb, bad, axis=0), Sb, q0, t0, **opts))
+        assert r.converged and np.isfinite(r.fitness) and np.isfinite(r.mse)
 
 
 def test_recovers_known_transform(icp_oracle):
