@@ -17,7 +17,8 @@
  *    and run on that context's single CUDA stream (the reference runs this path on one thread,
  *    laserMapping.cpp:1215).
  *  - *_dev variants take DEVICE pointers (inputs already resident in HBM) and enqueue on the context
- *    stream without synchronising; call ilsm_sync() before reading results on the host.
+ *    stream without synchronising; call ilsm_sync() before reading results on the host.  A *_dev variant checks its
+ *    arguments as its host form does, with the same status; both return an argument error before any CUDA call.
  */
 #ifndef ILSM_H_
 #define ILSM_H_
@@ -189,7 +190,9 @@ ILSM_API int ilsm_register_dev(ilsm_ctx* ctx, ilsm_map* map_corner, ilsm_map* ma
  * guess q, t, which is overwritten with the optimised pose.  sizes_out (may be NULL) = {less-sharp points, less-flat
  * points, corner stack, surf stack}.  The feature clouds stay on the device between the stages; the call synchronises
  * once for the feature counts (they size the VoxelGrid sorts) and once for the pose.  The _dev form takes the frame and
- * the pose (7 doubles, updated in place) on the device and returns without the final synchronisation. */
+ * the pose (7 doubles, updated in place) on the device and returns without the final synchronisation.  Both forms
+ * return ILSM_ERR_STATE when a map has not been built and ILSM_ERR_NOT_ENOUGH_MAP under the map-size guard of
+ * ilsm_register (opts->min_corner_map / min_surf_map), before any launch. */
 ILSM_API int ilsm_register_frame(ilsm_ctx* ctx, ilsm_map* map_corner, ilsm_map* map_surf, const float* xyzi, int n, int stride_bytes,
                                  float min_range, float line_res, float plane_res, double q_xyzw[4], double t_xyz[3],
                                  const ilsm_reg_opts* opts, ilsm_reg_report* report, int32_t sizes_out[4]);
@@ -608,7 +611,8 @@ ILSM_API int ilsm_sc_query_candidates(ilsm_sc* sc, const float* desc_20x60, int 
 
 /* n_queries descriptors (contiguous, 1200 floats each) scored against entries [0, n_search) in one call; outputs are
  * [n_queries][k].  The _dev form takes device descriptors and writes n_queries packed records (16 k bytes each, the
- * layout of ilsm_sc_merge_topk_dev) without synchronising. */
+ * layout of ilsm_sc_merge_topk_dev) without synchronising.  Both forms take 1 <= n_queries <= 4096 and 1 <= k <= 16,
+ * else ILSM_ERR_INVALID_ARG. */
 ILSM_API int ilsm_sc_query_topk_batch(ilsm_sc* sc, const float* desc_20x60, int n_queries, int n_search, int id_offset, int k,
                                       double* dist, int32_t* id, int32_t* shift);
 ILSM_API int ilsm_sc_query_topk_batch_dev(ilsm_sc* sc, const float* d_desc_20x60, int n_queries, int n_search, int id_offset, int k,
@@ -639,6 +643,7 @@ ILSM_API int ilsm_sc_nccl_version(int* version);
  * the whole batch are exchanged with ONE ncclAllGather (n_queries x 16 k bytes per rank) and merged by the same
  * deterministic kernel on every rank (ascending (distance, id)); nothing visits the host in between.  Every rank
  * receives the global top-k.  Without a communicator (n_ranks 1) it degenerates to ilsm_sc_query_topk_batch.
+ * n_queries and k have the bounds of ilsm_sc_query_topk_batch in both forms.
  * Replaces: the candidate scoring of Scancontext.cpp:299-312 over a database split across GPUs (BASELINE configs[4]). */
 ILSM_API int ilsm_sc_query_topk_sharded(ilsm_sc* sc, const float* desc_20x60, int n_queries, int n_search, int id_offset, int k,
                                         double* dist, int32_t* id, int32_t* shift);

@@ -1,5 +1,6 @@
 // api.cu -- the C ABI (include/ilsm.h) over the kernels: handle management, staging of caller buffers, errors.
 // No CPU fallback anywhere: without a CUDA device ilsm_create fails and nothing else can be called.
+#include <stdarg.h>
 #include <stdio.h>
 #include <string.h>
 
@@ -12,8 +13,11 @@ namespace ilsm {
 
 static thread_local char g_err[512] = "";
 
-int fail(int code, const char* msg) {
-  snprintf(g_err, sizeof(g_err), "%s", msg);
+int fail(int code, const char* fmt, ...) {
+  va_list ap;
+  va_start(ap, fmt);
+  vsnprintf(g_err, sizeof(g_err), fmt, ap);
+  va_end(ap);
   return code;
 }
 int fail_cuda(cudaError_t e, const char* where) {
@@ -84,6 +88,9 @@ Map::~Map() {
   if (stream) cudaStreamDestroy(stream);
 }
 
+// the LM iteration budget the solve kernel accepts
+static int clamp_iterations(int n) { return n < 0 ? 0 : (n > 200 ? 200 : n); }
+
 static ilsm_reg_opts sanitize(const ilsm_reg_opts* o) {
   ilsm_reg_opts r;
   if (o)
@@ -92,8 +99,7 @@ static ilsm_reg_opts sanitize(const ilsm_reg_opts* o) {
     ilsm_reg_opts_default(&r);
   if (r.outer_iterations < 1) r.outer_iterations = 1;
   if (r.outer_iterations > ILSM_MAX_OUTER) r.outer_iterations = ILSM_MAX_OUTER;
-  if (r.max_num_iterations < 0) r.max_num_iterations = 0;
-  if (r.max_num_iterations > 200) r.max_num_iterations = 200;
+  r.max_num_iterations = clamp_iterations(r.max_num_iterations);
   return r;
 }
 
@@ -153,7 +159,7 @@ ILSM_API void* ilsm_stream(ilsm_ctx* ctx) { return ctx ? (void*)ctx->c.stream : 
 // profiling aid (not in include/ilsm.h): copy the 64 clock64() stamps of the last kernels to the host
 ILSM_API int ilsm_debug_stamps(ilsm_ctx* ctx, long long* out64) {
   if (!ctx || !out64) return fail(ILSM_ERR_INVALID_ARG, "null");
-  std::lock_guard<std::mutex> lk(ctx->c.mu);
+  ILSM_ENTER(ctx->c);
   ILSM_CUDA(cudaStreamSynchronize(ctx->c.stream));
   ILSM_CUDA(cudaMemcpy(out64, ctx->c.lm.p->dbg, 64 * sizeof(long long), cudaMemcpyDeviceToHost));
   return ILSM_OK;
@@ -175,16 +181,13 @@ ILSM_API int ilsm_set_async(ilsm_ctx* ctx, int on) {
 
 ILSM_API int ilsm_map_create(ilsm_ctx* ctx, ilsm_map** out) {
   if (!ctx || !out) return fail(ILSM_ERR_INVALID_ARG, "ilsm_map_create: null argument");
+  ILSM_ENTER(ctx->c);
   ilsm_map* m = new (std::nothrow) ilsm_map();
   if (!m) return fail(ILSM_ERR_OUT_OF_MEMORY, "host allocation failed");
-  {
-    std::lock_guard<std::mutex> lk(ctx->c.mu);
-    cudaSetDevice(ctx->c.device);
-    int rc = m->m.init(&ctx->c);
-    if (rc) {
-      delete m;
-      return rc;
-    }
+  int rc = m->m.init(&ctx->c);
+  if (rc) {
+    delete m;
+    return rc;
   }
   *out = m;
   return ILSM_OK;
@@ -200,39 +203,42 @@ ILSM_API void ilsm_map_destroy(ilsm_map* map) {
 
 ILSM_API int ilsm_map_size(const ilsm_map* map) { return map ? map->m.n : 0; }
 
+// the argument check of ilsm_map_build[_dev] (and, per map, of ilsm_map_build_pair_dev)
+static int check_build_args(const ilsm_map* map, const float* xyz, int n, int stride_bytes, const char* who) {
+  if (!map || (n > 0 && !xyz)) return fail(ILSM_ERR_INVALID_ARG, "%s: null argument", who);
+  if (n < 0 || !valid_stride(stride_bytes)) return fail(ILSM_ERR_INVALID_ARG, "%s: bad n/stride", who);
+  return ILSM_OK;
+}
+
 ILSM_API int ilsm_map_build_dev(ilsm_map* map, const float* d_xyz, int n, int stride_bytes, float cell) {
-  if (!map || (n > 0 && !d_xyz)) return fail(ILSM_ERR_INVALID_ARG, "ilsm_map_build_dev: null argument");
-  std::lock_guard<std::mutex> lk(map->m.ctx->mu);
-  ILSM_CUDA(cudaSetDevice(map->m.ctx->device));
+  int rc = check_build_args(map, d_xyz, n, stride_bytes, "ilsm_map_build_dev");
+  if (rc) return rc;
+  ILSM_ENTER(*map->m.ctx);
   return map->m.build_dev(d_xyz, n, stride_bytes, cell);
 }
 
 ILSM_API int ilsm_map_build_pair_dev(ilsm_map* map_a, const float* d_xyz_a, int n_a, ilsm_map* map_b, const float* d_xyz_b, int n_b,
                                      int stride_bytes, float cell) {
-  if (!map_a || !map_b || (n_a > 0 && !d_xyz_a) || (n_b > 0 && !d_xyz_b)) return fail(ILSM_ERR_INVALID_ARG, "map_build_pair_dev: null argument");
-  if (n_a < 0 || n_b < 0 || !valid_stride(stride_bytes)) return fail(ILSM_ERR_INVALID_ARG, "map_build_pair_dev: bad n/stride");
-  Ctx& c = *map_a->m.ctx;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  int rc;
+  if ((rc = check_build_args(map_a, d_xyz_a, n_a, stride_bytes, "map_build_pair_dev")) ||
+      (rc = check_build_args(map_b, d_xyz_b, n_b, stride_bytes, "map_build_pair_dev")))
+    return rc;
+  ILSM_ENTER(*map_a->m.ctx);
   return build_pair_dev(&map_a->m, d_xyz_a, n_a, &map_b->m, d_xyz_b, n_b, stride_bytes, cell);
 }
 
 ILSM_API int ilsm_map_join(ilsm_map* map) {
   if (!map) return fail(ILSM_ERR_INVALID_ARG, "map_join: null map");
-  Ctx& c = *map->m.ctx;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
-  return map->m.wait_ready(c.stream);
+  ILSM_ENTER(*map->m.ctx);
+  return map->m.wait_ready(map->m.ctx->stream);
 }
 
 ILSM_API int ilsm_map_build(ilsm_map* map, const float* xyz, int n, int stride_bytes, float cell) {
-  if (!map || (n > 0 && !xyz)) return fail(ILSM_ERR_INVALID_ARG, "ilsm_map_build: null argument");
-  if (n < 0 || !valid_stride(stride_bytes)) return fail(ILSM_ERR_INVALID_ARG, "ilsm_map_build: bad n/stride");
+  int rc = check_build_args(map, xyz, n, stride_bytes, "ilsm_map_build");
+  if (rc) return rc;
   Map& m = map->m;
-  std::lock_guard<std::mutex> lk(m.ctx->mu);
-  ILSM_CUDA(cudaSetDevice(m.ctx->device));
+  ILSM_ENTER(*m.ctx);
   size_t bytes = (size_t)n * stride_bytes;
-  int rc;
   if ((rc = m.raw.reserve(bytes / 4 + 4))) return rc;
   // the staging buffer may still be read by users of the previous build on the context stream
   ILSM_CUDA(cudaEventRecord(m.ctx_done, m.ctx->stream));
@@ -247,8 +253,7 @@ ILSM_API int ilsm_map_insert(ilsm_map* map, const float* xyz, int n, int stride_
   if (!map || (n > 0 && !xyz)) return fail(ILSM_ERR_INVALID_ARG, "ilsm_map_insert: null argument");
   if (n < 0 || !valid_stride(stride_bytes)) return fail(ILSM_ERR_INVALID_ARG, "ilsm_map_insert: bad n/stride");
   Map& m = map->m;
-  std::lock_guard<std::mutex> lk(m.ctx->mu);
-  ILSM_CUDA(cudaSetDevice(m.ctx->device));
+  ILSM_ENTER(*m.ctx);
   if (m.table_size == 0) {  // Add_Points on an empty tree behaves like Build
     int rc0 = m.build_dev(nullptr, 0, 16, m.cell);
     if (rc0) return rc0;
@@ -267,8 +272,7 @@ ILSM_API int ilsm_map_insert(ilsm_map* map, const float* xyz, int n, int stride_
 ILSM_API int ilsm_map_points(ilsm_map* map, float* out_xyzi, int capacity, int* n_out) {
   if (!map || !n_out || (capacity > 0 && !out_xyzi)) return fail(ILSM_ERR_INVALID_ARG, "ilsm_map_points: null argument");
   Map& m = map->m;
-  std::lock_guard<std::mutex> lk(m.ctx->mu);
-  ILSM_CUDA(cudaSetDevice(m.ctx->device));
+  ILSM_ENTER(*m.ctx);
   *n_out = m.n;
   const int k = m.n < capacity ? m.n : capacity;
   if (k > 0) {
@@ -278,24 +282,30 @@ ILSM_API int ilsm_map_points(ilsm_map* map, float* out_xyzi, int capacity, int* 
   return ILSM_OK;
 }
 
+// the argument check of ilsm_knn[_dev]
+static int check_knn_args(const ilsm_map* map, const float* q, int nq, int stride_bytes, int k, const int32_t* idx, const float* d2,
+                          const char* who) {
+  if (!map || (nq > 0 && (!q || !idx || !d2))) return fail(ILSM_ERR_INVALID_ARG, "%s: null argument", who);
+  if (nq < 0 || !valid_stride(stride_bytes) || k < 1 || k > 8) return fail(ILSM_ERR_INVALID_ARG, "%s: bad nq/k/stride", who);
+  return ILSM_OK;
+}
+
 ILSM_API int ilsm_knn_dev(ilsm_map* map, const float* d_q, int nq, int stride_bytes, int k, float max_dist, int32_t* d_idx,
                  float* d_d2) {
-  if (!map || (nq > 0 && (!d_q || !d_idx || !d_d2))) return fail(ILSM_ERR_INVALID_ARG, "ilsm_knn_dev: null argument");
-  std::lock_guard<std::mutex> lk(map->m.ctx->mu);
-  ILSM_CUDA(cudaSetDevice(map->m.ctx->device));
+  int rc = check_knn_args(map, d_q, nq, stride_bytes, k, d_idx, d_d2, "ilsm_knn_dev");
+  if (rc) return rc;
+  ILSM_ENTER(*map->m.ctx);
   return map->m.knn_dev(d_q, nq, stride_bytes, k, max_dist, d_idx, d_d2);
 }
 
 ILSM_API int ilsm_knn(ilsm_map* map, const float* q, int nq, int stride_bytes, int k, float max_dist, int32_t* idx, float* d2) {
-  if (!map || (nq > 0 && (!q || !idx || !d2))) return fail(ILSM_ERR_INVALID_ARG, "ilsm_knn: null argument");
-  if (nq < 0 || !valid_stride(stride_bytes) || k < 1 || k > 8) return fail(ILSM_ERR_INVALID_ARG, "ilsm_knn: bad nq/k/stride");
+  int rc = check_knn_args(map, q, nq, stride_bytes, k, idx, d2, "ilsm_knn");
+  if (rc) return rc;
   Map& m = map->m;
   Ctx& c = *m.ctx;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   if (nq == 0) return ILSM_OK;
   size_t bytes = (size_t)nq * stride_bytes;
-  int rc;
   if ((rc = c.stack_raw.reserve(bytes / 4 + 4)) || (rc = c.out_idx.reserve((size_t)nq * k)) ||
       (rc = c.out_d2.reserve((size_t)nq * k)))
     return rc;
@@ -307,13 +317,16 @@ ILSM_API int ilsm_knn(ilsm_map* map, const float* q, int nq, int stride_bytes, i
   return ILSM_OK;
 }
 
+// the argument check of ilsm_register[_dev], ilsm_associate[_dev] and ilsm_odometry; `has_pose`: the pose pointers
+// are not null
 static int check_reg_args(ilsm_ctx* ctx, ilsm_map* mc, ilsm_map* ms, const float* corner, int nc, const float* surf,
-                          int ns, int stride_bytes) {
-  if (!ctx || !mc || !ms) return fail(ILSM_ERR_INVALID_ARG, "register: null handle");
-  if (mc->m.ctx != &ctx->c || ms->m.ctx != &ctx->c) return fail(ILSM_ERR_INVALID_ARG, "register: map belongs to another context");
-  if (nc < 0 || ns < 0 || !valid_stride(stride_bytes)) return fail(ILSM_ERR_INVALID_ARG, "register: bad counts/stride");
-  if ((nc > 0 && !corner) || (ns > 0 && !surf)) return fail(ILSM_ERR_INVALID_ARG, "register: null stack");
-  if (mc->m.table_size == 0 || ms->m.table_size == 0) return fail(ILSM_ERR_STATE, "register: map not built");
+                          int ns, int stride_bytes, bool has_pose, const char* who) {
+  if (!ctx || !mc || !ms) return fail(ILSM_ERR_INVALID_ARG, "%s: null handle", who);
+  if (mc->m.ctx != &ctx->c || ms->m.ctx != &ctx->c) return fail(ILSM_ERR_INVALID_ARG, "%s: map belongs to another context", who);
+  if (nc < 0 || ns < 0 || !valid_stride(stride_bytes)) return fail(ILSM_ERR_INVALID_ARG, "%s: bad counts/stride", who);
+  if ((nc > 0 && !corner) || (ns > 0 && !surf)) return fail(ILSM_ERR_INVALID_ARG, "%s: null stack", who);
+  if (mc->m.table_size == 0 || ms->m.table_size == 0) return fail(ILSM_ERR_STATE, "%s: map not built", who);
+  if (!has_pose) return fail(ILSM_ERR_INVALID_ARG, "%s: null pose", who);
   return ILSM_OK;
 }
 
@@ -363,13 +376,11 @@ static int stage_stacks(Ctx& c, const float* corner, int nc, const float* surf, 
 
 ILSM_API int ilsm_register_dev(ilsm_ctx* ctx, ilsm_map* mc, ilsm_map* ms, const float* d_corner, int nc, const float* d_surf,
                       int ns, int stride_bytes, double* d_pose7, const ilsm_reg_opts* opts, ilsm_reg_report* d_report) {
-  int rc = check_reg_args(ctx, mc, ms, d_corner, nc, d_surf, ns, stride_bytes);
+  int rc = check_reg_args(ctx, mc, ms, d_corner, nc, d_surf, ns, stride_bytes, d_pose7 != nullptr, "register_dev");
   if (rc) return rc;
-  if (!d_pose7) return fail(ILSM_ERR_INVALID_ARG, "register_dev: null pose");
   ilsm_reg_opts o = sanitize(opts);
   Ctx& c = ctx->c;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   if ((rc = check_map_size(o, mc, ms))) return rc;
   // the first association reads the pose straight from d_pose7 (and seeds the LM state), the last solve writes the
   // result and the report back: no separate pose upload / download launches
@@ -377,20 +388,17 @@ ILSM_API int ilsm_register_dev(ilsm_ctx* ctx, ilsm_map* mc, ilsm_map* ms, const 
   src.mode = 2, src.dptr = d_pose7;
   PoseDst dst;
   dst.d_pose7 = d_pose7, dst.d_report = d_report;
-  if (o.outer_iterations < 1) return ILSM_OK;
   return c.register_dev(&mc->m, &ms->m, d_corner, nc, d_surf, ns, stride_bytes, o, &src, &dst);
 }
 
 ILSM_API int ilsm_associate_dev(ilsm_ctx* ctx, ilsm_map* mc, ilsm_map* ms, const float* d_corner, int nc,
                                 const float* d_surf, int ns, int stride_bytes, const double* d_pose7,
                                 const ilsm_reg_opts* opts) {
-  int rc = check_reg_args(ctx, mc, ms, d_corner, nc, d_surf, ns, stride_bytes);
+  int rc = check_reg_args(ctx, mc, ms, d_corner, nc, d_surf, ns, stride_bytes, d_pose7 != nullptr, "associate_dev");
   if (rc) return rc;
-  if (!d_pose7) return fail(ILSM_ERR_INVALID_ARG, "associate_dev: null pose");
   ilsm_reg_opts o = sanitize(opts);
   Ctx& c = ctx->c;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   PoseSrc src;
   src.mode = 2, src.dptr = d_pose7;
   return c.associate_dev(&mc->m, &ms->m, d_corner, nc, d_surf, ns, stride_bytes, o, false, &src);
@@ -398,29 +406,27 @@ ILSM_API int ilsm_associate_dev(ilsm_ctx* ctx, ilsm_map* mc, ilsm_map* ms, const
 
 ILSM_API int ilsm_register(ilsm_ctx* ctx, ilsm_map* mc, ilsm_map* ms, const float* corner, int nc, const float* surf, int ns,
                   int stride_bytes, double q[4], double t[3], const ilsm_reg_opts* opts, ilsm_reg_report* report) {
-  int rc = check_reg_args(ctx, mc, ms, corner, nc, surf, ns, stride_bytes);
+  int rc = check_reg_args(ctx, mc, ms, corner, nc, surf, ns, stride_bytes, q && t, "register");
   if (rc) return rc;
-  if (!q || !t) return fail(ILSM_ERR_INVALID_ARG, "register: null pose");
   ilsm_reg_opts o = sanitize(opts);
   Ctx& c = ctx->c;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   if (report) memset(report, 0, sizeof(*report));
   if ((rc = check_map_size(o, mc, ms))) return rc;
   const float *d_corner, *d_surf;
   if ((rc = stage_stacks(c, corner, nc, surf, ns, stride_bytes, &d_corner, &d_surf))) return rc;
   const PoseSrc src = host_pose(q, t);
-  if (o.outer_iterations < 1) return ILSM_OK;
   if ((rc = c.register_dev(&mc->m, &ms->m, d_corner, nc, d_surf, ns, stride_bytes, o, &src, nullptr))) return rc;
   return c.lm_finish(q, t, report, o.outer_iterations);
 }
 
 // Front end + stacks + registration of one organised frame against two prebuilt maps, the frame already on the device.
 // One host synchronisation in the middle (the feature counts size the VoxelGrid sorts, as in the full loop).
+// min_range <= 0 takes the default 0.3 m.
 static int register_frame_core(Ctx& c, Map* mc, Map* ms, const float* d_frame, int n, int stride_bytes, float min_range, float line_res,
                                float plane_res, const ilsm_reg_opts& o, const PoseSrc* src, const PoseDst* dst, int counts_out[8]) {
   int rc;
-  if ((rc = c.features_dev(d_frame, n, stride_bytes, min_range))) return rc;
+  if ((rc = c.features_dev(d_frame, n, stride_bytes, min_range > 0.f ? min_range : 0.3f))) return rc;
   int* pin = reinterpret_cast<int*>(c.pinned.p);
   ILSM_CUDA(cudaMemcpyAsync(pin, c.fe.counts.p, 8 * sizeof(int), cudaMemcpyDeviceToHost, c.stream));
   ILSM_CUDA(cudaStreamSynchronize(c.stream));
@@ -437,7 +443,6 @@ static int register_frame_core(Ctx& c, Map* mc, Map* ms, const float* d_frame, i
   const Ctx::VgCloud vc[2] = {{reinterpret_cast<const float*>(c.rf_lsharp.p), n_lsharp, line_res, c.rf_stack_c.p, c.rf_stack_n.p},
                               {reinterpret_cast<const float*>(c.fe.lflat.p), n_lflat, plane_res, c.rf_stack_s.p, c.rf_stack_n.p + 1}};
   if ((rc = c.voxelgrid(vc, 2, 16, 3, c.stream))) return rc;
-  if (o.outer_iterations < 1) return ILSM_OK;
   // the association / solve block with the stack sizes read on the device (laserMapping.cpp:640-861)
   c.d_stack_counts = c.rf_stack_n.p;
   rc = c.register_dev(mc, ms, reinterpret_cast<const float*>(c.rf_stack_c.p), n_lsharp, reinterpret_cast<const float*>(c.rf_stack_s.p), n_lflat,
@@ -446,46 +451,40 @@ static int register_frame_core(Ctx& c, Map* mc, Map* ms, const float* d_frame, i
   return rc;
 }
 
-// the argument checks of ilsm_register_frame[_dev]; `who` names the entry point in the message
+// the argument check of ilsm_register_frame[_dev], the built maps and the map-size guard included
 static int check_frame_args(ilsm_ctx* ctx, ilsm_map* mc, ilsm_map* ms, const float* xyzi, int n, bool has_pose, int stride_bytes,
-                            float line_res, float plane_res, const char* who) {
-  char msg[160];
-  if (!ctx || !mc || !ms || (n > 0 && !xyzi) || !has_pose)
-    return snprintf(msg, sizeof(msg), "%s: null argument", who), fail(ILSM_ERR_INVALID_ARG, msg);
-  if (mc->m.ctx != &ctx->c || ms->m.ctx != &ctx->c)
-    return snprintf(msg, sizeof(msg), "%s: map belongs to another context", who), fail(ILSM_ERR_INVALID_ARG, msg);
+                            float line_res, float plane_res, const ilsm_reg_opts& o, const char* who) {
+  if (!ctx || !mc || !ms || (n > 0 && !xyzi) || !has_pose) return fail(ILSM_ERR_INVALID_ARG, "%s: null argument", who);
+  if (mc->m.ctx != &ctx->c || ms->m.ctx != &ctx->c) return fail(ILSM_ERR_INVALID_ARG, "%s: map belongs to another context", who);
   if (n < 0 || !valid_stride(stride_bytes) || stride_bytes < 16 || !(line_res > 0.f) || !(plane_res > 0.f))
-    return snprintf(msg, sizeof(msg), "%s: bad n/stride/resolution", who), fail(ILSM_ERR_INVALID_ARG, msg);
-  return ILSM_OK;
+    return fail(ILSM_ERR_INVALID_ARG, "%s: bad n/stride/resolution", who);
+  if (mc->m.table_size == 0 || ms->m.table_size == 0) return fail(ILSM_ERR_STATE, "%s: map not built", who);
+  return check_map_size(o, mc, ms);
 }
 
 ILSM_API int ilsm_register_frame(ilsm_ctx* ctx, ilsm_map* mc, ilsm_map* ms, const float* xyzi, int n, int stride_bytes, float min_range,
                                  float line_res, float plane_res, double q[4], double t[3], const ilsm_reg_opts* opts,
                                  ilsm_reg_report* report, int32_t sizes_out[4]) {
-  int rc = check_frame_args(ctx, mc, ms, xyzi, n, q && t, stride_bytes, line_res, plane_res, "register_frame");
-  if (rc) return rc;
-  ilsm_reg_opts o = sanitize(opts);
-  Ctx& c = ctx->c;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
   if (report) memset(report, 0, sizeof(*report));
-  if ((rc = check_map_size(o, mc, ms))) return rc;
+  const ilsm_reg_opts o = sanitize(opts);
+  int rc = check_frame_args(ctx, mc, ms, xyzi, n, q && t, stride_bytes, line_res, plane_res, o, "register_frame");
+  if (rc) return rc;
+  Ctx& c = ctx->c;
+  ILSM_ENTER(c);
   const size_t bytes = (size_t)n * stride_bytes;
   if ((rc = c.fe.raw.reserve(bytes / 4 + 4))) return rc;
   if (bytes) ILSM_CUDA(cudaMemcpyAsync(c.fe.raw.p, xyzi, bytes, cudaMemcpyHostToDevice, c.stream));
   const PoseSrc src = host_pose(q, t);
   int counts[8];
-  if ((rc = register_frame_core(c, &mc->m, &ms->m, c.fe.raw.p, n, stride_bytes, min_range > 0.f ? min_range : 0.3f, line_res, plane_res, o,
-                                &src, nullptr, counts)))
+  if ((rc = register_frame_core(c, &mc->m, &ms->m, c.fe.raw.p, n, stride_bytes, min_range, line_res, plane_res, o, &src, nullptr,
+                                counts)))
     return rc;
   int* sn = reinterpret_cast<int*>(c.pinned.p + Ctx::kPinSite);  // the down-sampled stack sizes
   if ((rc = c.read_back_lm(c.stream))) return rc;
   ILSM_CUDA(cudaMemcpyAsync(sn, c.rf_stack_n.p, 2 * sizeof(int), cudaMemcpyDeviceToHost, c.stream));
   ILSM_CUDA(cudaStreamSynchronize(c.stream));
-  if (o.outer_iterations >= 1) {
-    c.lm_result(q, t, report);
-    if (report) report->passes = o.outer_iterations;
-  }
+  c.lm_result(q, t, report);
+  if (report) report->passes = o.outer_iterations;
   if (sizes_out) {
     sizes_out[0] = counts[2], sizes_out[1] = counts[4], sizes_out[2] = sn[0], sizes_out[3] = sn[1];
   }
@@ -494,31 +493,27 @@ ILSM_API int ilsm_register_frame(ilsm_ctx* ctx, ilsm_map* mc, ilsm_map* ms, cons
 
 ILSM_API int ilsm_register_frame_dev(ilsm_ctx* ctx, ilsm_map* mc, ilsm_map* ms, const float* d_xyzi, int n, int stride_bytes,
                                      float min_range, float line_res, float plane_res, double* d_pose7, const ilsm_reg_opts* opts) {
-  int rc = check_frame_args(ctx, mc, ms, d_xyzi, n, d_pose7 != nullptr, stride_bytes, line_res, plane_res, "register_frame_dev");
+  const ilsm_reg_opts o = sanitize(opts);
+  int rc = check_frame_args(ctx, mc, ms, d_xyzi, n, d_pose7 != nullptr, stride_bytes, line_res, plane_res, o, "register_frame_dev");
   if (rc) return rc;
-  ilsm_reg_opts o = sanitize(opts);
   Ctx& c = ctx->c;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   PoseSrc src;
   src.mode = 2, src.dptr = d_pose7;
   PoseDst dst;
   dst.d_pose7 = d_pose7;
   int counts[8];
-  return register_frame_core(c, &mc->m, &ms->m, d_xyzi, n, stride_bytes, min_range > 0.f ? min_range : 0.3f, line_res, plane_res, o, &src,
-                             &dst, counts);
+  return register_frame_core(c, &mc->m, &ms->m, d_xyzi, n, stride_bytes, min_range, line_res, plane_res, o, &src, &dst, counts);
 }
 
 ILSM_API int ilsm_associate(ilsm_ctx* ctx, ilsm_map* mc, ilsm_map* ms, const float* corner, int nc, const float* surf, int ns,
                    int stride_bytes, const double q[4], const double t[3], const ilsm_reg_opts* opts,
                    ilsm_factor* factors, int32_t* knn_idx, float* knn_d2) {
-  int rc = check_reg_args(ctx, mc, ms, corner, nc, surf, ns, stride_bytes);
+  int rc = check_reg_args(ctx, mc, ms, corner, nc, surf, ns, stride_bytes, q && t, "associate");
   if (rc) return rc;
-  if (!q || !t) return fail(ILSM_ERR_INVALID_ARG, "associate: null pose");
   ilsm_reg_opts o = sanitize(opts);
   Ctx& c = ctx->c;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   const float *d_corner, *d_surf;
   if ((rc = stage_stacks(c, corner, nc, surf, ns, stride_bytes, &d_corner, &d_surf))) return rc;
   if ((rc = c.upload_pose(q, t, c.stream))) return rc;
@@ -538,13 +533,11 @@ ILSM_API int ilsm_associate(ilsm_ctx* ctx, ilsm_map* mc, ilsm_map* ms, const flo
 ILSM_API int ilsm_odometry(ilsm_ctx* ctx, ilsm_map* last_corner, ilsm_map* last_surf, const float* sharp, int nsh,
                            const float* flat, int nfl, int stride_bytes, double q[4], double t[3],
                            const ilsm_reg_opts* opts, ilsm_reg_report* report, ilsm_factor* factors) {
-  int rc = check_reg_args(ctx, last_corner, last_surf, sharp, nsh, flat, nfl, stride_bytes);
+  int rc = check_reg_args(ctx, last_corner, last_surf, sharp, nsh, flat, nfl, stride_bytes, q && t, "odometry");
   if (rc) return rc;
-  if (!q || !t) return fail(ILSM_ERR_INVALID_ARG, "odometry: null pose");
   ilsm_reg_opts o = sanitize(opts);
   Ctx& c = ctx->c;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   if (report) memset(report, 0, sizeof(*report));
   const float *d_sharp, *d_flat;
   if ((rc = stage_stacks(c, sharp, nsh, flat, nfl, stride_bytes, &d_sharp, &d_flat))) return rc;
@@ -562,16 +555,22 @@ ILSM_API int ilsm_odometry(ilsm_ctx* ctx, ilsm_map* last_corner, ilsm_map* last_
 }
 
 // ------------------------------------------------------------------------------------------------ front end
+// the argument check of ilsm_project[_dev]
+static int check_project_args(const ilsm_ctx* ctx, const float* xyzi, int H, int W, int stride_bytes, const uint8_t* range_img,
+                              const uint8_t* inten_img, const float* track, const char* who) {
+  if (!ctx || !xyzi || !range_img || !inten_img || !track) return fail(ILSM_ERR_INVALID_ARG, "%s: null argument", who);
+  if (H <= 0 || W <= 0 || !valid_stride(stride_bytes) || stride_bytes < 16) return fail(ILSM_ERR_INVALID_ARG, "%s: bad H/W/stride", who);
+  return ILSM_OK;
+}
+
 ILSM_API int ilsm_project(ilsm_ctx* ctx, const float* xyzi, int H, int W, int stride_bytes, uint8_t* range_img,
                           uint8_t* inten_img, float* cloud_track_xyzi) {
-  if (!ctx || !xyzi || !range_img || !inten_img || !cloud_track_xyzi) return fail(ILSM_ERR_INVALID_ARG, "project: null argument");
-  if (H <= 0 || W <= 0 || !valid_stride(stride_bytes) || stride_bytes < 16) return fail(ILSM_ERR_INVALID_ARG, "project: bad H/W/stride");
+  int rc = check_project_args(ctx, xyzi, H, W, stride_bytes, range_img, inten_img, cloud_track_xyzi, "project");
+  if (rc) return rc;
   Ctx& c = ctx->c;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   const int n = H * W;
   const size_t bytes = (size_t)n * stride_bytes;
-  int rc;
   if ((rc = c.fe.raw.reserve(bytes / 4 + 4)) || (rc = c.fe.img.reserve((size_t)2 * n + 8)) || (rc = c.fe.track.reserve(n + 4)))
     return rc;
   ILSM_CUDA(cudaMemcpyAsync(c.fe.raw.p, xyzi, bytes, cudaMemcpyHostToDevice, c.stream));
@@ -587,11 +586,10 @@ ILSM_API int ilsm_project(ilsm_ctx* ctx, const float* xyzi, int H, int W, int st
 
 ILSM_API int ilsm_project_dev(ilsm_ctx* ctx, const float* d_xyzi, int H, int W, int stride_bytes, uint8_t* d_range_img,
                               uint8_t* d_inten_img, float* d_cloud_track_xyzi) {
-  if (!ctx || !d_xyzi || !d_range_img || !d_inten_img || !d_cloud_track_xyzi) return fail(ILSM_ERR_INVALID_ARG, "project_dev: null argument");
-  if (H <= 0 || W <= 0 || !valid_stride(stride_bytes) || stride_bytes < 16) return fail(ILSM_ERR_INVALID_ARG, "project_dev: bad H/W/stride");
+  int rc = check_project_args(ctx, d_xyzi, H, W, stride_bytes, d_range_img, d_inten_img, d_cloud_track_xyzi, "project_dev");
+  if (rc) return rc;
   Ctx& c = ctx->c;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   return c.project_dev(d_xyzi, H * W, stride_bytes, d_range_img, d_inten_img, d_cloud_track_xyzi);
 }
 
@@ -656,26 +654,28 @@ static int check_pc2_pack_layout(const ilsm_pc2_layout* l) {
   return ILSM_OK;
 }
 
+// the argument check of ilsm_pc2_pack[_dev] (`pack`: the layout must be writable) and ilsm_pc2_unpack[_dev]
+static int check_pc2_args(const ilsm_ctx* ctx, const void* in, int n_points, const ilsm_pc2_layout* layout, const void* out, bool pack,
+                          const char* who) {
+  if (!ctx || (n_points > 0 && (!in || !out))) return fail(ILSM_ERR_INVALID_ARG, "%s: null argument", who);
+  if (n_points < 0) return fail(ILSM_ERR_INVALID_ARG, "%s: bad n_points", who);
+  return pack ? check_pc2_pack_layout(layout) : check_pc2_layout(layout);
+}
+
 ILSM_API int ilsm_pc2_pack_dev(ilsm_ctx* ctx, const float* d_xyzi, int n_points, const ilsm_pc2_layout* layout, uint8_t* d_data_out) {
-  if (!ctx || (n_points > 0 && (!d_xyzi || !d_data_out))) return fail(ILSM_ERR_INVALID_ARG, "pc2_pack_dev: null argument");
-  if (n_points < 0) return fail(ILSM_ERR_INVALID_ARG, "pc2_pack_dev: bad n_points");
-  int rc = check_pc2_pack_layout(layout);
+  int rc = check_pc2_args(ctx, d_xyzi, n_points, layout, d_data_out, true, "pc2_pack_dev");
   if (rc) return rc;
   Ctx& c = ctx->c;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   return c.pc2_pack_dev(reinterpret_cast<const float4*>(d_xyzi), n_points, *layout, d_data_out);
 }
 
 ILSM_API int ilsm_pc2_pack(ilsm_ctx* ctx, const float* xyzi, int n_points, const ilsm_pc2_layout* layout, uint8_t* data_out) {
-  if (!ctx || (n_points > 0 && (!xyzi || !data_out))) return fail(ILSM_ERR_INVALID_ARG, "pc2_pack: null argument");
-  if (n_points < 0) return fail(ILSM_ERR_INVALID_ARG, "pc2_pack: bad n_points");
-  int rc = check_pc2_pack_layout(layout);
+  int rc = check_pc2_args(ctx, xyzi, n_points, layout, data_out, true, "pc2_pack");
   if (rc) return rc;
   if (n_points == 0) return ILSM_OK;
   Ctx& c = ctx->c;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   const size_t bytes = (size_t)n_points * layout->point_step;
   if ((rc = c.fe.pc2.reserve(bytes + 16)) || (rc = c.fe.raw.reserve((size_t)n_points * 4 + 4))) return rc;
   ILSM_CUDA(cudaMemcpyAsync(c.fe.raw.p, xyzi, (size_t)n_points * 16, cudaMemcpyHostToDevice, c.stream));
@@ -686,25 +686,19 @@ ILSM_API int ilsm_pc2_pack(ilsm_ctx* ctx, const float* xyzi, int n_points, const
 }
 
 ILSM_API int ilsm_pc2_unpack_dev(ilsm_ctx* ctx, const uint8_t* d_data, int n_points, const ilsm_pc2_layout* layout, float* d_out_xyzi) {
-  if (!ctx || (n_points > 0 && (!d_data || !d_out_xyzi))) return fail(ILSM_ERR_INVALID_ARG, "pc2_unpack_dev: null argument");
-  if (n_points < 0) return fail(ILSM_ERR_INVALID_ARG, "pc2_unpack_dev: bad n_points");
-  int rc = check_pc2_layout(layout);
+  int rc = check_pc2_args(ctx, d_data, n_points, layout, d_out_xyzi, false, "pc2_unpack_dev");
   if (rc) return rc;
   Ctx& c = ctx->c;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   return c.pc2_unpack_dev(d_data, n_points, *layout, reinterpret_cast<float4*>(d_out_xyzi));
 }
 
 ILSM_API int ilsm_pc2_unpack(ilsm_ctx* ctx, const uint8_t* data, int n_points, const ilsm_pc2_layout* layout, float* out_xyzi) {
-  if (!ctx || (n_points > 0 && (!data || !out_xyzi))) return fail(ILSM_ERR_INVALID_ARG, "pc2_unpack: null argument");
-  if (n_points < 0) return fail(ILSM_ERR_INVALID_ARG, "pc2_unpack: bad n_points");
-  int rc = check_pc2_layout(layout);
+  int rc = check_pc2_args(ctx, data, n_points, layout, out_xyzi, false, "pc2_unpack");
   if (rc) return rc;
   if (n_points == 0) return ILSM_OK;
   Ctx& c = ctx->c;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   const size_t bytes = (size_t)n_points * layout->point_step;
   if ((rc = c.fe.pc2.reserve(bytes + 16)) || (rc = c.fe.raw.reserve((size_t)n_points * 4 + 4))) return rc;
   ILSM_CUDA(cudaMemcpyAsync(c.fe.pc2.p, data, bytes, cudaMemcpyHostToDevice, c.stream));
@@ -719,8 +713,7 @@ ILSM_API int ilsm_extract_features(ilsm_ctx* ctx, const float* xyzi, int n, int 
   if (!ctx || !out || (n > 0 && !xyzi)) return fail(ILSM_ERR_INVALID_ARG, "extract_features: null argument");
   if (n < 0 || !valid_stride(stride_bytes)) return fail(ILSM_ERR_INVALID_ARG, "extract_features: bad n/stride");
   Ctx& c = ctx->c;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   const size_t bytes = (size_t)n * stride_bytes;
   int rc;
   if ((rc = c.fe.raw.reserve(bytes / 4 + 4))) return rc;
@@ -766,8 +759,7 @@ ILSM_API int ilsm_voxelgrid(ilsm_ctx* ctx, const float* xyzi, int n, int stride_
   *n_out = 0;
   if (n == 0) return ILSM_OK;
   Ctx& c = ctx->c;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   const size_t bytes = (size_t)n * stride_bytes;
   int rc;
   if ((rc = c.fe.raw.reserve(bytes / 4 + 4)) || (rc = c.fe.vox_out.reserve(n + 4)) || (rc = c.fe.vox_n.reserve(4))) return rc;
@@ -811,8 +803,7 @@ ILSM_API int ilsm_sc_make(ilsm_sc* sc, const float* xyz, int n, int stride_bytes
   if (n < 0 || !valid_stride(stride_bytes)) return fail(ILSM_ERR_INVALID_ARG, "sc_make: bad n/stride");
   ScDb& d = sc->d;
   Ctx& c = *d.ctx;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   const size_t words = (size_t)n * stride_bytes / 4;
   int rc;
   if ((rc = d.stage.reserve(words + 1200 + 8))) return rc;
@@ -825,44 +816,54 @@ ILSM_API int ilsm_sc_make(ilsm_sc* sc, const float* xyz, int n, int stride_bytes
   return ILSM_OK;
 }
 
+// the argument check of ilsm_sc_add[_dev]
+static int check_sc_add_args(const ilsm_sc* sc, const float* desc, int count, const char* who) {
+  if (!sc || (count > 0 && !desc) || count < 0) return fail(ILSM_ERR_INVALID_ARG, "%s: bad argument", who);
+  return ILSM_OK;
+}
+
 ILSM_API int ilsm_sc_add(ilsm_sc* sc, const float* desc_20x60, int count) {
-  if (!sc || (count > 0 && !desc_20x60) || count < 0) return fail(ILSM_ERR_INVALID_ARG, "sc_add: bad argument");
-  Ctx& c = *sc->d.ctx;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
-  int rc = sc->d.append_dev(desc_20x60, count, true);
+  int rc = check_sc_add_args(sc, desc_20x60, count, "sc_add");
   if (rc) return rc;
+  Ctx& c = *sc->d.ctx;
+  ILSM_ENTER(c);
+  if ((rc = sc->d.append_dev(desc_20x60, count, true))) return rc;
   ILSM_CUDA(cudaStreamSynchronize(c.stream));
   return ILSM_OK;
 }
 
 ILSM_API int ilsm_sc_add_dev(ilsm_sc* sc, const float* d_desc_20x60, int count) {
-  if (!sc || (count > 0 && !d_desc_20x60) || count < 0) return fail(ILSM_ERR_INVALID_ARG, "sc_add_dev: bad argument");
+  int rc = check_sc_add_args(sc, d_desc_20x60, count, "sc_add_dev");
+  if (rc) return rc;
   Ctx& c = *sc->d.ctx;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   return sc->d.append_dev(d_desc_20x60, count, false);
+}
+
+// the argument check of ilsm_sc_query_topk[_dev]; n_search is checked against the database by ScDb::query_dev
+static int check_sc_query_args(const ilsm_sc* sc, const float* desc, int k, const double* dist, const int32_t* id, const int32_t* shift,
+                               const char* who) {
+  if (!sc || !desc || !dist || !id || !shift) return fail(ILSM_ERR_INVALID_ARG, "%s: null argument", who);
+  if (k < 1 || k > 16) return fail(ILSM_ERR_INVALID_ARG, "%s: k must be in [1,16]", who);
+  return ILSM_OK;
 }
 
 ILSM_API int ilsm_sc_query_topk_dev(ilsm_sc* sc, const float* d_desc_20x60, int n_search, int id_offset, int k,
                                     double* d_dist, int32_t* d_id, int32_t* d_shift) {
-  if (!sc || !d_desc_20x60 || !d_dist || !d_id || !d_shift) return fail(ILSM_ERR_INVALID_ARG, "sc_query_dev: null argument");
+  int rc = check_sc_query_args(sc, d_desc_20x60, k, d_dist, d_id, d_shift, "sc_query_dev");
+  if (rc) return rc;
   Ctx& c = *sc->d.ctx;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
-  if (n_search < 0) n_search = sc->d.count;
+  ILSM_ENTER(c);
   return sc->d.query_dev(d_desc_20x60, n_search, id_offset, k, d_dist, d_id, d_shift);
 }
 
 ILSM_API int ilsm_sc_query_topk(ilsm_sc* sc, const float* desc_20x60, int n_search, int id_offset, int k, double* dist,
                                 int32_t* id, int32_t* shift) {
-  if (!sc || !desc_20x60 || !dist || !id || !shift) return fail(ILSM_ERR_INVALID_ARG, "sc_query: null argument");
+  int rc = check_sc_query_args(sc, desc_20x60, k, dist, id, shift, "sc_query");
+  if (rc) return rc;
   ScDb& d = sc->d;
   Ctx& c = *d.ctx;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
-  if (n_search < 0) n_search = d.count;
-  int rc;
+  ILSM_ENTER(c);
   if ((rc = d.stage.reserve(1200 + 8)) || (rc = d.out_dist.reserve(16)) || (rc = d.out_id.reserve(16)) ||
       (rc = d.out_shift.reserve(16)))
     return rc;
@@ -903,18 +904,22 @@ ILSM_API int ilsm_sc_merge_topk_dev(ilsm_sc* sc, const void* d_packed, int shard
   if (!sc || !d_packed || !d_out_packed || shards < 1 || k < 1 || k > 16)
     return fail(ILSM_ERR_INVALID_ARG, "sc_merge_dev: bad argument");
   Ctx& c = *sc->d.ctx;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   return sc_merge_dev(&c, d_packed, shards, k, d_out_packed);
+}
+
+// the argument check of ilsm_eval_normal_eq[_dev] and ilsm_solve[_dev]; `have`: every pointer the form needs is set
+static int check_lm_args(const ilsm_ctx* ctx, bool have, const char* who) {
+  if (!ctx || !have) return fail(ILSM_ERR_INVALID_ARG, "%s: null argument", who);
+  return ILSM_OK;
 }
 
 ILSM_API int ilsm_eval_normal_eq(ilsm_ctx* ctx, const double q[4], const double t[3], double huber_a, double* cost, double JtJ[36],
                         double Jtr[6]) {
-  if (!ctx || !q || !t || !cost || !JtJ || !Jtr) return fail(ILSM_ERR_INVALID_ARG, "eval: null argument");
+  int rc = check_lm_args(ctx, q && t && cost && JtJ && Jtr, "eval");
+  if (rc) return rc;
   Ctx& c = ctx->c;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
-  int rc;
+  ILSM_ENTER(c);
   // the pose is evaluated where upload_pose leaves it (xq, xt: 7 contiguous doubles); the 32 sums go to out_d2 scratch
   if ((rc = c.upload_pose(q, t, c.stream)) || (rc = c.out_d2.reserve(128))) return rc;
   double* d_out = reinterpret_cast<double*>(c.out_d2.p);
@@ -935,40 +940,34 @@ ILSM_API int ilsm_eval_normal_eq(ilsm_ctx* ctx, const double q[4], const double 
 }
 
 ILSM_API int ilsm_eval_normal_eq_dev(ilsm_ctx* ctx, const double* d_pose7, double huber_a, double* d_out32) {
-  if (!ctx || !d_pose7 || !d_out32) return fail(ILSM_ERR_INVALID_ARG, "eval_dev: null argument");
+  int rc = check_lm_args(ctx, d_pose7 && d_out32, "eval_dev");
+  if (rc) return rc;
   Ctx& c = ctx->c;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   return eval_only_launch(&c, d_out32, d_pose7, huber_a);  // the kernel reads the pose straight from d_pose7
 }
 
 ILSM_API int ilsm_solve_dev(ilsm_ctx* ctx, const double* d_pose7_in, int max_num_iterations, double huber_a) {
-  if (!ctx) return fail(ILSM_ERR_INVALID_ARG, "solve_dev: null argument");
-  if (max_num_iterations < 0) max_num_iterations = 0;
-  if (max_num_iterations > 200) max_num_iterations = 200;
+  int rc = check_lm_args(ctx, true, "solve_dev");
+  if (rc) return rc;
   Ctx& c = ctx->c;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   if (d_pose7_in) {
     PoseSrc src;
     src.mode = 2, src.dptr = d_pose7_in;
-    int rc = c.seed_pose(src);
-    if (rc) return rc;
+    if ((rc = c.seed_pose(src))) return rc;
   }
-  return c.solve_launch(max_num_iterations, huber_a, 0);
+  return c.solve_launch(clamp_iterations(max_num_iterations), huber_a, 0);
 }
 
 ILSM_API int ilsm_solve(ilsm_ctx* ctx, double q[4], double t[3], int max_num_iterations, double huber_a,
                ilsm_solve_summary* summary) {
-  if (!ctx || !q || !t) return fail(ILSM_ERR_INVALID_ARG, "solve: null argument");
-  if (max_num_iterations < 0) max_num_iterations = 0;
-  if (max_num_iterations > 200) max_num_iterations = 200;
+  int rc = check_lm_args(ctx, q && t, "solve");
+  if (rc) return rc;
   Ctx& c = ctx->c;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
-  int rc;
+  ILSM_ENTER(c);
   ilsm_reg_report rep;
-  if ((rc = c.upload_pose(q, t, c.stream)) || (rc = c.solve_launch(max_num_iterations, huber_a, 0)) || (rc = c.lm_finish(q, t, &rep, 1)))
+  if ((rc = c.upload_pose(q, t, c.stream)) || (rc = c.solve_launch(clamp_iterations(max_num_iterations), huber_a, 0)) || (rc = c.lm_finish(q, t, &rep, 1)))
     return rc;
   if (summary) *summary = rep.pass[0];
   return ILSM_OK;

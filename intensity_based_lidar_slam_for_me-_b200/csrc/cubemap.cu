@@ -473,10 +473,8 @@ int cubemap_frame_collect(CubeMapH& m, double q_w[4], double t_w[3], ilsm_reg_re
     stats->flags = pin_i[0];
   }
   if (pin_i[0]) {
-    char msg[160];
-    snprintf(msg, sizeof(msg), "cube map: capacity exceeded (flags 0x%x: 16 down-sampled stack>16384, 32 cube slab full, 64 cube>16384, 2 leaf too small)", pin_i[0]);
     cudaMemsetAsync(m.err, 0, sizeof(int), c.stream);
-    return fail(ILSM_ERR_OUT_OF_MEMORY, msg);
+    return fail(ILSM_ERR_OUT_OF_MEMORY, "cube map: capacity exceeded (flags 0x%x: 16 down-sampled stack>16384, 32 cube slab full, 64 cube>16384, 2 leaf too small)", pin_i[0]);
   }
   return ILSM_OK;
 }
@@ -499,10 +497,9 @@ ILSM_API int ilsm_cubemap_create(ilsm_ctx* ctx_, float line_res, float plane_res
   if (!(line_res > 0.f) || !(plane_res > 0.f)) return fail(ILSM_ERR_INVALID_ARG, "cubemap_create: bad resolution");
   if (cube_capacity <= 0) cube_capacity = kVoxelBlockMax;
   if (cube_capacity > kVoxelBlockMax) cube_capacity = kVoxelBlockMax;
+  ILSM_ENTER(*c);
   ilsm_cubemap* h = new (std::nothrow) ilsm_cubemap();
   if (!h) return fail(ILSM_ERR_OUT_OF_MEMORY, "host allocation failed");
-  std::lock_guard<std::mutex> lk(c->mu);
-  cudaSetDevice(c->device);
   int rc = h->m.init(c, line_res, plane_res, cube_capacity);
   if (rc) {
     delete h;
@@ -547,8 +544,7 @@ ILSM_API int ilsm_cubemap_insert_world(ilsm_cubemap* cm, const float* corner, in
   if (nc < 0 || ns < 0 || !valid_stride(stride_bytes)) return fail(ILSM_ERR_INVALID_ARG, "cubemap_insert_world: bad n/stride");
   CubeMapH& m = cm->m;
   Ctx& c = *m.ctx;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   int rc;
   if ((rc = m.wait_tail()) || (rc = m.roll(centre))) return rc;
   const int ioff = stride_bytes >= 32 ? 4 : (stride_bytes >= 16 ? 3 : -1);
@@ -589,8 +585,7 @@ ILSM_API int ilsm_cubemap_frame(ilsm_cubemap* cm, const float* corner_last, int 
     return fail(ILSM_ERR_INVALID_ARG, "cubemap_frame: bad n/stride (fewer than 2^24 points per feature cloud)");
   CubeMapH& m = cm->m;
   Ctx& c = *m.ctx;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   ilsm_reg_opts o;
   if (opts) o = *opts; else ilsm_reg_opts_default(&o);
   if (report) memset(report, 0, sizeof(*report));
@@ -606,8 +601,7 @@ ILSM_API int ilsm_cubemap_cube(ilsm_cubemap* cm, int which, int cube_index, floa
   if (!cm || !n_out || cube_index < 0 || cube_index >= kCNum || (which != 0 && which != 1))
     return fail(ILSM_ERR_INVALID_ARG, "cubemap_cube: bad argument");
   CubeMapH& m = cm->m;
-  std::lock_guard<std::mutex> lk(m.ctx->mu);
-  ILSM_CUDA(cudaSetDevice(m.ctx->device));
+  ILSM_ENTER(*m.ctx);
   {
     int rcw = m.wait_tail();  // a deferred insertion of the last frame may still be running
     if (rcw) return rcw;

@@ -427,8 +427,7 @@ ILSM_API int ilsm_ground_extract(ilsm_ground* g, const float* xyz, int n, int st
   if (opts) o = *opts; else ilsm_ground_opts_default(&o);
   if (o.max_iterations < 1 || o.max_iterations > 62) return fail(ILSM_ERR_INVALID_ARG, "ground_extract: max_iterations must be in [1, 62]");
   Ctx& c = *g->ctx;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   int rc = ground_extract_core(g, xyz, true, n, stride_bytes, o, n_out, coeff_abcd, info);
   if (rc) return rc;
   const int ng = *n_out;

@@ -358,25 +358,19 @@ using namespace ilsm;
 
 static int icp_check(ilsm_ctx* ctx, ilsm_map* const* targets, int n_pairs, const float* src, const int* offs, int stride_bytes,
                      const ilsm_icp_opts* opts, ilsm_icp_result* results, const char* who) {
-  char msg[160];
-  if (!ctx) return snprintf(msg, sizeof(msg), "%s: null ctx", who), fail(ILSM_ERR_INVALID_ARG, msg);
-  if (n_pairs < 0) return snprintf(msg, sizeof(msg), "%s: n_pairs < 0", who), fail(ILSM_ERR_INVALID_ARG, msg);
+  if (!ctx) return fail(ILSM_ERR_INVALID_ARG, "%s: null ctx", who);
+  if (n_pairs < 0) return fail(ILSM_ERR_INVALID_ARG, "%s: n_pairs < 0", who);
   if (n_pairs == 0) return ILSM_OK;
-  if (!targets || !offs || !results)
-    return snprintf(msg, sizeof(msg), "%s: null targets / offsets / results", who), fail(ILSM_ERR_INVALID_ARG, msg);
-  if (!valid_stride(stride_bytes))
-    return snprintf(msg, sizeof(msg), "%s: bad stride", who), fail(ILSM_ERR_INVALID_ARG, msg);
-  if (opts && opts->max_iterations < 0)
-    return snprintf(msg, sizeof(msg), "%s: max_iterations < 0", who), fail(ILSM_ERR_INVALID_ARG, msg);
-  if (offs[0] < 0) return snprintf(msg, sizeof(msg), "%s: negative source offset", who), fail(ILSM_ERR_INVALID_ARG, msg);
+  if (!targets || !offs || !results) return fail(ILSM_ERR_INVALID_ARG, "%s: null targets / offsets / results", who);
+  if (!valid_stride(stride_bytes)) return fail(ILSM_ERR_INVALID_ARG, "%s: bad stride", who);
+  if (opts && opts->max_iterations < 0) return fail(ILSM_ERR_INVALID_ARG, "%s: max_iterations < 0", who);
+  if (offs[0] < 0) return fail(ILSM_ERR_INVALID_ARG, "%s: negative source offset", who);
   for (int p = 0; p < n_pairs; ++p)
-    if (offs[p + 1] < offs[p])
-      return snprintf(msg, sizeof(msg), "%s: source offsets decrease at pair %d", who, p), fail(ILSM_ERR_INVALID_ARG, msg);
-  if (offs[n_pairs] > offs[0] && !src) return snprintf(msg, sizeof(msg), "%s: null source points", who), fail(ILSM_ERR_INVALID_ARG, msg);
+    if (offs[p + 1] < offs[p]) return fail(ILSM_ERR_INVALID_ARG, "%s: source offsets decrease at pair %d", who, p);
+  if (offs[n_pairs] > offs[0] && !src) return fail(ILSM_ERR_INVALID_ARG, "%s: null source points", who);
   for (int p = 0; p < n_pairs; ++p) {
-    if (!targets[p]) return snprintf(msg, sizeof(msg), "%s: null target %d", who, p), fail(ILSM_ERR_INVALID_ARG, msg);
-    if (targets[p]->m.ctx != &ctx->c)
-      return snprintf(msg, sizeof(msg), "%s: target %d belongs to another context", who, p), fail(ILSM_ERR_INVALID_ARG, msg);
+    if (!targets[p]) return fail(ILSM_ERR_INVALID_ARG, "%s: null target %d", who, p);
+    if (targets[p]->m.ctx != &ctx->c) return fail(ILSM_ERR_INVALID_ARG, "%s: target %d belongs to another context", who, p);
   }
   return ILSM_OK;
 }
@@ -389,8 +383,7 @@ static int icp_run(ilsm_ctx* ctx, ilsm_map* const* targets, int n_pairs, const f
   else
     ilsm_icp_opts_default(&o);
   Ctx& c = ctx->c;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   const size_t bytes = (size_t)(offs[n_pairs] - offs[0]) * stride_bytes;
   const float* first = src + (size_t)offs[0] * (stride_bytes / 4);
   if (!on_device) {

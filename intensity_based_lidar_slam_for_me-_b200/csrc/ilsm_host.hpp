@@ -16,7 +16,7 @@
 
 namespace ilsm {
 
-int fail(int code, const char* msg);
+int fail(int code, const char* fmt, ...) __attribute__((format(printf, 2, 3)));
 int fail_cuda(cudaError_t e, const char* where);
 int check_launch(const char* where);
 void count_launches(int k);
@@ -107,7 +107,7 @@ struct Buf {
     void* np = nullptr;
     if (Mem::alloc(&np, want * sizeof(T)) != cudaSuccess) {
       cudaGetLastError();
-      return fail(ILSM_ERR_OUT_OF_MEMORY, Mem::what);
+      return fail(ILSM_ERR_OUT_OF_MEMORY, "%s", Mem::what);
     }
     release();  // only on growth
     p = static_cast<T*>(np);
@@ -364,6 +364,20 @@ struct Ctx {
                    const ilsm_reg_opts& o, const PoseSrc* src = nullptr, const PoseDst* dst = nullptr);
 };
 
+// The way into a context: holds its mutex and makes its device current.  `rc` is ILSM_OK, or the cudaSetDevice error
+// through fail_cuda.  ILSM_ENTER(c) is the form for a function that returns that error at once.
+struct CtxGuard {
+  std::lock_guard<std::mutex> lk;
+  int rc;
+  explicit CtxGuard(Ctx& c) : lk(c.mu) {
+    const cudaError_t e = cudaSetDevice(c.device);
+    rc = e == cudaSuccess ? ILSM_OK : fail_cuda(e, "cudaSetDevice");
+  }
+};
+#define ILSM_ENTER(c)               \
+  ::ilsm::CtxGuard ilsm_guard__(c); \
+  if (ilsm_guard__.rc) return ilsm_guard__.rc
+
 // ScanContext keyframe database (one shard when the database is split across ranks).
 struct ScQuery;
 struct ScDb {
@@ -398,6 +412,8 @@ struct ScDb {
   int candidates_dev(const float* d_qdesc, int n_search, int num_cand, int* d_id, float* d_key_d2, double* d_dist, int* d_shift);
   int make_dev(const float* d_pts, int n, int stride_bytes, float* d_desc);
   int query_dev(const float* d_qdesc, int n_search, int id_offset, int k, double* d_dist, int* d_id, int* d_shift);
+  // the entries a query scans: the first n_search, every entry when n_search < 0
+  int searched(int n_search) const { return n_search < 0 ? count : n_search; }
   ScDb();  // both in scancontext.cu, where ScQuery is complete
   ~ScDb();
 };

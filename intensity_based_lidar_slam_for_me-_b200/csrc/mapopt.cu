@@ -93,9 +93,8 @@ ILSM_API int ilsm_mapopt_create(ilsm_ctx* ctx, float voxel_leaf, float downsampl
   m.ds = downsample_size > 0.f ? downsample_size : 0.4f;  // KD_TREE(0.3, 0.6, 0.4)  :504
   int rc = ilsm_ground_create(ctx, &m.ground);
   if (rc == ILSM_OK) {
-    std::lock_guard<std::mutex> lk(ctx->c.mu);
-    cudaSetDevice(ctx->c.device);
-    if (!(rc = m.map.init(&ctx->c))) rc = m.empty.init(&ctx->c);
+    CtxGuard g(ctx->c);
+    if (!(rc = g.rc) && !(rc = m.map.init(&ctx->c))) rc = m.empty.init(&ctx->c);
     // the stand-in corner map must be a valid (empty) structure: the association kernel reads its bounding box
     if (!rc) rc = m.empty.build_dev(nullptr, 0, 16, 0.f);
     if (!rc) rc = m.empty.wait_ready(ctx->c.stream);
@@ -128,8 +127,7 @@ ILSM_API int ilsm_mapopt_map_size(const ilsm_mapopt* mo) { return mo ? mo->m.map
 ILSM_API int ilsm_mapopt_map_points(ilsm_mapopt* mo, float* out_xyzi, int capacity, int* n_out) {
   if (!mo || !n_out) return fail(ILSM_ERR_INVALID_ARG, "mapopt_map_points: null argument");
   MapOptH& m = mo->m;
-  std::lock_guard<std::mutex> lk(m.ctx->mu);
-  ILSM_CUDA(cudaSetDevice(m.ctx->device));
+  ILSM_ENTER(*m.ctx);
   *n_out = m.map.n;
   const int k = m.map.n < capacity ? m.map.n : capacity;
   if (k > 0 && out_xyzi) {
@@ -280,9 +278,7 @@ ILSM_API int ilsm_mapopt_frame(ilsm_mapopt* mo, const float* frame_xyz, int n, i
     return fail(ILSM_ERR_INVALID_ARG, "mapopt_frame: null argument");
   if (n < 0 || n_plane < 0 || !valid_stride(stride_bytes) || !valid_stride(plane_stride_bytes))
     return fail(ILSM_ERR_INVALID_ARG, "mapopt_frame: bad n/stride");
-  Ctx& c = *mo->m.ctx;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(*mo->m.ctx);
   return mapopt_frame_core(mo, frame_xyz, n, stride_bytes, plane_xyz, n_plane, plane_stride_bytes, true, q_wodom, t_wodom, q_w, t_w,
                            gopts, stats);
 }

@@ -136,8 +136,7 @@ ILSM_API int ilsm_orb_match(ilsm_ctx* ctx, const uint8_t* cur_desc, int n_cur, c
   *n_matches = 0, *n_good = 0;
   if (n_cur == 0 || n_prev == 0) return ILSM_OK;
   Ctx& c = ctx->c;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   // scratch layout in out_idx: cur desc | prev desc | best_t[n_cur] dist_q[n_cur] best_q[n_prev] dist_t[n_prev] counts[4]
   //                            | matches | good
   const size_t wq = (size_t)n_cur * 8, wt = (size_t)n_prev * 8;
@@ -182,8 +181,7 @@ ILSM_API int ilsm_align_points(ilsm_ctx* ctx, const float* src_xyz, const float*
   if (max_num_iterations < 0) max_num_iterations = 0;
   if (max_num_iterations > 200) max_num_iterations = 200;
   Ctx& c = ctx->c;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   int rc;
   FactorBufs& f = c.fac;
   const size_t bytes = (size_t)n * stride_bytes;

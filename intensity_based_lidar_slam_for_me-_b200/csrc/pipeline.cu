@@ -345,7 +345,7 @@ static int take_mapping_result(SlamH& s, double q_map[4], double t_map[3], ilsm_
   lk.unlock();
   s.maps_in_flight--;
   if (frame) *frame = r.frame;
-  if (r.rc) return fail(r.rc, r.err);
+  if (r.rc) return fail(r.rc, "%s", r.err);
   for (int i = 0; i < 4; ++i) q_map[i] = r.q[i];
   for (int i = 0; i < 3; ++i) t_map[i] = r.t[i];
   if (stats) stats->mapping = r.report, stats->cubemap = r.cstats;
@@ -403,7 +403,7 @@ static int take_frontend_result(SlamH& s, SlamH::FeResult* out) {
   s.n_fres.store(0, std::memory_order_relaxed);
   s.fe_in_flight = false;
   *out = s.fres;
-  if (out->rc) return fail(out->rc, out->err);
+  if (out->rc) return fail(out->rc, "%s", out->err);
   return ILSM_OK;
 }
 
@@ -444,9 +444,8 @@ static int slam_create_common(ilsm_ctx* ctx, float min_range, ilsm_slam** out, i
   h->s.min_range = min_range > 0.f ? min_range : 0.3f;
   int rc;
   {
-    std::lock_guard<std::mutex> lk(ctx->c.mu);
-    cudaSetDevice(ctx->c.device);
-    if (!(rc = h->s.last_corner.init(&ctx->c))) rc = h->s.last_surf.init(&ctx->c);
+    CtxGuard g(ctx->c);
+    if (!(rc = g.rc) && !(rc = h->s.last_corner.init(&ctx->c))) rc = h->s.last_surf.init(&ctx->c);
     if (!rc && !(rc = h->s.last_corner.reserve_points(16384))) rc = h->s.last_surf.reserve_points(65536);
     if (!rc) rc = reserve_frame_buffers(h->s);
   }
@@ -642,8 +641,7 @@ static int slam_frame_impl(ilsm_slam* slam, const float* xyzi, int n, int stride
     return fail(ILSM_ERR_STATE, "slam_frame: ilsm_slam_create_async handles take ilsm_slam_frame_async (and only those)");
   if (have_prev) *have_prev = 0;
   Ctx& c = *s.ctx;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   if (stats) memset(stats, 0, sizeof(*stats));
   int rc;
   PhaseClock clk(s.phase_s);
@@ -715,8 +713,7 @@ extern "C" ILSM_API int ilsm_slam_frame_staged(ilsm_slam* slam, const float* xyz
   if (!s.staged) return fail(ILSM_ERR_STATE, "slam_frame_staged: not an ilsm_slam_create_staged handle");
   *odom_frame = *map_frame = -1;
   Ctx& c = *s.ctx;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(c);
   if (stats) memset(stats, 0, sizeof(*stats));
   int rc;
   PhaseClock clk(s.phase_s);

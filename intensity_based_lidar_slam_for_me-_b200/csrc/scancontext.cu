@@ -630,6 +630,7 @@ int ScDb::make_dev(const float* d_pts, int n, int stride_bytes, float* d_desc) {
 }
 
 int ScDb::query_dev(const float* d_qdesc, int n_search, int id_offset, int k, double* d_dist, int* d_id, int* d_shift) {
+  n_search = searched(n_search);
   if (k < 1 || k > kTopKMax) return fail(ILSM_ERR_INVALID_ARG, "sc_query: k must be in [1,16]");
   if (n_search < 0 || n_search > count) return fail(ILSM_ERR_INVALID_ARG, "sc_query: n_search exceeds the database");
   // two resident blocks of 8 warps per SM; fewer blocks when the shard is small.  The final merge holds at most
@@ -680,6 +681,7 @@ int sc_score_lists_dev(ScDb* d, const float* d_qdesc, int B, int k, const u64* d
 }
 
 int ScDb::query_batch_dev(const float* d_qdesc, int B, int n_search, int id_offset, int k, unsigned char* d_packed) {
+  n_search = searched(n_search);
   // large shards: approximate scoring of every pair on the tensor cores, exact rescoring of the few that can matter
   if (n_search >= tc_min) return query_batch_tc_dev(d_qdesc, B, n_search, id_offset, k, d_packed, nullptr);
   for (int b = 0; b < B; ++b) {
@@ -696,6 +698,7 @@ int ScDb::query_batch_dev(const float* d_qdesc, int B, int n_search, int id_offs
 // order.  Outputs (device): ids, float key distances, distances, shifts -- num_cand entries each, id -1 when the
 // database holds fewer entries.
 int ScDb::candidates_dev(const float* d_qdesc, int n_search, int num_cand, int* d_id, float* d_key_d2, double* d_dist, int* d_shift) {
+  n_search = searched(n_search);
   if (num_cand < 1 || num_cand > kTopKMax) return fail(ILSM_ERR_INVALID_ARG, "sc_candidates: num_candidates must be in [1,16]");
   if (n_search < 0 || n_search > count) return fail(ILSM_ERR_INVALID_ARG, "sc_candidates: n_search exceeds the database");
   const int blocks = n_search > 0 ? (n_search + 1023) / 1024 : 1;

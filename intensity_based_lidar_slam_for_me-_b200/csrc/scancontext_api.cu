@@ -59,9 +59,7 @@ int nccl_load() {
 }
 
 int nccl_fail(ncclResult_t r, const char* where) {
-  char msg[256];
-  snprintf(msg, sizeof(msg), "%s: NCCL error %d (%s)", where, (int)r, g_nccl.GetErrorString ? g_nccl.GetErrorString(r) : "?");
-  return fail(ILSM_ERR_CUDA, msg);
+  return fail(ILSM_ERR_CUDA, "%s: NCCL error %d (%s)", where, (int)r, g_nccl.GetErrorString ? g_nccl.GetErrorString(r) : "?");
 }
 }  // namespace
 
@@ -81,9 +79,7 @@ ILSM_API int ilsm_sc_query_candidates(ilsm_sc* sc, const float* desc_20x60, int 
   if (num_candidates < 1 || num_candidates > 16) return fail(ILSM_ERR_INVALID_ARG, "sc_candidates: num_candidates must be in [1,16]");
   ScDb& d = sc->d;
   Ctx& c = *d.ctx;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
-  if (n_search < 0) n_search = d.count;
+  ILSM_ENTER(c);
   const int k = num_candidates;
   int rc;
   if ((rc = d.stage.reserve(1200 + 8)) || (rc = d.cand_out.reserve(24 * 16 + 64)) || (rc = c.pinned.reserve(4096))) return rc;
@@ -105,10 +101,11 @@ ILSM_API int ilsm_sc_query_candidates(ilsm_sc* sc, const float* desc_20x60, int 
   return ILSM_OK;
 }
 
-static int batch_args_ok(const ilsm_sc* sc, const void* desc, int n_queries, int k, const void* a, const void* b, const void* c3,
-                         const char* who) {
-  if (!sc || !desc || !a || !b || !c3) return fail(ILSM_ERR_INVALID_ARG, who);
-  if (n_queries < 1 || n_queries > 4096 || k < 1 || k > 16) return fail(ILSM_ERR_INVALID_ARG, who);
+// the argument check of ilsm_sc_query_topk_batch[_dev] and ilsm_sc_query_topk_sharded[_dev]: 1 <= n_queries <= 4096,
+// 1 <= k <= 16; `have_out`: the output pointers are set
+static int check_batch_args(const ilsm_sc* sc, const float* desc, int n_queries, int k, bool have_out, const char* who) {
+  if (!sc || !desc || !have_out || n_queries < 1 || n_queries > 4096 || k < 1 || k > 16)
+    return fail(ILSM_ERR_INVALID_ARG, "%s: bad argument", who);
   return ILSM_OK;
 }
 
@@ -130,13 +127,11 @@ static int unpack_to_host(Ctx& c, const unsigned char* d_packed, int B, int k, d
 
 ILSM_API int ilsm_sc_query_topk_batch(ilsm_sc* sc, const float* desc_20x60, int n_queries, int n_search, int id_offset, int k,
                                       double* dist, int32_t* id, int32_t* shift) {
-  int rc = batch_args_ok(sc, desc_20x60, n_queries, k, dist, id, shift, "sc_query_batch: bad argument");
+  int rc = check_batch_args(sc, desc_20x60, n_queries, k, dist && id && shift, "sc_query_batch");
   if (rc) return rc;
   ScDb& d = sc->d;
   Ctx& c = *d.ctx;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
-  if (n_search < 0) n_search = d.count;
+  ILSM_ENTER(c);
   if ((rc = d.qbatch.reserve((size_t)n_queries * 1200 + 8)) || (rc = d.pk_out.reserve((size_t)n_queries * 16 * k + 64))) return rc;
   ILSM_CUDA(cudaMemcpyAsync(d.qbatch.p, desc_20x60, (size_t)n_queries * 1200 * sizeof(float), cudaMemcpyHostToDevice, c.stream));
   if ((rc = d.query_batch_dev(d.qbatch.p, n_queries, n_search, id_offset, k, d.pk_out.p))) return rc;
@@ -145,11 +140,9 @@ ILSM_API int ilsm_sc_query_topk_batch(ilsm_sc* sc, const float* desc_20x60, int 
 
 ILSM_API int ilsm_sc_query_topk_batch_dev(ilsm_sc* sc, const float* d_desc_20x60, int n_queries, int n_search, int id_offset, int k,
                                           void* d_packed) {
-  if (!sc || !d_desc_20x60 || !d_packed || n_queries < 1 || k < 1 || k > 16) return fail(ILSM_ERR_INVALID_ARG, "sc_query_batch_dev: bad argument");
-  Ctx& c = *sc->d.ctx;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
-  if (n_search < 0) n_search = sc->d.count;
+  int rc = check_batch_args(sc, d_desc_20x60, n_queries, k, d_packed != nullptr, "sc_query_batch_dev");
+  if (rc) return rc;
+  ILSM_ENTER(*sc->d.ctx);
   return sc->d.query_batch_dev(d_desc_20x60, n_queries, n_search, id_offset, k, reinterpret_cast<unsigned char*>(d_packed));
 }
 
@@ -160,9 +153,8 @@ ILSM_API int ilsm_sc_prefilter_debug(ilsm_sc* sc, const float* desc_20x60, int n
   if (!sc || !desc_20x60 || !approx || !aligned_shift || n_queries < 1 || n_queries > 8) return fail(ILSM_ERR_INVALID_ARG, "sc_prefilter_debug: bad argument");
   ScDb& d = sc->d;
   Ctx& c = *d.ctx;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
-  if (n_search < 0) n_search = d.count;
+  ILSM_ENTER(c);
+  n_search = d.searched(n_search);
   if (n_search < 1 || n_search > d.count) return fail(ILSM_ERR_INVALID_ARG, "sc_prefilter_debug: bad n_search");
   int rc;
   DevBuf<unsigned char> sh;
@@ -197,9 +189,7 @@ ILSM_API int ilsm_sc_init_nccl_rank(ilsm_sc* sc, const char id[128], int n_ranks
   int rc = nccl_load();
   if (rc) return rc;
   ScDb& d = sc->d;
-  Ctx& c = *d.ctx;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
+  ILSM_ENTER(*d.ctx);
   sc_nccl_release(d);
   ncclUniqueId uid;
   memcpy(&uid, id, 128);
@@ -248,13 +238,11 @@ static int sharded_enqueue(ScDb& d, const float* d_q, int B, int n_search, int i
 
 ILSM_API int ilsm_sc_query_topk_sharded(ilsm_sc* sc, const float* desc_20x60, int n_queries, int n_search, int id_offset, int k,
                                         double* dist, int32_t* id, int32_t* shift) {
-  int rc = batch_args_ok(sc, desc_20x60, n_queries, k, dist, id, shift, "sc_query_sharded: bad argument");
+  int rc = check_batch_args(sc, desc_20x60, n_queries, k, dist && id && shift, "sc_query_sharded");
   if (rc) return rc;
   ScDb& d = sc->d;
   Ctx& c = *d.ctx;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
-  if (n_search < 0) n_search = d.count;
+  ILSM_ENTER(c);
   if ((rc = d.qbatch.reserve((size_t)n_queries * 1200 + 8))) return rc;
   ILSM_CUDA(cudaMemcpyAsync(d.qbatch.p, desc_20x60, (size_t)n_queries * 1200 * sizeof(float), cudaMemcpyHostToDevice, c.stream));
   if ((rc = sharded_enqueue(d, d.qbatch.p, n_queries, n_search, id_offset, k))) return rc;
@@ -263,15 +251,12 @@ ILSM_API int ilsm_sc_query_topk_sharded(ilsm_sc* sc, const float* desc_20x60, in
 
 ILSM_API int ilsm_sc_query_topk_sharded_dev(ilsm_sc* sc, const float* d_desc_20x60, int n_queries, int n_search, int id_offset, int k,
                                             void* d_packed_out) {
-  if (!sc || !d_desc_20x60 || !d_packed_out || n_queries < 1 || k < 1 || k > 16)
-    return fail(ILSM_ERR_INVALID_ARG, "sc_query_sharded_dev: bad argument");
+  int rc = check_batch_args(sc, d_desc_20x60, n_queries, k, d_packed_out != nullptr, "sc_query_sharded_dev");
+  if (rc) return rc;
   ScDb& d = sc->d;
   Ctx& c = *d.ctx;
-  std::lock_guard<std::mutex> lk(c.mu);
-  ILSM_CUDA(cudaSetDevice(c.device));
-  if (n_search < 0) n_search = d.count;
-  int rc = sharded_enqueue(d, d_desc_20x60, n_queries, n_search, id_offset, k);
-  if (rc) return rc;
+  ILSM_ENTER(c);
+  if ((rc = sharded_enqueue(d, d_desc_20x60, n_queries, n_search, id_offset, k))) return rc;
   ILSM_CUDA(cudaMemcpyAsync(d_packed_out, d.pk_out.p, (size_t)n_queries * 16 * k, cudaMemcpyDeviceToDevice, c.stream));
   return ILSM_OK;
 }
