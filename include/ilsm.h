@@ -350,7 +350,9 @@ ILSM_API int ilsm_slam_frame_staged(ilsm_slam* slam, const float* xyzi, int n, i
  * read): [0] upload + front-end launches, [1] wait for the previous frame's mapping (pipelined mode), [2] wait for the front
  * end, [3] gathers / VoxelGrid / odometry launches, [4] wait for the odometry, [5] tree builds + mapping stage; pipelined mode:
  * [6] launches and [7] waits of the mapping stage's own thread.  Staged mode: [2] wait for the front-end stage, [0] hand-over to it,
- * [3] odometry launches, [1] wait for the mapping stage, [4] wait for the odometry, [5] tree builds + hand-over to the mapping stage. */
+ * [3] odometry launches, [1] wait for the mapping stage, [4] wait for the odometry, [5] tree builds + hand-over to the mapping stage,
+ * [6] and [7] as in pipelined mode.  [6] and [7] of a frame are counted by the call that hands out its mapped pose, not
+ * while the frame runs: over a run they add up to the mapping stage's time for every frame whose pose was handed out. */
 ILSM_API int ilsm_slam_host_phases(ilsm_slam* slam, double out8[8]);
 
 /* ------------------------------------------------------------------- scan-to-scan odometry (laserOdometry) ---- */

@@ -12,13 +12,10 @@
 #include <string.h>
 
 #include <chrono>
-#include <atomic>
-#include <condition_variable>
-#include <deque>
 #include <new>
-#include <thread>
 
 #include "ilsm_cubemap.hpp"
+#include "ilsm_stage.hpp"
 
 struct ilsm_mapopt;
 
@@ -31,6 +28,15 @@ int mapopt_frame_core(ilsm_mapopt* mo, const float* frame_xyz, int n, int stride
 // voxel edge of the "last frame" search structures: the odometry gate is 5 m (DISTANCE_SQ_THRESHOLD 25,
 // laserOdometry.cpp:31), the clouds are sparse (a few thousand points)
 constexpr float kOdomCell = 1.0f;
+
+// The host phase clocks.  The first eight are those of ilsm_slam_host_phases, in the order include/ilsm.h documents;
+// the rest are the stage threads' detail that ILSM_STAGE_TRACE prints.
+enum Phase {
+  kFeLaunch, kWaitMapping, kWaitFrontEnd, kOdomLaunch, kWaitOdom, kMapping, kMapLaunch, kMapWait,
+  kMapTailWait, kFeStageLaunch, kFeStageWait, kFeStageGather, kNumPhases
+};
+
+static int fail_text(int code, const char* text) { return fail(code, "%s", text); }
 
 struct SlamH {
   Ctx* ctx = nullptr;
@@ -66,6 +72,8 @@ struct SlamH {
   bool async = false;
   // The mapping stage has its own host thread, like the reference's laserMapping node has its own process: its ~25
   // launches per frame (3-4 us of host time each) are issued while the caller's thread launches the next front end.
+  // At most two jobs queue: the staged loop posts frame k before it collects frame k - 1, so the mapping thread goes
+  // from one frame to the next without a round trip through the caller.
   struct MapJob {
     int n_lsharp = 0, n_lflat = 0;
     const float4 *d_lsharp = nullptr, *d_lflat = nullptr;  // this frame's slot
@@ -75,64 +83,49 @@ struct SlamH {
     long long frame = -1;
   };
   struct MapResult {
-    int rc = 0;
-    char err[256] = "";
     double q[4] = {0, 0, 0, 1}, t[3] = {0, 0, 0};
-    ilsm_reg_report report;
-    ilsm_cubemap_stats cstats;
+    ilsm_reg_report report = {};
+    ilsm_cubemap_stats cstats = {};
     long long frame = -1;
+    double phase_s[kNumPhases] = {};  // the stage's own phases, added to SlamH::phase_s when the result is taken
   };
-  // jobs and results queue up (at most two of each: the staged loop posts frame k before it collects frame k - 1, so the
-  // mapping thread goes from one frame to the next without a round trip through the caller)
-  std::deque<MapJob> jobs;
-  std::deque<MapResult> results;
-  std::thread worker;
-  std::mutex wmu;
-  std::condition_variable wcv;
-  bool stop = false;
-  int maps_in_flight = 0;
-  // queue / mailbox occupancy mirrored in atomics: a stage that finds its input empty SPINS on these for up to ~100 us
-  // before it sleeps on the condition variable -- a futex wake-up costs 10-50 us, a third of a stage's time per frame
-  std::atomic<int> n_jobs{0}, n_results{0}, n_fjobs{0}, n_fres{0};
+  Stage<MapJob, MapResult> mapping{ilsm_last_error, fail_text};
   // staged mode (ilsm_slam_create_staged): the three nodes as three stages, each with its own context (streams, scratch)
-  // and host thread like the reference's three processes -- scanRegistration on ctx0 + fworker, laserOdometry on the
-  // caller's context and thread, laserMapping on ctx2 + worker.  Frame k's front end, frame k-1's odometry and frame
+  // and host thread like the reference's three processes -- scanRegistration on ctx0 + `frontend`, laserOdometry on the
+  // caller's context and thread, laserMapping on ctx2 + `mapping`.  Frame k's front end, frame k-1's odometry and frame
   // k-2's / k-1's mapping are in flight together.
   ilsm_ctx* ctx0 = nullptr;
-  bool staged = false, fe_in_flight = false;
+  bool staged = false;
   struct FeJob {
     const float* xyzi = nullptr;
     int n = 0, stride = 16, use_aloam = 1;
     long long frame = 0;
-  } fjob;
+  };
   struct FeResult {
-    int rc = 0, use_aloam = 1;
-    char err[256] = "";
+    int use_aloam = 1;
     int counts[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     long long frame = 0;
-  } fres;
-  std::thread fworker;
-  std::mutex fmu;
-  std::condition_variable fcv;
-  bool fjob_posted = false, fres_ready = false, fstop = false;
+    double phase_s[kNumPhases] = {};
+  };
+  Stage<FeJob, FeResult> frontend{ilsm_last_error, fail_text};
   long long pushed = 0;
-  // host-side phase clock (profiling aid, read with ilsm_slam_host_phases): seconds accumulated per phase
-  double phase_s[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};  // [8..] mapping-stage detail (ILSM_STAGE_TRACE)
+  // host-side phase clock (profiling aid, ilsm_slam_host_phases): seconds per phase, written by the caller's thread only
+  double phase_s[kNumPhases] = {};
 };
 
-static inline void spin_until_nonzero(const std::atomic<int>& a, const bool* stop = nullptr) {
-  for (int i = 0; i < 4000 && a.load(std::memory_order_acquire) == 0 && !(stop && *stop); ++i) {
-#if defined(__x86_64__) || defined(__i386__)
-    __builtin_ia32_pause();
-#endif
-  }
+// a stage's oldest result, with the phase times it took added to the handle's
+template <typename Job, typename Result>
+static int take_result(SlamH& s, Stage<Job, Result>& stage, Result& r) {
+  const int rc = stage.take(r);
+  for (int i = 0; i < kNumPhases; ++i) s.phase_s[i] += r.phase_s[i];
+  return rc;
 }
 
 struct PhaseClock {
   double* acc;
   std::chrono::steady_clock::time_point t;
   explicit PhaseClock(double* a) : acc(a), t(std::chrono::steady_clock::now()) {}
-  void lap(int k) {
+  void lap(Phase k) {
     const auto n = std::chrono::steady_clock::now();
     acc[k] += std::chrono::duration<double>(n - t).count();
     t = n;
@@ -145,7 +138,7 @@ struct PhaseClock {
 // launches: uploads the frame -- a sensor_msgs/PointCloud2 blob as it is when `pc2` is set, pcl::fromROSMsg's repacking
 // (:235) then runs as a kernel -- runs the front end on f.stream and waits for the counts.
 static int frontend_counts(Ctx& f, const float* xyzi, int n, int stride_bytes, const ilsm_pc2_layout* pc2, float min_range,
-                           int cnt[8], PhaseClock& clk, int lap_launch, int lap_wait) {
+                           int cnt[8], PhaseClock& clk, Phase lap_launch, Phase lap_wait) {
   const size_t bytes = (size_t)n * stride_bytes;
   int rc;
   if ((rc = f.fe.raw.reserve((pc2 ? (size_t)n * 4 : bytes / 4) + 4))) return rc;
@@ -233,13 +226,13 @@ static int odometry_launch(SlamH& s, Ctx& c, const SlamH::FeSlot& o, const int c
 // q/t_last_curr is composed; the first frame only sets systemInited) and rebuild both "last" trees from this frame.
 static int odometry_finish(SlamH& s, Ctx& c, const SlamH::FeSlot& o, const int cnt[8], bool solve, double q_odom[4],
                            double t_odom[3], ilsm_slam_stats* stats, PhaseClock& clk) {
-  clk.lap(3);  // odometry launches
+  clk.lap(kOdomLaunch);
   if (solve) {
     ILSM_CUDA(cudaStreamSynchronize(c.stream));
     c.lm_result(s.para_q, s.para_t, stats ? &stats->odometry : nullptr);
     if (stats) stats->odometry.passes = odometry_opts().outer_iterations, stats->ran_odometry = 1;
   }
-  clk.lap(4);  // wait for the odometry
+  clk.lap(kWaitOdom);
   if (!s.inited) {
     s.inited = true;
   } else {  // t_w_curr = t_w_curr + q_w_curr * t_last_curr;  q_w_curr = q_w_curr * q_last_curr   (laserOdometry.cpp:716-717)
@@ -269,55 +262,30 @@ static int mapping_enqueue(CubeMapH& cm, const SlamH::StackSet& set, const float
   return rc;
 }
 
-// body of the mapping stage's thread: one process() iteration per posted job, enqueue + collect on the second context
-static void mapping_worker(SlamH* sp) {
-  SlamH& s = *sp;
+// one process() iteration of the mapping stage: enqueue + collect on the second context
+static int mapping_job(SlamH& s, const SlamH::MapJob& j, SlamH::MapResult& r) {
   Ctx& c2 = s.ctx2->c;
-  cudaSetDevice(c2.device);
-  for (;;) {
-    SlamH::MapJob j;
-    spin_until_nonzero(s.n_jobs, &s.stop);
-    {
-      std::unique_lock<std::mutex> lk(s.wmu);
-      s.wcv.wait(lk, [&] { return !s.jobs.empty() || s.stop; });
-      if (s.jobs.empty()) return;  // (stop is only raised once the queue has drained)
-      j = s.jobs.front();
-      s.jobs.pop_front();
-      s.n_jobs.fetch_sub(1, std::memory_order_relaxed);
-    }
-    SlamH::MapResult r;
-    r.frame = j.frame;
-    {
-      std::lock_guard<std::mutex> lk2(c2.mu);
-      memset(&r.report, 0, sizeof(r.report)), memset(&r.cstats, 0, sizeof(r.cstats));
-      cudaError_t e = cudaStreamWaitEvent(c2.stream, j.ev_in, 0);
-      r.rc = e == cudaSuccess ? ILSM_OK : fail_cuda(e, "cudaStreamWaitEvent(mapping stage)");
-      PhaseClock wclk(s.phase_s);  // [6] mapping-stage launches, [7] wait for the mapped pose (written by this thread only)
-      CubeMapH& cm = s.cube->m;
-      SlamH::StackSet& set = s.stk[j.stack_set];
-      if (!r.rc) r.rc = cm.wait_tail();
-      wclk.lap(8);  // wait for the previous frame's deferred insertion
-      if (!r.rc) r.rc = mapping_enqueue(cm, set, j.d_lsharp, j.n_lsharp, j.d_lflat, j.n_lflat, j.q_odom, j.t_odom);
-      if (!r.rc) {  // the deferred insertion (side stream) is the set's last reader
-        e = cudaEventRecord(set.ev_free, c2.aux);
-        if (e != cudaSuccess) r.rc = fail_cuda(e, "cudaEventRecord(stack set)");
-        set.free_recorded = true;
-      }
-      wclk.lap(6);
-      if (!r.rc) r.rc = cubemap_frame_collect(cm, r.q, r.t, &r.report, &r.cstats);
-      wclk.lap(7);
-      if (r.rc) snprintf(r.err, sizeof(r.err), "%s", ilsm_last_error());  // the error text is thread-local: carry it over
-    }
-    {
-      std::lock_guard<std::mutex> lk(s.wmu);
-      s.results.push_back(r);
-      s.n_results.fetch_add(1, std::memory_order_release);
-    }
-    s.wcv.notify_all();
-  }
+  std::lock_guard<std::mutex> lk(c2.mu);
+  r.frame = j.frame;
+  cudaError_t e = cudaStreamWaitEvent(c2.stream, j.ev_in, 0);
+  if (e != cudaSuccess) return fail_cuda(e, "cudaStreamWaitEvent(mapping stage)");
+  PhaseClock clk(r.phase_s);
+  CubeMapH& cm = s.cube->m;
+  SlamH::StackSet& set = s.stk[j.stack_set];
+  int rc;
+  if ((rc = cm.wait_tail())) return rc;
+  clk.lap(kMapTailWait);
+  if ((rc = mapping_enqueue(cm, set, j.d_lsharp, j.n_lsharp, j.d_lflat, j.n_lflat, j.q_odom, j.t_odom))) return rc;
+  e = cudaEventRecord(set.ev_free, c2.aux);  // the deferred insertion (side stream) is the set's last reader
+  set.free_recorded = true;
+  if (e != cudaSuccess) return fail_cuda(e, "cudaEventRecord(stack set)");
+  clk.lap(kMapLaunch);
+  if ((rc = cubemap_frame_collect(cm, r.q, r.t, &r.report, &r.cstats))) return rc;
+  clk.lap(kMapWait);
+  return ILSM_OK;
 }
 
-// hand frame `frame`, written into slot `o` and stack set frame & 1, to the mapping thread
+// hand frame `frame`, written into slot `o` and stack set frame & 1, to the mapping stage
 static void post_mapping_job(SlamH& s, const SlamH::FeSlot& o, const int cnt[8], long long frame, const double q_odom[4],
                              const double t_odom[3]) {
   SlamH::MapJob j;
@@ -325,85 +293,32 @@ static void post_mapping_job(SlamH& s, const SlamH::FeSlot& o, const int cnt[8],
   j.d_lsharp = o.lsharp.p, j.d_lflat = o.lf, j.ev_in = o.ev, j.stack_set = (int)(frame & 1);
   for (int i = 0; i < 4; ++i) j.q_odom[i] = q_odom[i];
   for (int i = 0; i < 3; ++i) j.t_odom[i] = t_odom[i];
-  {
-    std::lock_guard<std::mutex> lk(s.wmu);
-    s.jobs.push_back(j);
-    s.n_jobs.fetch_add(1, std::memory_order_release);
-  }
-  s.maps_in_flight++;
-  s.wcv.notify_all();
+  s.mapping.post(j);
 }
 
 // wait for the mapping stage's answer to its oldest job and hand it out
-static int take_mapping_result(SlamH& s, double q_map[4], double t_map[3], ilsm_slam_stats* stats, long long* frame = nullptr) {
-  spin_until_nonzero(s.n_results);
-  std::unique_lock<std::mutex> lk(s.wmu);
-  s.wcv.wait(lk, [&] { return !s.results.empty(); });
-  const SlamH::MapResult r = s.results.front();
-  s.results.pop_front();
-  s.n_results.fetch_sub(1, std::memory_order_relaxed);
-  lk.unlock();
-  s.maps_in_flight--;
-  if (frame) *frame = r.frame;
-  if (r.rc) return fail(r.rc, "%s", r.err);
+static int take_mapping_result(SlamH& s, double q_map[4], double t_map[3], ilsm_slam_stats* stats, int* frame = nullptr) {
+  SlamH::MapResult r;
+  const int rc = take_result(s, s.mapping, r);
+  if (rc) return rc;
+  if (frame) *frame = (int)r.frame;
   for (int i = 0; i < 4; ++i) q_map[i] = r.q[i];
   for (int i = 0; i < 3; ++i) t_map[i] = r.t[i];
   if (stats) stats->mapping = r.report, stats->cubemap = r.cstats;
   return ILSM_OK;
 }
 
-// ---- staged mode: scanRegistration as its own stage
-static int frontend_stage(SlamH& s, Ctx& f, const SlamH::FeJob& j, SlamH::FeResult& r) {
-  PhaseClock fclk(s.phase_s);  // [9] upload + front-end launches, [10] wait for the feature counts, [11] gathers (this thread only)
+// ---- staged mode: scanRegistration as its own stage, on ctx0
+static int frontend_job(SlamH& s, const SlamH::FeJob& j, SlamH::FeResult& r) {
+  Ctx& f = s.ctx0->c;
+  std::lock_guard<std::mutex> lk(f.mu);
+  r.frame = j.frame, r.use_aloam = j.use_aloam;
+  PhaseClock clk(r.phase_s);
   int rc;
-  if ((rc = frontend_counts(f, j.xyzi, j.n, j.stride, nullptr, s.min_range, r.counts, fclk, 9, 10)) ||
+  if ((rc = frontend_counts(f, j.xyzi, j.n, j.stride, nullptr, s.min_range, r.counts, clk, kFeStageLaunch, kFeStageWait)) ||
       (rc = frontend_gather(f, r.counts, s.fslot[j.frame % 3], true)))
     return rc;
-  fclk.lap(11);
-  return ILSM_OK;
-}
-
-static void frontend_worker(SlamH* sp) {
-  SlamH& s = *sp;
-  Ctx& f = s.ctx0->c;
-  cudaSetDevice(f.device);
-  for (;;) {
-    SlamH::FeJob j;
-    spin_until_nonzero(s.n_fjobs, &s.fstop);
-    {
-      std::unique_lock<std::mutex> lk(s.fmu);
-      s.fcv.wait(lk, [&] { return s.fjob_posted || s.fstop; });
-      if (s.fstop) return;
-      j = s.fjob;
-      s.fjob_posted = false;
-      s.n_fjobs.store(0, std::memory_order_relaxed);
-    }
-    SlamH::FeResult r;
-    r.frame = j.frame, r.use_aloam = j.use_aloam;
-    {
-      std::lock_guard<std::mutex> lk2(f.mu);
-      r.rc = frontend_stage(s, f, j, r);
-      if (r.rc) snprintf(r.err, sizeof(r.err), "%s", ilsm_last_error());
-    }
-    {
-      std::lock_guard<std::mutex> lk(s.fmu);
-      s.fres = r;
-      s.fres_ready = true;
-      s.n_fres.store(1, std::memory_order_release);
-    }
-    s.fcv.notify_all();
-  }
-}
-
-static int take_frontend_result(SlamH& s, SlamH::FeResult* out) {
-  spin_until_nonzero(s.n_fres);
-  std::unique_lock<std::mutex> lk(s.fmu);
-  s.fcv.wait(lk, [&] { return s.fres_ready; });
-  s.fres_ready = false;
-  s.n_fres.store(0, std::memory_order_relaxed);
-  s.fe_in_flight = false;
-  *out = s.fres;
-  if (out->rc) return fail(out->rc, "%s", out->err);
+  clk.lap(kFeStageGather);
   return ILSM_OK;
 }
 
@@ -463,7 +378,9 @@ static int slam_create_mapping_stage(ilsm_slam* h, float line_res, float plane_r
   if ((rc = ilsm_create(h->s.ctx->device, &h->s.ctx2)) ||
       (rc = ilsm_cubemap_create(h->s.ctx2, line_res, plane_res, cube_capacity, &h->s.cube)))
     return rc;
-  h->s.worker = std::thread(mapping_worker, &h->s);
+  SlamH* s = &h->s;
+  s->mapping.start([s] { cudaSetDevice(s->ctx2->c.device); },
+                   [s](const SlamH::MapJob& j, SlamH::MapResult& r) { return mapping_job(*s, j, r); });
   return ILSM_OK;
 }
 
@@ -517,7 +434,9 @@ ILSM_API int ilsm_slam_create_staged(ilsm_ctx* ctx, float line_res, float plane_
     ilsm_slam_destroy(h);
     return rc;
   }
-  h->s.fworker = std::thread(frontend_worker, &h->s);
+  SlamH* s = &h->s;
+  s->frontend.start([s] { cudaSetDevice(s->ctx0->c.device); },
+                    [s](const SlamH::FeJob& j, SlamH::FeResult& r) { return frontend_job(*s, j, r); });
   *out = h;
   return ILSM_OK;
 }
@@ -525,35 +444,19 @@ ILSM_API int ilsm_slam_create_staged(ilsm_ctx* ctx, float line_res, float plane_
 ILSM_API void ilsm_slam_destroy(ilsm_slam* slam) {
   if (!slam) return;
   SlamH& s = slam->s;
-  if (s.fworker.joinable()) {
-    {
-      std::unique_lock<std::mutex> lk(s.fmu);
-      s.fcv.wait(lk, [&] { return !s.fjob_posted; });
-      s.fstop = true;
-    }
-    s.fcv.notify_all();
-    s.fworker.join();
-  }
+  s.frontend.stop();
+  const double us = 1e6 / (s.frames ? s.frames : 1);  // per frame
   if (getenv("ILSM_STAGE_TRACE"))
     fprintf(stderr, "[ilsm stage trace] frames %lld  mapping: tail-wait %.1f us  enqueue %.1f us  collect %.1f us   front end: launches %.1f us  "
                     "wait %.1f us  gathers %.1f us per frame\n", s.frames,
-            1e6 * s.phase_s[8] / (s.frames ? s.frames : 1), 1e6 * s.phase_s[6] / (s.frames ? s.frames : 1),
-            1e6 * s.phase_s[7] / (s.frames ? s.frames : 1), 1e6 * s.phase_s[9] / (s.frames ? s.frames : 1),
-            1e6 * s.phase_s[10] / (s.frames ? s.frames : 1), 1e6 * s.phase_s[11] / (s.frames ? s.frames : 1));
+            us * s.phase_s[kMapTailWait], us * s.phase_s[kMapLaunch], us * s.phase_s[kMapWait], us * s.phase_s[kFeStageLaunch],
+            us * s.phase_s[kFeStageWait], us * s.phase_s[kFeStageGather]);
   if (s.ctx0) {
     std::lock_guard<std::mutex> lk0(s.ctx0->c.mu);
     cudaSetDevice(s.ctx0->c.device);
     cudaStreamSynchronize(s.ctx0->c.stream);
   }
-  if (s.worker.joinable()) {
-    {
-      std::unique_lock<std::mutex> lk(s.wmu);
-      s.wcv.wait(lk, [&] { return s.jobs.empty(); });  // posted jobs are taken (and finished) before the thread is told to stop
-      s.stop = true;
-    }
-    s.wcv.notify_all();
-    s.worker.join();
-  }
+  s.mapping.stop();
   if (s.ctx2) {  // let the mapping stage drain before anything it reads goes away
     std::lock_guard<std::mutex> lk2(s.ctx2->c.mu);
     cudaSetDevice(s.ctx2->c.device);
@@ -620,7 +523,7 @@ ILSM_API int ilsm_slam_flush(ilsm_slam* slam, double q_map[4], double t_map[3], 
   SlamH& s = slam->s;
   *have = 0;
   if (s.staged) return fail(ILSM_ERR_STATE, "slam_flush: staged handles drain with ilsm_slam_frame_staged(n = -1)");
-  if (!s.async || s.maps_in_flight == 0) return ILSM_OK;
+  if (!s.async || s.mapping.in_flight() == 0) return ILSM_OK;
   std::lock_guard<std::mutex> lk(s.ctx->mu);
   int rc = take_mapping_result(s, q_map, t_map, stats);
   if (rc) return rc;
@@ -650,13 +553,13 @@ static int slam_frame_impl(ilsm_slam* slam, const float* xyzi, int n, int stride
   // frame's front end after them
   if ((rc = s.last_corner.wait_ready(c.stream)) || (rc = s.last_surf.wait_ready(c.stream))) return rc;
   int cnt[8];
-  if ((rc = frontend_counts(c, xyzi, n, stride_bytes, pc2, s.min_range, cnt, clk, 0, 2))) return rc;
-  if (s.async && s.maps_in_flight > 0) {
+  if ((rc = frontend_counts(c, xyzi, n, stride_bytes, pc2, s.min_range, cnt, clk, kFeLaunch, kWaitFrontEnd))) return rc;
+  if (s.async && s.mapping.in_flight() > 0) {
     // the previous frame's mapped pose: the mapping stage's thread has had this frame's upload and front end to finish
     if ((rc = take_mapping_result(s, q_map, t_map, stats))) return rc;
     *have_prev = 1;
   }
-  clk.lap(1);  // (pipelined) wait for the previous frame's mapping
+  clk.lap(kWaitMapping);  // (pipelined)
   feature_stats(stats, cnt);
   SlamH::FeSlot& o = s.fslot[s.frames % 3];
   SlamH::StackSet& set = s.stk[s.frames & 1];
@@ -694,7 +597,7 @@ static int slam_frame_impl(ilsm_slam* slam, const float* xyzi, int n, int stride
       stats->cubemap.n_valid = ms.converged;
     }
   }
-  clk.lap(5);  // tree builds + mapping stage (synchronous: enqueue and wait; pipelined: enqueue only)
+  clk.lap(kMapping);  // synchronous: enqueue and wait; pipelined: enqueue only
   if (rc) return rc;
   s.frames++;
   return ILSM_OK;
@@ -718,28 +621,14 @@ extern "C" ILSM_API int ilsm_slam_frame_staged(ilsm_slam* slam, const float* xyz
   int rc;
   PhaseClock clk(s.phase_s);
   SlamH::FeResult fr;
-  const bool have_fe = s.fe_in_flight;
-  if (have_fe && (rc = take_frontend_result(s, &fr))) return rc;
-  clk.lap(2);  // wait for the front-end stage
-  if (n >= 0) {
-    {
-      std::lock_guard<std::mutex> lkf(s.fmu);
-      s.fjob.xyzi = xyzi, s.fjob.n = n, s.fjob.stride = stride_bytes, s.fjob.use_aloam = use_aloam, s.fjob.frame = s.pushed;
-      s.fjob_posted = true;
-      s.n_fjobs.store(1, std::memory_order_release);
-    }
-    s.fcv.notify_all();
-    s.fe_in_flight = true;
-    s.pushed++;
-  }
-  clk.lap(0);  // hand-over to the front-end stage
+  const bool have_fe = s.frontend.in_flight() > 0;
+  if (have_fe && (rc = take_result(s, s.frontend, fr))) return rc;
+  clk.lap(kWaitFrontEnd);
+  if (n >= 0) s.frontend.post({xyzi, n, stride_bytes, use_aloam, s.pushed++});
+  clk.lap(kFeLaunch);  // hand-over to the front-end stage
   if (!have_fe) {  // nothing for the odometry: first call, or the pipeline is draining
-    if (s.maps_in_flight > 0) {
-      long long mf = -1;
-      if ((rc = take_mapping_result(s, q_map, t_map, stats, &mf))) return rc;
-      *map_frame = (int)mf;
-    }
-    clk.lap(1);
+    if (s.mapping.in_flight() > 0 && (rc = take_mapping_result(s, q_map, t_map, stats, map_frame))) return rc;
+    clk.lap(kWaitMapping);
     return ILSM_OK;
   }
   const int* cnt = fr.counts;
@@ -756,15 +645,11 @@ extern "C" ILSM_API int ilsm_slam_frame_staged(ilsm_slam* slam, const float* xyz
   *odom_frame = (int)fr.frame;
   // this frame goes to the mapping stage BEFORE the previous frame's result is collected: the mapping thread moves on to
   // it the moment it has finished the previous one
-  const bool collect_prev = s.maps_in_flight > 0;
+  const bool collect_prev = s.mapping.in_flight() > 0;
   post_mapping_job(s, o, cnt, fr.frame, q_odom, t_odom);
-  clk.lap(5);  // tree builds + hand-over to the mapping stage
-  if (collect_prev) {
-    long long mf = -1;
-    if ((rc = take_mapping_result(s, q_map, t_map, stats, &mf))) return rc;
-    *map_frame = (int)mf;
-  }
-  clk.lap(1);  // wait for the mapping stage (the frame before)
+  clk.lap(kMapping);  // tree builds + hand-over to the mapping stage
+  if (collect_prev && (rc = take_mapping_result(s, q_map, t_map, stats, map_frame))) return rc;
+  clk.lap(kWaitMapping);  // the frame before
   s.frames++;
   return ILSM_OK;
 }
