@@ -705,6 +705,64 @@ ILSM_API int ilsm_icp_align_batch_dev(ilsm_ctx* ctx, ilsm_map* const* targets, i
                                       const int* src_offsets, int stride_bytes, const double* guess7,
                                       const ilsm_icp_opts* opts, ilsm_icp_result* results);
 
+/* ------------------------------------------- K7: loop closure per keyframe against a resident keyframe store ---- */
+/* One handle per loop-closure thread (give it its own ilsm_ctx, the way the reference runs loopClosureThread on its own
+ * thread).  Every keyframe passed in is stored on the device -- its ScanContext descriptor, VoxelGrid(leaf) of its cloud and
+ * its pose -- and answered with that keyframe's loop decision; choosing which frames are keyframes stays with the caller.
+ * Replaces: the body of loopClosureThread (intensity_feature_tracker.cpp:195-393) around SCManager::
+ *           makeAndSaveScancontextAndKeys + detectLoopClosureID (Scancontext.cpp:237-344) and the ICP check. */
+typedef struct ilsm_loop ilsm_loop;
+
+typedef struct ilsm_loop_opts {
+  int32_t exclude_recent;     /* NUM_EXCLUDE_RECENT = 50; >= 1 */
+  int32_t tree_period;        /* TREE_MAKING_PERIOD_ = 50; >= 1 */
+  int32_t num_candidates;     /* NUM_CANDIDATES_FROM_TREE = 10; 1..16 */
+  int32_t submap_half;        /* target = keyframes c-h .. c+h; 0..7 (2) */
+  double sc_dist_threshold;   /* SC_DIST_THRES = 0.13: a loop iff min_dist < this */
+  float leaf;                 /* VoxelGrid leaf of the stored keyframes and of the submap (0.4); > 0 */
+  float cell;                 /* k-NN cell of the submap's map (1.0); > 0 */
+  double fitness_threshold;   /* accepted iff the ICP converged && fitness < this (0.3) */
+  ilsm_icp_opts icp;          /* 2.0 m, 50 iterations, transformation_epsilon 1e-8, euclidean_fitness_epsilon 1e-6 */
+} ilsm_loop_opts;
+
+typedef struct ilsm_loop_result {
+  int32_t keyframe_id;   /* id of this keyframe (0, 1, 2, ... in call order) */
+  int32_t loop_id;       /* detectLoopClosureID's loop id, -1: none */
+  int32_t nn_id;         /* best candidate, -1: early return (fewer than exclude_recent + 1 keyframes) */
+  int32_t shift;         /* its aligning column shift (sectors of 6 degrees) */
+  double sc_dist;        /* its distance (min_dist) */
+  double yaw_diff_rad;   /* deg2rad(shift * 6) as the reference returns it (a float) */
+  int32_t verified;      /* 1 when loop_id >= 0: the ICP ran */
+  int32_t accepted;      /* verified && icp.converged && icp.fitness < fitness_threshold */
+  int32_t submap_first, submap_last; /* the target's keyframes: [loop_id - h, loop_id + h] within [0, size - exclude_recent) */
+  int32_t submap_points; /* VoxelGrid(leaf) size of the world-frame target */
+  int32_t reserved;
+  double q_rel_xyzw[4], t_rel[3]; /* when accepted: T_loop^-1 * T_icp, this keyframe in the frame of keyframe loop_id */
+  ilsm_icp_result icp;   /* when verified: the world pose of this keyframe ICP found (source = this keyframe's stored
+                            cloud, guess = (q_loop * Rz(-yaw_diff_rad), t_loop)) */
+} ilsm_loop_result;
+
+/* The values above. */
+ILSM_API void ilsm_loop_opts_default(ilsm_loop_opts* o);
+/* opts NULL: the defaults; options outside the ranges above: ILSM_ERR_INVALID_ARG.  ILSM_ERR_NO_DEVICE without a GPU. */
+ILSM_API int ilsm_loop_create(ilsm_ctx* ctx, const ilsm_loop_opts* opts, ilsm_loop** out);
+ILSM_API void ilsm_loop_destroy(ilsm_loop* loop);
+/* keyframes stored */
+ILSM_API int ilsm_loop_size(const ilsm_loop* loop);
+/* Store one keyframe (n xyzi points, stride_bytes >= 16, intensity at the fourth float, or the fifth from 32 bytes; n < 2^24)
+ * with its world pose (q unit within 1e-6, else ILSM_ERR_INVALID_ARG) and return its loop decision in *result:
+ *   detect  SCManager's state machine -- fewer than exclude_recent + 1 keyframes: early return, the refresh counter stays;
+ *           every tree_period-th search the searchable size becomes size - exclude_recent; the num_candidates nearest
+ *           ring keys are scored (ilsm_sc_query_candidates), the first strict minimum wins, min_dist < sc_dist_threshold;
+ *   verify  with a loop: keyframes [c-h, c+h] of the store to the world frame (double math, float store), VoxelGrid(leaf),
+ *           a map with cell `cell`, one ICP pair (ilsm_icp_align_batch) from the guess above.
+ * One host synchronisation per call; two more for a verified keyframe.  The _dev form reads the points from device memory.
+ * Argument errors come back before any CUDA call. */
+ILSM_API int ilsm_loop_add_keyframe(ilsm_loop* loop, const float* xyz, int n, int stride_bytes, const double q_xyzw[4],
+                                    const double t_xyz[3], ilsm_loop_result* result);
+ILSM_API int ilsm_loop_add_keyframe_dev(ilsm_loop* loop, const float* d_xyz, int n, int stride_bytes, const double q_xyzw[4],
+                                        const double t_xyz[3], ilsm_loop_result* result);
+
 #ifdef __cplusplus
 }
 #endif

@@ -496,6 +496,37 @@ class IterativeClosestPoint {
   Matrix4f final_;
 };
 
+// ------------------------------------------------------------------------------------------------ loop closure per keyframe
+// The body of loopClosureThread (intensity_feature_tracker.cpp:195-393) over ilsm_loop: every keyframe passed in is stored
+// on the device and answered with its loop decision (ScanContext detection, ICP verification of the best candidate
+// against the world-frame submap of its neighbours).  Give it a Context of its own when the mapping loop runs on another
+// thread, as the reference runs loopClosureThread on its own.
+class LoopClosure {
+ public:
+  explicit LoopClosure(ContextPtr ctx = Context::shared(), const ilsm_loop_opts* opts = nullptr) : ctx_(std::move(ctx)) {
+    check(ilsm_loop_create(ctx_->get(), opts, &h_), "ilsm_loop_create");
+  }
+  ~LoopClosure() { ilsm_loop_destroy(h_); }
+  LoopClosure(const LoopClosure&) = delete;
+  LoopClosure& operator=(const LoopClosure&) = delete;
+
+  // cloud: the keyframe's points (16- or 32-byte PCL points) in its own frame; (q, t): its world pose.  Returns
+  // result->accepted.
+  template <typename CloudT>
+  bool addKeyframe(const CloudT& cloud, const double q_xyzw[4], const double t_xyz[3], ilsm_loop_result* result) {
+    typedef typename std::remove_reference<decltype(cloud.points[0])>::type P;
+    check(ilsm_loop_add_keyframe(h_, cloud_ptr(cloud), (int)cloud.points.size(), stride_of<P>(), q_xyzw, t_xyz, result),
+          "LoopClosure::addKeyframe");
+    return result->accepted != 0;
+  }
+  int size() const { return ilsm_loop_size(h_); }
+  ilsm_loop* handle() const { return h_; }
+
+ private:
+  ContextPtr ctx_;
+  ilsm_loop* h_ = nullptr;
+};
+
 // ------------------------------------------------------------------------------------------------ ImageHandler
 class ImageHandler {
  public:

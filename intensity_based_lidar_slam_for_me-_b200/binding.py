@@ -118,6 +118,37 @@ class IcpResult(C.Structure):
         return np.array(self.t[:], np.float64)
 
 
+class LoopOpts(C.Structure):
+    """ilsm_loop_opts; LoopOpts() holds the library's defaults (the reference's constants, the ICP settings of the tests)."""
+    _fields_ = [("exclude_recent", C.c_int32), ("tree_period", C.c_int32), ("num_candidates", C.c_int32), ("submap_half", C.c_int32),
+                ("sc_dist_threshold", C.c_double), ("leaf", C.c_float), ("cell", C.c_float), ("fitness_threshold", C.c_double),
+                ("icp", IcpOpts)]
+
+    def __init__(self, icp=None, **kw):
+        super().__init__()
+        load_library().ilsm_loop_opts_default(C.byref(self))
+        for k, v in kw.items():
+            setattr(self, k, v)
+        for k, v in (icp or {}).items():
+            setattr(self.icp, k, v)
+
+
+class LoopResult(C.Structure):
+    """ilsm_loop_result: one keyframe's loop decision; .q / .tv = T_loop^-1 * T_icp (filled when accepted)."""
+    _fields_ = [("keyframe_id", C.c_int32), ("loop_id", C.c_int32), ("nn_id", C.c_int32), ("shift", C.c_int32),
+                ("sc_dist", C.c_double), ("yaw_diff_rad", C.c_double), ("verified", C.c_int32), ("accepted", C.c_int32),
+                ("submap_first", C.c_int32), ("submap_last", C.c_int32), ("submap_points", C.c_int32), ("reserved", C.c_int32),
+                ("q_rel_xyzw", C.c_double * 4), ("t_rel", C.c_double * 3), ("icp", IcpResult)]
+
+    @property
+    def q(self):
+        return np.array(self.q_rel_xyzw[:], np.float64)
+
+    @property
+    def tv(self):
+        return np.array(self.t_rel[:], np.float64)
+
+
 DMATCH_DTYPE = np.dtype([("queryIdx", "<i4"), ("trainIdx", "<i4"), ("imgIdx", "<i4"), ("distance", "<f4")])
 FACTOR_DTYPE = np.dtype([("type", "<i4"), ("src", "<i4"), ("p", "<f8", 3), ("a", "<f8", 3), ("b", "<f8", 3)])
 
@@ -237,6 +268,12 @@ def load_library(path: str | None = None):
         "ilsm_icp_opts_default": (None, [C.POINTER(IcpOpts)]),
         "ilsm_icp_align_batch": (i32, [vp, vp, i32, vp, vp, i32, vp, C.POINTER(IcpOpts), vp]),
         "ilsm_icp_align_batch_dev": (i32, [vp, vp, i32, vp, vp, i32, vp, C.POINTER(IcpOpts), vp]),
+        "ilsm_loop_opts_default": (None, [C.POINTER(LoopOpts)]),
+        "ilsm_loop_create": (i32, [vp, C.POINTER(LoopOpts), C.POINTER(vp)]),
+        "ilsm_loop_destroy": (None, [vp]),
+        "ilsm_loop_size": (i32, [vp]),
+        "ilsm_loop_add_keyframe": (i32, [vp, vp, i32, i32, vp, vp, C.POINTER(LoopResult)]),
+        "ilsm_loop_add_keyframe_dev": (i32, [vp, vp, i32, i32, vp, vp, C.POINTER(LoopResult)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
@@ -593,6 +630,59 @@ class LocalMap:
 
     def knn_dev(self, d_q_ptr: int, nq: int, stride: int, k: int, max_dist: float, d_idx_ptr: int, d_d2_ptr: int):
         _check(self._lib.ilsm_knn_dev(self._h, d_q_ptr, nq, stride, k, max_dist, d_idx_ptr, d_d2_ptr))
+
+
+class LoopClosure:
+    """ilsm_loop: loopClosureThread's body per keyframe -- ScanContext store and detection, ICP verification of the best
+    candidate against a world-frame submap of the stored keyframes.  opts: LoopOpts fields (icp=dict of IcpOpts fields).
+    Give it a Context of its own when the mapping loop runs on another thread."""
+
+    def __init__(self, ctx: Context, **opts):
+        self._ctx = ctx
+        self._lib = ctx._lib
+        o = LoopOpts(**opts)
+        h = C.c_void_p()
+        _check(self._lib.ilsm_loop_create(ctx._h, C.byref(o), C.byref(h)))
+        self._h = h
+
+    def close(self):
+        if getattr(self, "_h", None) and getattr(self._ctx, "_h", None):
+            self._lib.ilsm_loop_destroy(self._h)
+        self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __len__(self):
+        return int(self._lib.ilsm_loop_size(self._h))
+
+    @staticmethod
+    def _pose(q, t):
+        return np.ascontiguousarray(q, np.float64).reshape(4), np.ascontiguousarray(t, np.float64).reshape(3)
+
+    def add_keyframe(self, cloud, q, t) -> LoopResult:
+        """cloud: (n, >=3) points in the keyframe's frame (xyz-only clouds get intensity 0); (q, t): its world pose."""
+        a = np.asarray(cloud, np.float32)
+        if a.ndim == 2 and a.shape[1] == 3:
+            a = np.concatenate([a, np.zeros((len(a), 1), np.float32)], axis=1)
+        a, n, stride = _cloud(a)
+        qq, tt = self._pose(q, t)
+        r = LoopResult()
+        _check(self._lib.ilsm_loop_add_keyframe(self._h, _ptr(a), n, stride, _ptr(qq), _ptr(tt), C.byref(r)))
+        return r
+
+    def add_keyframe_dev(self, tensor, q, t) -> LoopResult:
+        """tensor: a CUDA float32 (n, >=4) tensor with contiguous rows, ready on the device (synchronise its stream first)."""
+        if tensor.dtype.itemsize != 4 or tensor.dim() != 2 or tensor.shape[1] < 4 or tensor.stride(1) != 1 or not tensor.is_cuda:
+            raise ValueError("add_keyframe_dev needs a CUDA float32 (n, >=4) tensor with contiguous rows")
+        qq, tt = self._pose(q, t)
+        r = LoopResult()
+        _check(self._lib.ilsm_loop_add_keyframe_dev(self._h, tensor.data_ptr(), tensor.shape[0], 4 * tensor.stride(0), _ptr(qq),
+                                                    _ptr(tt), C.byref(r)))
+        return r
 
 
 def merge_topk(dist, ids, shifts, k):

@@ -434,6 +434,20 @@ def loop_keyframes(n_per_lap=12, laps=2, radius=8.0, leaf=0.4, seed=0x5EED1C00, 
     return out
 
 
+def revisit_keyframe(kf, yaw_deg, offset=-0.1, seed=77, leaf=0.4, scene=None):
+    """Keyframe `kf` (of loop_keyframes) re-observed `offset` m further from the loop centre (default: 0.1 m nearer) with
+    its yaw turned by `yaw_deg`: the same place seen at another heading.  Same fields as a loop keyframe (q, t, src,
+    world)."""
+    scene = scene or Scene()
+    out = np.array([kf["t"][0], kf["t"][1], 0.0])
+    t = np.asarray(kf["t"], np.float64) + offset * out / np.linalg.norm(out)
+    q = quat_mul(kf["q"], quat_from_rotvec([0.0, 0.0, np.deg2rad(yaw_deg)]))
+    cloud, _ = make_frame(scene, q, t, seed=seed)
+    src = voxel_centroid_np(cloud[np.any(cloud[:, :3] != 0, axis=1), :3], leaf)
+    world = (src.astype(np.float64) @ quat_to_mat(q).T + t).astype(np.float32)
+    return dict(q=q, t=t, src=src, world=world, lap=-1, k=kf["k"])
+
+
 def loop_submap(kfs, c, n_per_lap, half=2, leaf=0.4):
     """World-frame submap around keyframe c: keyframes c-half .. c+half of c's lap (cyclic), VoxelGrid(leaf)."""
     lap0 = (c // n_per_lap) * n_per_lap
