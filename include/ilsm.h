@@ -763,6 +763,47 @@ ILSM_API int ilsm_loop_add_keyframe(ilsm_loop* loop, const float* xyz, int n, in
 ILSM_API int ilsm_loop_add_keyframe_dev(ilsm_loop* loop, const float* d_xyz, int n, int stride_bytes, const double q_xyzw[4],
                                         const double t_xyz[3], ilsm_loop_result* result);
 
+/* ---------------------------------------------- the full loop with loop closure as its own stage ---- */
+/* A full-loop handle (ilsm_slam, every kind) can run loop closure beside mapping, the way the reference runs
+ * loopClosureThread beside its mapping loop.  Every mapped pose the handle hands out is checked against the keyframe rule:
+ * frame k is a keyframe when it is the first frame handed out, or when ||t_k - t_kf|| >= keyframe_dist, or when
+ * 2 atan2(||v||, |w|) >= keyframe_angle_rad for (v, w) = q_kf^-1 * q_k, where (q_kf, t_kf) is the mapped pose of the last
+ * keyframe (fp64 on the host; DESIGN section 2 gives the order of operations).  Both thresholds 0: every frame is one.
+ * A keyframe's cloud never leaves the device: the front end's ring-ordered cloud (/velodyne_cloud_2, what
+ * ilsm_extract_features returns as cloud_xyzi, n_cloud points of 16 bytes, after the range filter) is copied into one of
+ * max_pending device buffers and handed, with the mapped pose, to an ilsm_loop on a context and host thread the handle
+ * owns.  The cloud's fourth float is scanID + 0.1 relTime, not intensity; neither ScanContext nor the ICP reads it.
+ * Loop closure only reads: every odometry and mapped pose is bit-identical to the same handle without it. */
+typedef struct ilsm_slam_loop_opts {
+  double keyframe_dist;       /* m (1.0); finite, >= 0 */
+  double keyframe_angle_rad;  /* (0.2); finite, >= 0 */
+  int32_t max_pending;        /* keyframes handed to the loop stage and not yet answered before a frame call waits (8); >= 1 */
+  int32_t reserved;
+  ilsm_loop_opts loop;        /* the loop handle's options (ilsm_loop_opts_default) */
+} ilsm_slam_loop_opts;
+
+typedef struct ilsm_slam_loop_event {
+  int64_t frame;              /* index of the frame that became the keyframe, 0-based in hand-in order */
+  double q_xyzw[4], t[3];     /* its mapped pose, as stored */
+  ilsm_loop_result result;    /* its loop decision; result.keyframe_id = 0, 1, 2, ... */
+} ilsm_slam_loop_event;
+
+/* keyframe_dist 1.0, keyframe_angle_rad 0.2, max_pending 8, loop = ilsm_loop_opts_default */
+ILSM_API void ilsm_slam_loop_opts_default(ilsm_slam_loop_opts* o);
+/* Turn loop closure on.  opts NULL: the defaults.  Call before the first frame (ILSM_ERR_STATE after it, or when it is
+ * already on).  Options outside the ranges above, including those of ilsm_loop_create: ILSM_ERR_INVALID_ARG, before any
+ * CUDA call; ILSM_ERR_NO_DEVICE without a GPU.  The slot and pending buffers are reserved here, at 65 536 points.
+ * A frame call waits for loop closure only when a new keyframe finds all max_pending buffers in flight: it then waits
+ * for the oldest answer and queues it for ilsm_slam_loop_results. */
+ILSM_API int ilsm_slam_enable_loop(ilsm_slam* slam, const ilsm_slam_loop_opts* opts);
+/* The decisions of the keyframes answered so far, in keyframe order, at most `capacity` of them into out[0 .. *n_out).
+ * wait != 0: first wait until every keyframe selected so far has been answered.  The rest stay queued for the next call.
+ * Call it from the thread that hands in the frames, not during a frame call; it takes no context lock.  ILSM_ERR_STATE on a
+ * handle without loop closure.  A keyframe that failed (on the loop stage, or while being handed over) is reported here
+ * and only here, in keyframe order: the call that reaches it with nothing handed out before it returns its status and
+ * error text and drops it; later keyframes stay queued.  Frame calls never return loop-closure errors. */
+ILSM_API int ilsm_slam_loop_results(ilsm_slam* slam, int wait, ilsm_slam_loop_event* out, int capacity, int* n_out);
+
 #ifdef __cplusplus
 }
 #endif

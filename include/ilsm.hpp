@@ -716,6 +716,20 @@ class MapOptimization {
   ilsm_mapopt* mo_ = nullptr;
 };
 
+// Loop closure of a full-loop handle (ilsm_slam_enable_loop / ilsm_slam_loop_results), shared by LoamPipeline and
+// StagedLoamPipeline: enable before the first frame; collect the decisions of the keyframes answered so far (wait: first
+// wait for every keyframe selected so far), appended to `out` in keyframe order.
+inline void slam_enable_loop(ilsm_slam* slam, const ilsm_slam_loop_opts& opts) {
+  check(ilsm_slam_enable_loop(slam, &opts), "ilsm_slam_enable_loop");
+}
+inline void slam_loop_results(ilsm_slam* slam, std::vector<ilsm_slam_loop_event>& out, bool wait) {
+  ilsm_slam_loop_event buf[32];
+  for (int n = 32; n == 32;) {
+    check(ilsm_slam_loop_results(slam, wait ? 1 : 0, buf, 32, &n), "ilsm_slam_loop_results");
+    out.insert(out.end(), buf, buf + n);
+  }
+}
+
 // The three LiDAR nodes chained on one GPU (ilsm_slam): scanRegistration -> laserOdometry -> laserMapping, inter-node
 // clouds resident in HBM.  pipelined = true runs laserMapping as its own stage (second context + host thread inside the
 // handle, like the reference's separate node): frame() then returns the mapped pose of the PREVIOUS frame
@@ -757,6 +771,8 @@ class LoamPipeline {
     has_mapped_pose = have != 0;
     return has_mapped_pose;
   }
+  void enableLoopClosure(const ilsm_slam_loop_opts& opts) { slam_enable_loop(slam_, opts); }
+  void loopResults(std::vector<ilsm_slam_loop_event>& out, bool wait) { slam_loop_results(slam_, out, wait); }
   ilsm_slam* handle() const { return slam_; }
 
  private:
@@ -799,6 +815,8 @@ class StagedLoamPipeline {
     check(ilsm_slam_frame_staged(slam_, nullptr, -1, 16, 1, q_odom, t_odom, &odom_frame, q_map, t_map, &map_frame, &stats),
           "ilsm_slam_frame_staged");
   }
+  void enableLoopClosure(const ilsm_slam_loop_opts& opts) { slam_enable_loop(slam_, opts); }
+  void loopResults(std::vector<ilsm_slam_loop_event>& out, bool wait) { slam_loop_results(slam_, out, wait); }
   ilsm_slam* handle() const { return slam_; }
 
  private:

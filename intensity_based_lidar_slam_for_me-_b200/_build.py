@@ -12,8 +12,11 @@ LIB = os.path.join(HERE, "libilsm_cuda.so")
 
 NVCC_FLAGS = [
     "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
-    "-Xcompiler", "-fPIC,-fvisibility=hidden",
+    "-Xcompiler", "-fPIC,-fvisibility=hidden,-ffp-contract=off",
 ]
+# Host code is never contracted either (-ffp-contract=off): fp64 rules a caller restates bit for bit, like the full loop's
+# keyframe rule (csrc/ilsm_keyframe.hpp), must not depend on whether the host ISA has FMA (x86-64 baseline has none,
+# AArch64 has it and GCC contracts there by default).
 # Parity with the reference's x86-64 SSE2 build (CMakeLists.txt:5-6, no FMA): files whose float results are compared
 # bit for bit are compiled without a*b+c contraction.  registration.cu keeps its bit-exact parts (pose transform,
 # float distances) in explicit round-to-nearest intrinsics and is compared with a tolerance elsewhere (fits, residuals,

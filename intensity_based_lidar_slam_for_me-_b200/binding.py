@@ -149,6 +149,37 @@ class LoopResult(C.Structure):
         return np.array(self.t_rel[:], np.float64)
 
 
+class SlamLoopOpts(C.Structure):
+    """ilsm_slam_loop_opts: the keyframe rule and the loop stage of a full-loop handle; SlamLoopOpts() holds the defaults."""
+    _fields_ = [("keyframe_dist", C.c_double), ("keyframe_angle_rad", C.c_double), ("max_pending", C.c_int32),
+                ("reserved", C.c_int32), ("loop", LoopOpts)]
+
+    def __init__(self, loop=None, **kw):
+        super().__init__()
+        load_library().ilsm_slam_loop_opts_default(C.byref(self))
+        for k, v in kw.items():
+            setattr(self, k, v)
+        for k, v in (loop or {}).items():
+            if k == "icp":
+                for ik, iv in v.items():
+                    setattr(self.loop.icp, ik, iv)
+            else:
+                setattr(self.loop, k, v)
+
+
+class SlamLoopEvent(C.Structure):
+    """ilsm_slam_loop_event: the frame that became a keyframe, its mapped pose as stored and its loop decision."""
+    _fields_ = [("frame", C.c_int64), ("q_xyzw", C.c_double * 4), ("t", C.c_double * 3), ("result", LoopResult)]
+
+    @property
+    def q(self):
+        return np.array(self.q_xyzw[:], np.float64)
+
+    @property
+    def tv(self):
+        return np.array(self.t[:], np.float64)
+
+
 DMATCH_DTYPE = np.dtype([("queryIdx", "<i4"), ("trainIdx", "<i4"), ("imgIdx", "<i4"), ("distance", "<f4")])
 FACTOR_DTYPE = np.dtype([("type", "<i4"), ("src", "<i4"), ("p", "<f8", 3), ("a", "<f8", 3), ("b", "<f8", 3)])
 
@@ -274,6 +305,9 @@ def load_library(path: str | None = None):
         "ilsm_loop_size": (i32, [vp]),
         "ilsm_loop_add_keyframe": (i32, [vp, vp, i32, i32, vp, vp, C.POINTER(LoopResult)]),
         "ilsm_loop_add_keyframe_dev": (i32, [vp, vp, i32, i32, vp, vp, C.POINTER(LoopResult)]),
+        "ilsm_slam_loop_opts_default": (None, [C.POINTER(SlamLoopOpts)]),
+        "ilsm_slam_enable_loop": (i32, [vp, C.POINTER(SlamLoopOpts)]),
+        "ilsm_slam_loop_results": (i32, [vp, i32, C.POINTER(SlamLoopEvent), i32, C.POINTER(i32)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
@@ -976,6 +1010,30 @@ class Slam:
         st, have = SlamStats(), C.c_int32(0)
         _check(self._lib.ilsm_slam_flush(self._h, _ptr(qm), _ptr(tm), C.byref(have), C.byref(st)))
         return (qm, tm, st) if have.value else (None, None, st)
+
+    def enable_loop(self, **opts):
+        """Loop closure beside mapping (ilsm_slam_enable_loop), before the first frame.  opts: keyframe_dist,
+        keyframe_angle_rad, max_pending, and the LoopOpts fields of the loop stage (icp=dict of IcpOpts fields)."""
+        top = {k: opts.pop(k) for k in ("keyframe_dist", "keyframe_angle_rad", "max_pending") if k in opts}
+        o = SlamLoopOpts(loop=opts, **top)
+        _check(self._lib.ilsm_slam_enable_loop(self._h, C.byref(o)))
+
+    def loop_results(self, wait: bool = False, capacity: int | None = None) -> list:
+        """Loop decisions (SlamLoopEvent) of the keyframes answered so far, in keyframe order; wait=True first waits for every
+        keyframe selected so far.  capacity: at most this many (the rest stay queued); None: all of them.  A failed keyframe
+        raises IlsmError when it is next in order; the events taken out before it are on the exception as `.events`."""
+        out = []
+        while True:
+            cap = 64 if capacity is None else capacity - len(out)
+            buf, n = (SlamLoopEvent * max(cap, 1))(), C.c_int32(0)
+            try:
+                _check(self._lib.ilsm_slam_loop_results(self._h, 1 if wait else 0, buf, cap, C.byref(n)))
+            except IlsmError as e:
+                e.events = out
+                raise
+            out += [SlamLoopEvent.from_buffer_copy(buf[i]) for i in range(n.value)]
+            if n.value < cap or cap == 0 or capacity is not None:
+                return out
 
     def frame_pc2(self, blob, layout: "Pc2Layout", use_aloam: bool = True):
         """One frame handed over as the sensor_msgs/PointCloud2 `data` blob (uint8, n_points * point_step bytes)."""

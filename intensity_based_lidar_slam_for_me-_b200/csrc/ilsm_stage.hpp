@@ -51,6 +51,9 @@ class Stage {
 
   int in_flight() const { return in_flight_; }  // jobs posted and not yet taken
 
+  // Whether take() would return at once: the oldest job not yet taken has finished.  Does not wait.
+  bool ready() const { return n_results_.load(std::memory_order_acquire) > 0; }
+
   // Lets the thread run every job posted so far, then joins it.  Results not taken are dropped.
   void stop() {
     if (!thread_.joinable()) return;

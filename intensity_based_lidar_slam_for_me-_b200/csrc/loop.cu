@@ -207,7 +207,8 @@ struct ilsm_loop {
 
 using namespace ilsm;
 
-static int check_loop_opts(const ilsm_loop_opts& o) {
+// also the check of ilsm_slam_enable_loop's loop options (pipeline.cu)
+int check_loop_opts(const ilsm_loop_opts& o) {
   if (o.exclude_recent < 1 || o.tree_period < 1 || o.num_candidates < 1 || o.num_candidates > 16 || o.submap_half < 0 ||
       o.submap_half > 7)
     return fail(ILSM_ERR_INVALID_ARG, "loop_create: exclude_recent >= 1, tree_period >= 1, num_candidates in [1,16], submap_half in [0,7]");

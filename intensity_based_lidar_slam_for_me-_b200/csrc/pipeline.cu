@@ -12,12 +12,17 @@
 #include <string.h>
 
 #include <chrono>
+#include <deque>
+#include <memory>
 #include <new>
+#include <string>
 
 #include "ilsm_cubemap.hpp"
+#include "ilsm_keyframe.hpp"
 #include "ilsm_stage.hpp"
 
 struct ilsm_mapopt;
+int check_loop_opts(const ilsm_loop_opts& o);  // loop.cu
 
 namespace ilsm {
 
@@ -28,6 +33,8 @@ int mapopt_frame_core(ilsm_mapopt* mo, const float* frame_xyz, int n, int stride
 // voxel edge of the "last frame" search structures: the odometry gate is 5 m (DISTANCE_SQ_THRESHOLD 25,
 // laserOdometry.cpp:31), the clouds are sparse (a few thousand points)
 constexpr float kOdomCell = 1.0f;
+// points of one OS0-64 frame (64 x 1024): the size the loop-closure buffers are reserved at
+constexpr int kFramePoints = 65536;
 
 // The host phase clocks.  The first eight are those of ilsm_slam_host_phases, in the order include/ilsm.h documents;
 // the rest are the stage threads' detail that ILSM_STAGE_TRACE prints.
@@ -56,6 +63,11 @@ struct SlamH {
     DevBuf<float4> sharp, flat, lsharp, lflat;
     const float4* lf = nullptr;  // this frame's less-flat cloud: lflat, or the front end's own fe.lflat (synchronous loop)
     cudaEvent_t ev = nullptr;    // recorded once the slot is written
+    // loop closure in the pipelined and staged loops: the front end's cloud, kept until the frame's mapped pose is known
+    DevBuf<float4> cloud;
+    int n_cloud = 0;
+    cudaEvent_t ev_read = nullptr;  // recorded after a keyframe's copy read `cloud`
+    bool read_pending = false;      // the next front end into this slot waits for ev_read
   } fslot[3];
   // the two mapping stacks (VoxelGrid of the less-sharp / less-flat clouds, laserMapping.cpp:608-616), double-buffered:
   // the odometry stage's side stream writes set k & 1 for frame k under its solve while the mapping of frame k - 1 (solve
@@ -109,6 +121,37 @@ struct SlamH {
   };
   Stage<FeJob, FeResult> frontend{ilsm_last_error, fail_text};
   long long pushed = 0;
+  // loop closure (ilsm_slam_enable_loop): an ilsm_loop on its own context (ctx3) and host thread, like the reference's
+  // loopClosureThread.  Each keyframe's cloud is copied on the device into one of max_pending buffers; a buffer is used
+  // again only after the job that read it has been answered.
+  struct LoopJob {
+    int buf = 0, n = 0;
+    long long frame = -1;
+    double q[4] = {0, 0, 0, 1}, t[3] = {0, 0, 0};
+  };
+  struct LoopDone {
+    ilsm_slam_loop_event ev = {};
+    double seconds = 0;  // the stage's time on this keyframe
+  };
+  struct LoopBuf {
+    DevBuf<float4> cloud;
+    cudaEvent_t ev = nullptr;  // recorded once the keyframe's cloud is copied in
+  };
+  ilsm_ctx* ctx3 = nullptr;
+  ilsm_loop* loop = nullptr;
+  ilsm_slam_loop_opts lopts = {};
+  std::unique_ptr<LoopBuf[]> lbuf;
+  bool kf_have = false;  // (kf_q, kf_t): the mapped pose of the last keyframe
+  double kf_q[4] = {0, 0, 0, 1}, kf_t[3] = {0, 0, 0};
+  long long keyframes = 0;                    // selected so far
+  struct LoopAnswer {
+    ilsm_slam_loop_event ev = {};
+    int rc = 0;       // a keyframe that failed: its status and error text, reported by ilsm_slam_loop_results in its turn
+    std::string err;
+  };
+  std::deque<LoopAnswer> answered;  // taken from the loop stage, not yet handed out
+  double loop_s = 0;                          // the loop stage's time over the answered keyframes
+  Stage<LoopJob, LoopDone> looper{ilsm_last_error, fail_text};
   // host-side phase clock (profiling aid, ilsm_slam_host_phases): seconds per phase, written by the caller's thread only
   double phase_s[kNumPhases] = {};
 };
@@ -163,12 +206,21 @@ static int frontend_counts(Ctx& f, const float* xyzi, int n, int stride_bytes, c
 
 // The front end's sharp, less-sharp and flat clouds gathered into slot `o`.  Less-flat is copied there when `copy_lflat`
 // (a later front end on `f` may rewrite fe.lflat before this frame's last reader has run); otherwise o.lf is fe.lflat.
-static int frontend_gather(Ctx& f, const int cnt[8], SlamH::FeSlot& o, bool copy_lflat) {
+// With `copy_cloud` (loop closure, under the same condition) the ring-ordered cloud is copied there too, for the keyframe
+// copy that follows once the frame's mapped pose is known; it waits for that copy of the slot's previous frame.
+static int frontend_gather(Ctx& f, const int cnt[8], SlamH::FeSlot& o, bool copy_lflat, bool copy_cloud) {
   const int n_sharp = cnt[1], n_lsharp = cnt[2], n_flat = cnt[3], n_lflat = cnt[4];
   int rc;
   if ((rc = o.sharp.reserve(n_sharp + 4)) || (rc = o.flat.reserve(n_flat + 4)) || (rc = o.lsharp.reserve(n_lsharp + 4)) ||
-      (copy_lflat && (rc = o.lflat.reserve(n_lflat + 4))))
+      (copy_lflat && (rc = o.lflat.reserve(n_lflat + 4))) || (copy_cloud && (rc = o.cloud.reserve((size_t)cnt[0] + 4))))
     return rc;
+  o.n_cloud = cnt[0];
+  if (copy_cloud) {
+    if (o.read_pending) ILSM_CUDA(cudaStreamWaitEvent(f.stream, o.ev_read, 0));
+    o.read_pending = false;
+    if (cnt[0])
+      ILSM_CUDA(cudaMemcpyAsync(o.cloud.p, f.fe.cloud.p, (size_t)cnt[0] * sizeof(float4), cudaMemcpyDeviceToDevice, f.stream));
+  }
   if ((rc = f.gather_dev(f.fe.cloud.p, f.fe.sharp.p, f.fe.counts.p, 1, n_sharp, o.sharp.p)) ||
       (rc = f.gather_dev(f.fe.cloud.p, f.fe.lsharp.p, f.fe.counts.p, 2, n_lsharp, o.lsharp.p)) ||
       (rc = f.gather_dev(f.fe.cloud.p, f.fe.flat.p, f.fe.counts.p, 3, n_flat, o.flat.p)))
@@ -296,15 +348,93 @@ static void post_mapping_job(SlamH& s, const SlamH::FeSlot& o, const int cnt[8],
   s.mapping.post(j);
 }
 
+// ---- loop closure: the keyframe rule on every mapped pose handed out, the keyframe's cloud to the loop stage
+
+// The loop stage's answer to its oldest keyframe, queued for ilsm_slam_loop_results.  A failed keyframe is queued too, with
+// its error: it is reported there, in keyframe order, and never by a frame call.
+static void take_loop_result(SlamH& s) {
+  SlamH::LoopDone d;
+  SlamH::LoopAnswer a;
+  if ((a.rc = s.looper.take(d))) a.err = ilsm_last_error();
+  a.ev = d.ev;
+  s.loop_s += d.seconds;
+  s.answered.push_back(std::move(a));
+}
+
+// hand keyframe `frame` to the loop stage (loop_offer)
+static int loop_post(SlamH& s, long long frame, SlamH::FeSlot* o, const float4* cloud, int n, const double q[4], const double t[3]) {
+  // every buffer in flight: wait for the oldest answer, which frees the buffer this keyframe takes
+  if (s.looper.in_flight() >= s.lopts.max_pending) take_loop_result(s);
+  int rc;
+  SlamH::LoopJob j;
+  j.buf = (int)(s.keyframes % s.lopts.max_pending), j.n = n, j.frame = frame;
+  for (int i = 0; i < 4; ++i) j.q[i] = q[i];
+  for (int i = 0; i < 3; ++i) j.t[i] = t[i];
+  SlamH::LoopBuf& b = s.lbuf[j.buf];
+  Ctx& c = *s.ctx;
+  if ((rc = b.cloud.reserve((size_t)n + 4))) return rc;
+  if (o) ILSM_CUDA(cudaStreamWaitEvent(c.stream, o->ev, 0));
+  if (n) ILSM_CUDA(cudaMemcpyAsync(b.cloud.p, cloud, (size_t)n * sizeof(float4), cudaMemcpyDeviceToDevice, c.stream));
+  if (o) {
+    ILSM_CUDA(cudaEventRecord(o->ev_read, c.stream));
+    o->read_pending = true;
+  }
+  ILSM_CUDA(cudaEventRecord(b.ev, c.stream));
+  s.looper.post(j);
+  s.keyframes++;
+  return ILSM_OK;
+}
+
+// Frame `frame`'s mapped pose is being handed out: when it is a keyframe, copy its cloud (n points of 16 bytes at `cloud`,
+// on c's stream: the front end's own buffer in the synchronous loop, slot `o` otherwise) into a free loop buffer and post
+// it to the loop stage.  The copy is ordered after the slot's event, and the next front end into the slot after the copy.
+// Nothing here fails the frame call: the frame's odometry and mapping have already advanced the handle.  A keyframe that
+// cannot be handed over is queued as a failed answer behind every keyframe before it.
+static void loop_offer(SlamH& s, long long frame, SlamH::FeSlot* o, const float4* cloud, int n, const double q[4], const double t[3]) {
+  if (!s.loop) return;
+  if (s.kf_have && !keyframe_due(s.kf_q, s.kf_t, q, t, s.lopts.keyframe_dist, s.lopts.keyframe_angle_rad)) return;
+  s.kf_have = true;
+  for (int i = 0; i < 4; ++i) s.kf_q[i] = q[i];
+  for (int i = 0; i < 3; ++i) s.kf_t[i] = t[i];
+  SlamH::LoopAnswer a;
+  if (!(a.rc = loop_post(s, frame, o, cloud, n, q, t))) return;
+  a.err = ilsm_last_error();
+  a.ev.frame = frame;
+  for (int i = 0; i < 4; ++i) a.ev.q_xyzw[i] = q[i];
+  for (int i = 0; i < 3; ++i) a.ev.t[i] = t[i];
+  while (s.looper.in_flight() > 0) take_loop_result(s);
+  s.answered.push_back(std::move(a));
+}
+
+// one keyframe on the loop stage: ilsm_loop_add_keyframe_dev on ctx3, after the copy into its buffer
+static int loop_job(SlamH& s, const SlamH::LoopJob& j, SlamH::LoopDone& r) {
+  const auto t0 = std::chrono::steady_clock::now();
+  r.ev.frame = j.frame;
+  for (int i = 0; i < 4; ++i) r.ev.q_xyzw[i] = j.q[i];
+  for (int i = 0; i < 3; ++i) r.ev.t[i] = j.t[i];
+  const SlamH::LoopBuf& b = s.lbuf[j.buf];
+  {
+    Ctx& l = s.ctx3->c;
+    std::lock_guard<std::mutex> lk(l.mu);
+    const cudaError_t e = cudaStreamWaitEvent(l.stream, b.ev, 0);
+    if (e != cudaSuccess) return fail_cuda(e, "cudaStreamWaitEvent(loop stage)");
+  }
+  const int rc = ilsm_loop_add_keyframe_dev(s.loop, reinterpret_cast<const float*>(b.cloud.p), j.n, 16, j.q, j.t, &r.ev.result);
+  r.seconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+  return rc;
+}
+
 // wait for the mapping stage's answer to its oldest job and hand it out
 static int take_mapping_result(SlamH& s, double q_map[4], double t_map[3], ilsm_slam_stats* stats, int* frame = nullptr) {
   SlamH::MapResult r;
-  const int rc = take_result(s, s.mapping, r);
+  int rc = take_result(s, s.mapping, r);
   if (rc) return rc;
   if (frame) *frame = (int)r.frame;
   for (int i = 0; i < 4; ++i) q_map[i] = r.q[i];
   for (int i = 0; i < 3; ++i) t_map[i] = r.t[i];
   if (stats) stats->mapping = r.report, stats->cubemap = r.cstats;
+  SlamH::FeSlot& o = s.fslot[r.frame % 3];
+  loop_offer(s, r.frame, &o, o.cloud.p, o.n_cloud, r.q, r.t);
   return ILSM_OK;
 }
 
@@ -316,7 +446,7 @@ static int frontend_job(SlamH& s, const SlamH::FeJob& j, SlamH::FeResult& r) {
   PhaseClock clk(r.phase_s);
   int rc;
   if ((rc = frontend_counts(f, j.xyzi, j.n, j.stride, nullptr, s.min_range, r.counts, clk, kFeStageLaunch, kFeStageWait)) ||
-      (rc = frontend_gather(f, r.counts, s.fslot[j.frame % 3], true)))
+      (rc = frontend_gather(f, r.counts, s.fslot[j.frame % 3], true, s.loop != nullptr)))
     return rc;
   clk.lap(kFeStageGather);
   return ILSM_OK;
@@ -349,6 +479,25 @@ static int reserve_frame_buffers(SlamH& s) {
     if ((rc = set.c.reserve(8192)) || (rc = set.s.reserve(32768)) || (rc = set.n.reserve(4))) return rc;
   }
   return ILSM_OK;
+}
+
+// undo a failed ilsm_slam_enable_loop: the handle stays as it was
+static int loop_stage_abort(SlamH& s, int rc) {
+  if (s.loop) ilsm_loop_destroy(s.loop);
+  {
+    std::lock_guard<std::mutex> lk(s.ctx->mu);
+    cudaSetDevice(s.ctx->device);
+    for (SlamH::FeSlot& o : s.fslot) {
+      if (o.ev_read) cudaEventDestroy(o.ev_read);
+      o.ev_read = nullptr;
+    }
+    for (int i = 0; s.lbuf && i < s.lopts.max_pending; ++i)
+      if (s.lbuf[i].ev) cudaEventDestroy(s.lbuf[i].ev);
+    s.lbuf.reset();
+  }
+  if (s.ctx3) ilsm_destroy(s.ctx3);
+  s.loop = nullptr, s.ctx3 = nullptr;
+  return rc;
 }
 
 static int slam_create_common(ilsm_ctx* ctx, float min_range, ilsm_slam** out, ilsm_slam** h_out) {
@@ -463,12 +612,23 @@ ILSM_API void ilsm_slam_destroy(ilsm_slam* slam) {
     cudaStreamSynchronize(s.ctx2->c.stream);
     cudaStreamSynchronize(s.ctx2->c.aux);
   }
+  if (s.loop && getenv("ILSM_STAGE_TRACE")) {
+    const long long taken = s.keyframes - s.looper.in_flight();  // the answers the caller collected, with their stage times
+    fprintf(stderr, "[ilsm stage trace] loop: keyframes %lld  collected %lld  stage %.1f us per collected keyframe\n", s.keyframes,
+            taken, 1e6 * s.loop_s / (taken ? taken : 1));
+  }
+  s.looper.stop();  // every posted keyframe is answered; the loop handle's destroy synchronises its stream
+  if (s.loop) ilsm_loop_destroy(s.loop);
   {
     std::lock_guard<std::mutex> lk(s.ctx->mu);
     cudaSetDevice(s.ctx->device);
     cudaStreamSynchronize(s.ctx->stream);
-    for (SlamH::FeSlot& o : s.fslot)
+    for (SlamH::FeSlot& o : s.fslot) {
       if (o.ev) cudaEventDestroy(o.ev);
+      if (o.ev_read) cudaEventDestroy(o.ev_read);
+    }
+    for (int i = 0; s.lbuf && i < s.lopts.max_pending; ++i)
+      if (s.lbuf[i].ev) cudaEventDestroy(s.lbuf[i].ev);
     for (SlamH::StackSet& set : s.stk) {
       if (set.ev_ready) cudaEventDestroy(set.ev_ready);
       if (set.ev_free) cudaEventDestroy(set.ev_free);
@@ -478,8 +638,86 @@ ILSM_API void ilsm_slam_destroy(ilsm_slam* slam) {
   if (s.mapopt) ilsm_mapopt_destroy(s.mapopt);
   if (s.ctx2) ilsm_destroy(s.ctx2);
   if (s.ctx0) ilsm_destroy(s.ctx0);
+  if (s.ctx3) ilsm_destroy(s.ctx3);
   cudaSetDevice(s.ctx->device);
   delete slam;  // frees the slots, stack sets and last-frame maps: no stage reads them any more
+}
+
+ILSM_API void ilsm_slam_loop_opts_default(ilsm_slam_loop_opts* o) {
+  if (!o) return;
+  memset(o, 0, sizeof(*o));
+  o->keyframe_dist = 1.0;
+  o->keyframe_angle_rad = 0.2;
+  o->max_pending = 8;
+  ilsm_loop_opts_default(&o->loop);
+}
+
+ILSM_API int ilsm_slam_enable_loop(ilsm_slam* slam, const ilsm_slam_loop_opts* opts) {
+  if (!slam) return fail(ILSM_ERR_INVALID_ARG, "slam_enable_loop: null handle");
+  ilsm_slam_loop_opts o;
+  if (opts)
+    o = *opts;
+  else
+    ilsm_slam_loop_opts_default(&o);
+  if (!(o.keyframe_dist >= 0.0) || !(o.keyframe_angle_rad >= 0.0) || !isfinite(o.keyframe_dist) || !isfinite(o.keyframe_angle_rad))
+    return fail(ILSM_ERR_INVALID_ARG, "slam_enable_loop: keyframe_dist and keyframe_angle_rad must be finite and >= 0");
+  if (o.max_pending < 1) return fail(ILSM_ERR_INVALID_ARG, "slam_enable_loop: max_pending must be >= 1");
+  int rc = check_loop_opts(o.loop);
+  if (rc) return rc;
+  int count = 0;
+  if (cudaGetDeviceCount(&count) != cudaSuccess || count <= 0) {
+    cudaGetLastError();
+    return fail(ILSM_ERR_NO_DEVICE, "slam_enable_loop: no CUDA device available (libilsm_cuda has no CPU fallback)");
+  }
+  SlamH& s = slam->s;
+  if (s.loop) return fail(ILSM_ERR_STATE, "slam_enable_loop: loop closure is already on");
+  if (s.frames > 0 || s.pushed > 0) return fail(ILSM_ERR_STATE, "slam_enable_loop: call it before the first frame");
+  if ((rc = ilsm_create(s.ctx->device, &s.ctx3)) || (rc = ilsm_loop_create(s.ctx3, &o.loop, &s.loop))) return loop_stage_abort(s, rc);
+  s.lopts = o;
+  {
+    CtxGuard g(*s.ctx);
+    if ((rc = g.rc)) return loop_stage_abort(s, rc);
+    s.lbuf.reset(new (std::nothrow) SlamH::LoopBuf[o.max_pending]);
+    if (!s.lbuf) return loop_stage_abort(s, fail(ILSM_ERR_OUT_OF_MEMORY, "host allocation failed"));
+    // the frame's size up front: a growing buffer costs a device-wide synchronisation (reserve_frame_buffers)
+    for (int i = 0; i < o.max_pending; ++i) {
+      if (cudaEventCreateWithFlags(&s.lbuf[i].ev, cudaEventDisableTiming) != cudaSuccess)
+        return loop_stage_abort(s, fail(ILSM_ERR_CUDA, "slam_enable_loop: event creation failed"));
+      if ((rc = s.lbuf[i].cloud.reserve(kFramePoints + 4))) return loop_stage_abort(s, rc);
+    }
+    for (SlamH::FeSlot& sl : s.fslot) {
+      if (cudaEventCreateWithFlags(&sl.ev_read, cudaEventDisableTiming) != cudaSuccess)
+        return loop_stage_abort(s, fail(ILSM_ERR_CUDA, "slam_enable_loop: event creation failed"));
+      if (s.ctx2 && (rc = sl.cloud.reserve(kFramePoints + 4))) return loop_stage_abort(s, rc);
+    }
+  }
+  SlamH* sp = &s;
+  s.looper.start([sp] { cudaSetDevice(sp->ctx3->c.device); },
+                 [sp](const SlamH::LoopJob& j, SlamH::LoopDone& r) { return loop_job(*sp, j, r); });
+  return ILSM_OK;
+}
+
+ILSM_API int ilsm_slam_loop_results(ilsm_slam* slam, int wait, ilsm_slam_loop_event* out, int capacity, int* n_out) {
+  if (!slam || !n_out || (capacity > 0 && !out)) return fail(ILSM_ERR_INVALID_ARG, "slam_loop_results: null argument");
+  if (capacity < 0) return fail(ILSM_ERR_INVALID_ARG, "slam_loop_results: capacity < 0");
+  *n_out = 0;
+  SlamH& s = slam->s;
+  if (!s.loop) return fail(ILSM_ERR_STATE, "slam_loop_results: loop closure is not on (ilsm_slam_enable_loop)");
+  // no context lock: the queue and the stage's in-flight count belong to the thread that hands in the frames, and a drain
+  // must not hold up other users of the caller's context
+  while (s.looper.in_flight() > 0 && (wait || s.looper.ready())) take_loop_result(s);
+  int k = 0;
+  for (; k < capacity && !s.answered.empty() && !s.answered.front().rc; ++k) {
+    out[k] = s.answered.front().ev;
+    s.answered.pop_front();
+  }
+  *n_out = k;
+  if (k == 0 && capacity > 0 && !s.answered.empty()) {  // a failed keyframe is next in order: report it
+    const SlamH::LoopAnswer a = std::move(s.answered.front());
+    s.answered.pop_front();
+    return fail(a.rc, "slam_loop_results: keyframe of frame %lld: %s", (long long)a.ev.frame, a.err.c_str());
+  }
+  return ILSM_OK;
 }
 
 ILSM_API ilsm_cubemap* ilsm_slam_cubemap(ilsm_slam* slam) { return slam ? slam->s.cube : nullptr; }
@@ -566,7 +804,7 @@ static int slam_frame_impl(ilsm_slam* slam, const float* xyzi, int n, int stride
   CubeMapH* cmp = s.cube ? &s.cube->m : nullptr;
   // With the mapping stage on its own context nothing orders the next call's front end, which rewrites fe.lflat, after
   // this frame's stack VoxelGrid: that reads a copy in the slot.
-  if ((rc = frontend_gather(c, cnt, o, s.ctx2 != nullptr))) return rc;
+  if ((rc = frontend_gather(c, cnt, o, s.ctx2 != nullptr, s.ctx2 != nullptr && s.loop != nullptr))) return rc;
   if (cmp && (rc = stack_voxelgrid(c, *cmp, o, cnt, set))) return rc;
   // ---- laserOdometry
   // the previous frame's deferred map insertion (side stream) reads the mapped pose from the LM state the odometry is
@@ -597,6 +835,8 @@ static int slam_frame_impl(ilsm_slam* slam, const float* xyzi, int n, int stride
       stats->cubemap.n_valid = ms.converged;
     }
   }
+  // the synchronous loops hand out this frame's mapped pose now, while the front end's cloud is still this frame's
+  if (!rc && !s.async) loop_offer(s, s.frames, nullptr, c.fe.cloud.p, cnt[0], q_map, t_map);
   clk.lap(kMapping);  // synchronous: enqueue and wait; pipelined: enqueue only
   if (rc) return rc;
   s.frames++;

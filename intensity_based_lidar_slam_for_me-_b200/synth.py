@@ -5,6 +5,8 @@ product kernel -- it only manufactures inputs.
 """
 from __future__ import annotations
 
+import math
+
 import numpy as np
 
 SEED_FRAME = 0x5EED0001
@@ -453,3 +455,46 @@ def loop_submap(kfs, c, n_per_lap, half=2, leaf=0.4):
     lap0 = (c // n_per_lap) * n_per_lap
     ids = [lap0 + (c - lap0 + d) % n_per_lap for d in range(-half, half + 1)]
     return voxel_centroid_np(np.concatenate([kfs[i]["world"] for i in ids]), leaf)
+
+
+def closed_loop_poses(laps=2, radius=8.0, step=0.25, widen=0.1, turn_deg=3.0, z=1.5):
+    """Ground-truth poses (q, t) of a closed-loop sequence through the box scene (Scene()): one continuous path `laps`
+    times around the circle of loop_keyframes(), `step` m per frame (about 1.8 degrees of turn per frame at 8 m), every
+    lap `widen` m wider and its heading `turn_deg` more turned than the one before, so that a later lap passes within
+    `widen` m of the places of the earlier ones.  Ray-cast it with make_frames_torch(Scene(), poses, ...)."""
+    n_per_lap = int(round(2 * np.pi * radius / step))
+    poses = []
+    for k in range(laps * n_per_lap):
+        u = k / n_per_lap  # laps done
+        a = 2 * np.pi * u
+        r = radius + widen * u
+        q = quat_from_rotvec([0.0, 0.0, a + np.pi / 2 + np.deg2rad(turn_deg * u)])
+        poses.append((q, np.array([r * np.cos(a), r * np.sin(a), z])))
+    return poses
+
+
+def keyframe_due(q_kf, t_kf, q, t, keyframe_dist, keyframe_angle_rad):
+    """The full loop's keyframe rule (ilsm_slam_enable_loop) restated in the library's fp64 order of operations: is the
+    frame with mapped pose (q, t) a keyframe after the keyframe (q_kf, t_kf)?  Quaternions xyzw."""
+    kx, ky, kz, kw = (float(v) for v in q_kf)
+    x, y, zq, w = (float(v) for v in q)
+    dx, dy, dz = float(t[0]) - float(t_kf[0]), float(t[1]) - float(t_kf[1]), float(t[2]) - float(t_kf[2])
+    d = math.sqrt(dx * dx + dy * dy + dz * dz)
+    ax, ay, az, aw = -kx, -ky, -kz, kw  # conj(q_kf) * q
+    vx = aw * x + ax * w + ay * zq - az * y
+    vy = aw * y - ax * zq + ay * w + az * x
+    vz = aw * zq + ax * y - ay * x + az * w
+    vw = aw * w - ax * x - ay * y - az * zq
+    angle = 2.0 * math.atan2(math.sqrt(vx * vx + vy * vy + vz * vz), abs(vw))
+    return d >= keyframe_dist or angle >= keyframe_angle_rad
+
+
+def select_keyframes(poses, keyframe_dist=1.0, keyframe_angle_rad=0.2):
+    """Indices of the keyframes among mapped poses [(q, t)] in hand-out order: the first, then every pose keyframe_due
+    after the last keyframe."""
+    out, last = [], None
+    for k, (q, t) in enumerate(poses):
+        if last is None or keyframe_due(last[0], last[1], q, t, keyframe_dist, keyframe_angle_rad):
+            out.append(k)
+            last = (q, t)
+    return out
