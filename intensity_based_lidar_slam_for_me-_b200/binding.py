@@ -292,6 +292,7 @@ def load_library(path: str | None = None):
         "ilsm_associate_dev": (i32, [vp, vp, vp, vp, i32, vp, i32, i32, vp, C.POINTER(RegOpts)]),
         "ilsm_launch_count": (C.c_longlong, []),
         "ilsm_debug_live_bytes": (None, [C.POINTER(C.c_longlong), C.POINTER(C.c_longlong)]),
+        "ilsm_debug_live_handles": (None, [C.POINTER(C.c_longlong)]),
         "ilsm_eval_normal_eq": (i32, [vp, vp, vp, f64, C.POINTER(f64), vp, vp]),
         "ilsm_eval_normal_eq_dev": (i32, [vp, vp, f64, vp]),
         "ilsm_solve_dev": (i32, [vp, vp, i32, f64]),
@@ -325,6 +326,13 @@ def live_bytes() -> tuple[int, int]:
     dev, pin = C.c_longlong(0), C.c_longlong(0)
     load_library().ilsm_debug_live_bytes(C.byref(dev), C.byref(pin))
     return dev.value, pin.value
+
+
+def live_handles() -> int:
+    """CUDA events, streams and graph execs the library holds, all handles of the process together.  Makes no CUDA call."""
+    n = C.c_longlong(0)
+    load_library().ilsm_debug_live_handles(C.byref(n))
+    return n.value
 
 
 def _check(rc):

@@ -28,6 +28,7 @@ int fail_cuda(cudaError_t e, const char* where) {
 static std::atomic<long long> g_launches{0};
 void count_launches(int k) { g_launches.fetch_add(k, std::memory_order_relaxed); }
 std::atomic<long long> g_live_bytes[2] = {{0}, {0}};
+std::atomic<long long> g_live_handles{0};
 
 int check_launch(const char* where) {
   cudaError_t e = cudaGetLastError();
@@ -53,12 +54,9 @@ int Ctx::init(int dev) {
   cudaDeviceProp prop;
   ILSM_CUDA(cudaGetDeviceProperties(&prop, dev));
   sm_count = prop.multiProcessorCount;
-  ILSM_CUDA(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
-  ILSM_CUDA(cudaStreamCreateWithFlags(&aux, cudaStreamNonBlocking));
-  ILSM_CUDA(cudaEventCreateWithFlags(&ev_fork, cudaEventDisableTiming));
-  ILSM_CUDA(cudaEventCreateWithFlags(&ev_join, cudaEventDisableTiming));
   int rc;
-  if ((rc = lm.reserve(1))) return rc;
+  if ((rc = stream.create()) || (rc = aux.create()) || (rc = ev_fork.create()) || (rc = ev_join.create()) || (rc = lm.reserve(1)))
+    return rc;
   ILSM_CUDA(cudaMemsetAsync(lm.p, 0, sizeof(LmState), stream));
   if ((rc = pinned.reserve(4096))) return rc;
   ILSM_CUDA(cudaStreamSynchronize(stream));
@@ -71,21 +69,12 @@ int Ctx::init(int dev) {
 }
 
 Ctx::~Ctx() {
-  if (fe_graph_exec) cudaGraphExecDestroy(fe_graph_exec);
   if (stream) cudaStreamSynchronize(stream);
   if (aux) cudaStreamSynchronize(aux);
-  delete qbin;
-  if (ev_fork) cudaEventDestroy(ev_fork);
-  if (ev_join) cudaEventDestroy(ev_join);
-  if (aux) cudaStreamDestroy(aux);
-  if (stream) cudaStreamDestroy(stream);
 }
 
 Map::~Map() {
   if (stream) cudaStreamSynchronize(stream);
-  if (ready) cudaEventDestroy(ready);
-  if (ctx_done) cudaEventDestroy(ctx_done);
-  if (stream) cudaStreamDestroy(stream);
 }
 
 // the LM iteration budget the solve kernel accepts
@@ -170,6 +159,12 @@ ILSM_API int ilsm_debug_stamps(ilsm_ctx* ctx, long long* out64) {
 ILSM_API void ilsm_debug_live_bytes(long long* device, long long* pinned) {
   if (device) *device = g_live_bytes[0].load();
   if (pinned) *pinned = g_live_bytes[1].load();
+}
+
+// testing aid (not in include/ilsm.h): CUDA events, streams and graph execs held by every handle of the process; makes
+// no CUDA call
+ILSM_API void ilsm_debug_live_handles(long long* handles) {
+  if (handles) *handles = g_live_handles.load();
 }
 
 ILSM_API int ilsm_set_async(ilsm_ctx* ctx, int on) {

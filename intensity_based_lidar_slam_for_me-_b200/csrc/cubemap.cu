@@ -211,7 +211,7 @@ int CubeMapH::init(Ctx* c, float lres, float pres, int cube_cap) {
   // the two count arrays and the error word sit back to back (cnt_all): the host mirror is refreshed with ONE copy per frame;
   // cnt_c / cnt_s / err are views into it
   cnt_c = cnt_all.p, cnt_s = cnt_all.p + kCNum, err = cnt_all.p + 2 * kCNum;
-  ILSM_CUDA(cudaEventCreateWithFlags(&ev_tail, cudaEventDisableTiming));
+  if ((rc = ev_tail.create())) return rc;
   slab_of.resize(kCNum);
   for (int i = 0; i < kCNum; ++i) slab_of[i] = i;
   cnt_c_h.assign(kCNum, 0), cnt_s_h.assign(kCNum, 0);
@@ -229,7 +229,6 @@ int CubeMapH::init(Ctx* c, float lres, float pres, int cube_cap) {
 CubeMapH::~CubeMapH() {
   if (ctx && ctx->stream) cudaStreamSynchronize(ctx->stream);
   if (ctx && ctx->aux) cudaStreamSynchronize(ctx->aux);
-  if (ev_tail) cudaEventDestroy(ev_tail);
 }
 
 static int cube_coord_h(double v, int cen) {

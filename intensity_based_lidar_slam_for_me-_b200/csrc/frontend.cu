@@ -991,7 +991,7 @@ int Ctx::features_dev(const float* d_in, int n, int stride_bytes, float min_rang
   }
   bool capturing = false;
   if (fe_graphs_ok) {
-    if (fe_graph_exec) cudaGraphExecDestroy(fe_graph_exec), fe_graph_exec = nullptr;
+    fe_graph_exec.reset();
     capturing = cudaStreamBeginCapture(stream, cudaStreamCaptureModeThreadLocal) == cudaSuccess;
     if (!capturing) cudaGetLastError(), fe_graphs_ok = false;
   }
@@ -999,11 +999,11 @@ int Ctx::features_dev(const float* d_in, int n, int stride_bytes, float min_rang
   if (capturing) {
     cudaGraph_t g = nullptr;
     cudaError_t e = cudaStreamEndCapture(stream, &g);
-    if (e == cudaSuccess && rcl == ILSM_OK) e = cudaGraphInstantiate(&fe_graph_exec, g, 0);
+    const bool ok = e == cudaSuccess && rcl == ILSM_OK && fe_graph_exec.create(g) == ILSM_OK;
     if (g) cudaGraphDestroy(g);
-    if (e != cudaSuccess || rcl != ILSM_OK || !fe_graph_exec) {  // capture not possible here: plain launches from now on
+    if (!ok) {  // capture not possible here: plain launches from now on
       cudaGetLastError();
-      fe_graph_exec = nullptr, fe_graphs_ok = false;
+      fe_graphs_ok = false;
       return features_launch(d_in, n, stride_bytes, min_range, ring_cap);
     }
     fe_graph_key = key;

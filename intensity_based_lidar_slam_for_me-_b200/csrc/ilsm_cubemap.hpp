@@ -69,7 +69,7 @@ struct CubeMapH {
   PinnedBuf<int> pin;
 
   int init(Ctx* c, float lres, float pres, int cube_cap);
-  ~CubeMapH();  // synchronises the context's streams, then destroys ev_tail
+  ~CubeMapH();  // synchronises the context's streams
   int roll(const double t[3]);
   int gather(int* n_mc, int* n_ms);
   int insert(const int* d_counts, int nc_host, int ns_host, int world_frame, cudaStream_t s = nullptr);
@@ -78,7 +78,7 @@ struct CubeMapH {
   int adopt_counts();
   int wait_tail();
   PinnedBuf<int> pin_counts;
-  cudaEvent_t ev_tail = nullptr;
+  Event ev_tail;
   bool tail_pending = false, counts_in_flight = false;
   int tail_flags = 0;
   struct Pending {  // a frame enqueued by cubemap_frame_enqueue and not yet collected

@@ -8,6 +8,7 @@
 #include <string.h>
 
 #include <atomic>
+#include <memory>
 #include <mutex>
 #include <string>
 
@@ -130,6 +131,53 @@ using DevBuf = Buf<T, DeviceMem>;
 template <typename T>
 using PinnedBuf = Buf<T, PinnedMem>;
 
+// CUDA events, streams and graph execs held by all owners of the process (ilsm_debug_live_handles), for the same check.
+extern std::atomic<long long> g_live_handles;
+
+// how each kind of handle is made and released: events without timing, non-blocking streams
+inline cudaError_t create_handle(cudaEvent_t* h) { return cudaEventCreateWithFlags(h, cudaEventDisableTiming); }
+inline cudaError_t create_handle(cudaStream_t* h) { return cudaStreamCreateWithFlags(h, cudaStreamNonBlocking); }
+inline cudaError_t create_handle(cudaGraphExec_t* h, cudaGraph_t g) { return cudaGraphInstantiate(h, g, 0); }
+inline void destroy_handle(cudaEvent_t h) { cudaEventDestroy(h); }
+inline void destroy_handle(cudaStream_t h) { cudaStreamDestroy(h); }
+inline void destroy_handle(cudaGraphExec_t h) { cudaGraphExecDestroy(h); }
+
+// Move-only owner of one CUDA handle, released when the owner is destroyed: its owner's teardown must have synchronised
+// every stream that still uses it.  Converts to the raw handle (nullptr while empty).
+template <typename Raw>
+class Owned {
+ public:
+  Owned() = default;
+  Owned(const Owned&) = delete;
+  Owned& operator=(const Owned&) = delete;
+  Owned(Owned&& o) noexcept : h_(o.h_) { o.h_ = nullptr; }
+  ~Owned() { reset(); }
+  operator Raw() const { return h_; }
+  // releases the handle held, then makes a new one: ILSM_OK, or ILSM_ERR_CUDA through fail_cuda (the owner is left empty)
+  template <typename... Args>
+  int create(Args... args) {
+    reset();
+    Raw h = nullptr;
+    const cudaError_t e = create_handle(&h, args...);
+    if (e != cudaSuccess) return fail_cuda(e, "Owned::create");
+    h_ = h;
+    g_live_handles.fetch_add(1, std::memory_order_relaxed);
+    return ILSM_OK;
+  }
+  void reset() {
+    if (!h_) return;
+    destroy_handle(h_);
+    g_live_handles.fetch_sub(1, std::memory_order_relaxed);
+    h_ = nullptr;
+  }
+
+ private:
+  Raw h_ = nullptr;
+};
+using Event = Owned<cudaEvent_t>;
+using Stream = Owned<cudaStream_t>;
+using GraphExec = Owned<cudaGraphExec_t>;
+
 // Levenberg-Marquardt state that lives in HBM for the duration of a registration: the trust-region loop of
 // ceres::Solve runs on the device, one evaluation kernel per iteration, no host round trip.
 struct LmState {
@@ -195,12 +243,12 @@ struct Map {
   DevBuf<float> raw;  // staging of caller bytes for the host-pointer entry points
   // Each map builds on its own stream so that the corner and surf structures of a frame are built concurrently
   // (and their H2D copies overlap); users on the context stream wait on `ready`.
-  cudaStream_t stream = nullptr;
+  Stream stream;
   // builds run in line on the context's stream, with no fork / join events: for callers whose builds have nothing to
   // overlap with (the cube map's two search structures sit on the mapping stage's critical path, and every event call is
   // host time there)
   bool in_line = false;
-  cudaEvent_t ready = nullptr, ctx_done = nullptr;
+  Event ready, ctx_done;
   bool pending = false;
 
   // Add_Points scratch (ikdmap.cu)
@@ -221,7 +269,7 @@ struct Map {
   const uint32_t* cur_counters() const { return counters.p + 8 * cur; }
   int knn_dev(const float* d_q, int nq, int stride_bytes, int k, float max_dist, int32_t* d_idx, float* d_d2);
   GridView view() const;
-  ~Map();  // synchronises the map's stream, then destroys it and the events
+  ~Map();  // synchronises the map's stream
 };
 
 // Device-side factor storage (SoA), one slot per stack point (corner slots first).
@@ -264,9 +312,9 @@ struct FeBufs {
 struct Ctx {
   int device = 0;
   int sm_count = 148;
-  cudaStream_t stream = nullptr;
-  cudaStream_t aux = nullptr;                       // side stream: work of a frame that does not depend on the odometry
-  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
+  Stream stream;
+  Stream aux;  // side stream: work of a frame that does not depend on the odometry
+  Event ev_fork, ev_join;
   std::mutex mu;
   DevBuf<LmState> lm;
   DevBuf<double> partials;  // [blocks][32]
@@ -280,7 +328,7 @@ struct Ctx {
   int solve_wide = -1;                  // LM solve as a 16-CTA cluster (1) or the portable 8 (0); -1: not probed yet
   DevBuf<float4> rf_lsharp, rf_stack_c, rf_stack_s;  // ilsm_register_frame: less-sharp cloud and the two down-sampled stacks
   DevBuf<int> rf_stack_n;
-  Map* qbin = nullptr;        // query binning of the throughput k-NN path (knn_binned.cu): the query cloud grouped by voxel
+  std::unique_ptr<Map> qbin;  // query binning of the throughput k-NN path (knn_binned.cu): the query cloud grouped by voxel
   DevBuf<int> qwork;          // its work items (4 ints each) + the item counter
   int knn_group = 8;          // queries per group of the binned search (ILSM_KNN_GROUP: 1, 2, 4, 8, 16 or 32)
   int knn_binned_min = 8192;  // query sets at least this large take the binned path (ILSM_KNN_BINNED_MIN overrides)
@@ -342,9 +390,9 @@ struct Ctx {
                   float* d_track);
   int features_dev(const float* d_in, int n, int stride_bytes, float min_range);
   int features_launch(const float* d_in, int n, int stride_bytes, float min_range, int ring_cap);  // the 10 plain launches
-  cudaGraphExec_t fe_graph_exec = nullptr;  // the captured front-end chain and the parameter hash it was captured for
+  GraphExec fe_graph_exec;  // the captured front-end chain and the parameter hash it was captured for
   unsigned long long fe_graph_key = 0;
-  bool fe_graphs_ok = true;                 // false after a failed capture: plain launches from then on
+  bool fe_graphs_ok = true;  // false after a failed capture: plain launches from then on
   int pc2_unpack_dev(const unsigned char* d_data, int n, const ilsm_pc2_layout& l, float4* d_out);
   int pc2_pack_dev(const float4* d_in, int n, const ilsm_pc2_layout& l, unsigned char* d_out);
   // VoxelGrid of 1 or 2 clouds on stream s; d_err: the error word the kernels OR their flags into (nullptr: the front

@@ -363,12 +363,13 @@ static int launch_binned(Ctx* ctx, Map* m, Map* qb, const float* d_q, int nq, in
 // Exact k-NN of a large query set: bin the queries by voxel (the map's own cell size), then one warp per group.
 int knn_binned_dev(Ctx* ctx, Map* m, const float* d_q, int nq, int stride_bytes, int k, float max_dist, int32_t* d_idx, float* d_d2) {
   int rc;
-  if (!ctx->qbin) {
-    ctx->qbin = new (std::nothrow) Map();
-    if (!ctx->qbin) return fail(ILSM_ERR_OUT_OF_MEMORY, "host allocation failed");
-    if ((rc = ctx->qbin->init(ctx))) return rc;
+  if (!ctx->qbin) {  // installed only once it is complete: a failed init leaves the context without one
+    std::unique_ptr<Map> qb(new (std::nothrow) Map());
+    if (!qb) return fail(ILSM_ERR_OUT_OF_MEMORY, "host allocation failed");
+    if ((rc = qb->init(ctx))) return rc;
+    ctx->qbin = std::move(qb);
   }
-  Map* qb = ctx->qbin;
+  Map* qb = ctx->qbin.get();
   if ((rc = ctx->qwork.reserve((size_t)4 * qwork_items(nq) + 16))) return rc;  // QWork = 4 ints; the counter sits behind the list
   // the query cloud through the map build's count / alloc / scatter: queries grouped by voxel, original index in .w
   const int occ_slot = 4;  // occupied-voxel count of the build's own counter set

@@ -282,9 +282,8 @@ static inline int ilog2_ceil(uint32_t v) {
 
 int Map::init(Ctx* c) {
   ctx = c;
-  ILSM_CUDA(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
-  ILSM_CUDA(cudaEventCreateWithFlags(&ready, cudaEventDisableTiming));
-  ILSM_CUDA(cudaEventCreateWithFlags(&ctx_done, cudaEventDisableTiming));
+  int rc;
+  if ((rc = stream.create()) || (rc = ready.create()) || (rc = ctx_done.create())) return rc;
   return ILSM_OK;
 }
 

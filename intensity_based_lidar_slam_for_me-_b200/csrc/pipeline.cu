@@ -16,6 +16,7 @@
 #include <memory>
 #include <new>
 #include <string>
+#include <vector>
 
 #include "ilsm_cubemap.hpp"
 #include "ilsm_keyframe.hpp"
@@ -45,10 +46,35 @@ enum Phase {
 
 static int fail_text(int code, const char* text) { return fail(code, "%s", text); }
 
+// A sub-handle created through the C ABI and released through its destroy function.
+template <typename T>
+using Owner = std::unique_ptr<T, void (*)(T*)>;
+
+// Runs `create`, a C entry point that returns a new T through its last argument, and hands the result to `o`.
+template <typename T, typename... P, typename... A>
+static int create_into(Owner<T>& o, int (*create)(P...), A... args) {
+  T* p = nullptr;
+  const int rc = create(args..., &p);
+  o.reset(p);
+  return rc;
+}
+
+// Members are declared in dependency order, so that the destructor releases them in the right one: each context before
+// the handles that live on it, and the stage threads last, so that they are joined first.
 struct SlamH {
-  Ctx* ctx = nullptr;
-  ilsm_cubemap* cube = nullptr;   // mapping = laserMapping (rolling cube map)
-  ilsm_mapopt* mapopt = nullptr;  // mapping = mapOptimization (ground map), the node spot.launch starts
+  Ctx* ctx = nullptr;  // the caller's
+  // asynchronous mapping (ilsm_slam_create_async, ilsm_slam_create_staged): the cube map lives on a second, owned context;
+  // the mapping of frame k runs there while the front end and the odometry of frame k + 1 run on other contexts
+  Owner<ilsm_ctx> ctx2{nullptr, ilsm_destroy};
+  bool async = false;
+  // staged mode (ilsm_slam_create_staged): the three nodes as three stages, each with its own context (streams, scratch)
+  // and host thread like the reference's three processes -- scanRegistration on ctx0 + `frontend`, laserOdometry on the
+  // caller's context and thread, laserMapping on ctx2 + `mapping`.  Frame k's front end, frame k-1's odometry and frame
+  // k-2's / k-1's mapping are in flight together.
+  Owner<ilsm_ctx> ctx0{nullptr, ilsm_destroy};
+  bool staged = false;
+  Owner<ilsm_cubemap> cube{nullptr, ilsm_cubemap_destroy};  // mapping = laserMapping (rolling cube map)
+  Owner<ilsm_mapopt> mapopt{nullptr, ilsm_mapopt_destroy};  // mapping = mapOptimization (ground map), the node spot.launch starts
   Map last_corner, last_surf;  // kdtreeCornerLast / kdtreeSurfLast (laserOdometry.cpp:807-808)
   bool inited = false;        // systemInited (laserOdometry.cpp:384)
   double para_q[4] = {0, 0, 0, 1}, para_t[3] = {0, 0, 0};  // q_last_curr / t_last_curr, kept between frames (:51-52)
@@ -56,18 +82,19 @@ struct SlamH {
   double t_w_curr[3] = {0, 0, 0};
   float min_range = 0.3f;
   long long frames = 0;
+  long long pushed = 0;
   // The clouds between the nodes live in three rotating slots (frame % 3), so that the stage after the front end can
   // still read frame k while frame k + 1 or k + 2 is produced: a slot is rewritten by the front end of frame k + 3, after
   // the mapped pose of frame k has been handed out.
   struct FeSlot {
     DevBuf<float4> sharp, flat, lsharp, lflat;
     const float4* lf = nullptr;  // this frame's less-flat cloud: lflat, or the front end's own fe.lflat (synchronous loop)
-    cudaEvent_t ev = nullptr;    // recorded once the slot is written
+    Event ev;                    // recorded once the slot is written
     // loop closure in the pipelined and staged loops: the front end's cloud, kept until the frame's mapped pose is known
     DevBuf<float4> cloud;
     int n_cloud = 0;
-    cudaEvent_t ev_read = nullptr;  // recorded after a keyframe's copy read `cloud`
-    bool read_pending = false;      // the next front end into this slot waits for ev_read
+    Event ev_read;              // recorded after a keyframe's copy read `cloud`
+    bool read_pending = false;  // the next front end into this slot waits for ev_read
   } fslot[3];
   // the two mapping stacks (VoxelGrid of the less-sharp / less-flat clouds, laserMapping.cpp:608-616), double-buffered:
   // the odometry stage's side stream writes set k & 1 for frame k under its solve while the mapping of frame k - 1 (solve
@@ -75,13 +102,45 @@ struct SlamH {
   struct StackSet {
     DevBuf<float4> c, s;
     DevBuf<int> n;
-    cudaEvent_t ev_ready = nullptr, ev_free = nullptr;  // stacks written / last reader (deferred insertion) enqueued
+    Event ev_ready, ev_free;  // stacks written / last reader (deferred insertion) enqueued
     bool free_recorded = false;
   } stk[2];
-  // asynchronous mapping (ilsm_slam_create_async, ilsm_slam_create_staged): the cube map lives on a second, owned context;
-  // the mapping of frame k runs there while the front end and the odometry of frame k + 1 run on other contexts
-  ilsm_ctx* ctx2 = nullptr;
-  bool async = false;
+  // host-side phase clock (profiling aid, ilsm_slam_host_phases): seconds per phase, written by the caller's thread only
+  double phase_s[kNumPhases] = {};
+  // loop closure (ilsm_slam_enable_loop): an ilsm_loop on its own context (ctx3) and host thread, like the reference's
+  // loopClosureThread.  Each keyframe's cloud is copied on the device into one of the buffers; a buffer is used again only
+  // after the job that read it has been answered.
+  struct LoopJob {
+    int buf = 0, n = 0;
+    long long frame = -1;
+    double q[4] = {0, 0, 0, 1}, t[3] = {0, 0, 0};
+  };
+  struct LoopDone {
+    ilsm_slam_loop_event ev = {};
+    double seconds = 0;  // the stage's time on this keyframe
+  };
+  struct LoopBuf {
+    DevBuf<float4> cloud;
+    Event ev;  // recorded once the keyframe's cloud is copied in
+  };
+  struct LoopAnswer {
+    ilsm_slam_loop_event ev = {};
+    int rc = 0;  // a keyframe that failed: its status and error text, reported by ilsm_slam_loop_results in its turn
+    std::string err;
+  };
+  struct LoopStage {
+    Owner<ilsm_ctx> ctx3{nullptr, ilsm_destroy};
+    Owner<ilsm_loop> loop{nullptr, ilsm_loop_destroy};
+    ilsm_slam_loop_opts opts = {};
+    std::vector<LoopBuf> bufs;  // opts.max_pending of them
+    bool kf_have = false;       // (kf_q, kf_t): the mapped pose of the last keyframe
+    double kf_q[4] = {0, 0, 0, 1}, kf_t[3] = {0, 0, 0};
+    long long keyframes = 0;          // selected so far
+    std::deque<LoopAnswer> answered;  // taken from the loop stage, not yet handed out
+    double loop_s = 0;                // the loop stage's time over the answered keyframes
+    Stage<LoopJob, LoopDone> looper{ilsm_last_error, fail_text};
+  };
+  std::unique_ptr<LoopStage> loop;
   // The mapping stage has its own host thread, like the reference's laserMapping node has its own process: its ~25
   // launches per frame (3-4 us of host time each) are issued while the caller's thread launches the next front end.
   // At most two jobs queue: the staged loop posts frame k before it collects frame k - 1, so the mapping thread goes
@@ -102,12 +161,6 @@ struct SlamH {
     double phase_s[kNumPhases] = {};  // the stage's own phases, added to SlamH::phase_s when the result is taken
   };
   Stage<MapJob, MapResult> mapping{ilsm_last_error, fail_text};
-  // staged mode (ilsm_slam_create_staged): the three nodes as three stages, each with its own context (streams, scratch)
-  // and host thread like the reference's three processes -- scanRegistration on ctx0 + `frontend`, laserOdometry on the
-  // caller's context and thread, laserMapping on ctx2 + `mapping`.  Frame k's front end, frame k-1's odometry and frame
-  // k-2's / k-1's mapping are in flight together.
-  ilsm_ctx* ctx0 = nullptr;
-  bool staged = false;
   struct FeJob {
     const float* xyzi = nullptr;
     int n = 0, stride = 16, use_aloam = 1;
@@ -120,40 +173,6 @@ struct SlamH {
     double phase_s[kNumPhases] = {};
   };
   Stage<FeJob, FeResult> frontend{ilsm_last_error, fail_text};
-  long long pushed = 0;
-  // loop closure (ilsm_slam_enable_loop): an ilsm_loop on its own context (ctx3) and host thread, like the reference's
-  // loopClosureThread.  Each keyframe's cloud is copied on the device into one of max_pending buffers; a buffer is used
-  // again only after the job that read it has been answered.
-  struct LoopJob {
-    int buf = 0, n = 0;
-    long long frame = -1;
-    double q[4] = {0, 0, 0, 1}, t[3] = {0, 0, 0};
-  };
-  struct LoopDone {
-    ilsm_slam_loop_event ev = {};
-    double seconds = 0;  // the stage's time on this keyframe
-  };
-  struct LoopBuf {
-    DevBuf<float4> cloud;
-    cudaEvent_t ev = nullptr;  // recorded once the keyframe's cloud is copied in
-  };
-  ilsm_ctx* ctx3 = nullptr;
-  ilsm_loop* loop = nullptr;
-  ilsm_slam_loop_opts lopts = {};
-  std::unique_ptr<LoopBuf[]> lbuf;
-  bool kf_have = false;  // (kf_q, kf_t): the mapped pose of the last keyframe
-  double kf_q[4] = {0, 0, 0, 1}, kf_t[3] = {0, 0, 0};
-  long long keyframes = 0;                    // selected so far
-  struct LoopAnswer {
-    ilsm_slam_loop_event ev = {};
-    int rc = 0;       // a keyframe that failed: its status and error text, reported by ilsm_slam_loop_results in its turn
-    std::string err;
-  };
-  std::deque<LoopAnswer> answered;  // taken from the loop stage, not yet handed out
-  double loop_s = 0;                          // the loop stage's time over the answered keyframes
-  Stage<LoopJob, LoopDone> looper{ilsm_last_error, fail_text};
-  // host-side phase clock (profiling aid, ilsm_slam_host_phases): seconds per phase, written by the caller's thread only
-  double phase_s[kNumPhases] = {};
 };
 
 // a stage's oldest result, with the phase times it took added to the handle's
@@ -352,26 +371,27 @@ static void post_mapping_job(SlamH& s, const SlamH::FeSlot& o, const int cnt[8],
 
 // The loop stage's answer to its oldest keyframe, queued for ilsm_slam_loop_results.  A failed keyframe is queued too, with
 // its error: it is reported there, in keyframe order, and never by a frame call.
-static void take_loop_result(SlamH& s) {
+static void take_loop_result(SlamH::LoopStage& L) {
   SlamH::LoopDone d;
   SlamH::LoopAnswer a;
-  if ((a.rc = s.looper.take(d))) a.err = ilsm_last_error();
+  if ((a.rc = L.looper.take(d))) a.err = ilsm_last_error();
   a.ev = d.ev;
-  s.loop_s += d.seconds;
-  s.answered.push_back(std::move(a));
+  L.loop_s += d.seconds;
+  L.answered.push_back(std::move(a));
 }
 
 // hand keyframe `frame` to the loop stage (loop_offer)
-static int loop_post(SlamH& s, long long frame, SlamH::FeSlot* o, const float4* cloud, int n, const double q[4], const double t[3]) {
+static int loop_post(Ctx& c, SlamH::LoopStage& L, long long frame, SlamH::FeSlot* o, const float4* cloud, int n, const double q[4],
+                     const double t[3]) {
+  const int max_pending = (int)L.bufs.size();
   // every buffer in flight: wait for the oldest answer, which frees the buffer this keyframe takes
-  if (s.looper.in_flight() >= s.lopts.max_pending) take_loop_result(s);
+  if (L.looper.in_flight() >= max_pending) take_loop_result(L);
   int rc;
   SlamH::LoopJob j;
-  j.buf = (int)(s.keyframes % s.lopts.max_pending), j.n = n, j.frame = frame;
+  j.buf = (int)(L.keyframes % max_pending), j.n = n, j.frame = frame;
   for (int i = 0; i < 4; ++i) j.q[i] = q[i];
   for (int i = 0; i < 3; ++i) j.t[i] = t[i];
-  SlamH::LoopBuf& b = s.lbuf[j.buf];
-  Ctx& c = *s.ctx;
+  SlamH::LoopBuf& b = L.bufs[j.buf];
   if ((rc = b.cloud.reserve((size_t)n + 4))) return rc;
   if (o) ILSM_CUDA(cudaStreamWaitEvent(c.stream, o->ev, 0));
   if (n) ILSM_CUDA(cudaMemcpyAsync(b.cloud.p, cloud, (size_t)n * sizeof(float4), cudaMemcpyDeviceToDevice, c.stream));
@@ -380,8 +400,8 @@ static int loop_post(SlamH& s, long long frame, SlamH::FeSlot* o, const float4* 
     o->read_pending = true;
   }
   ILSM_CUDA(cudaEventRecord(b.ev, c.stream));
-  s.looper.post(j);
-  s.keyframes++;
+  L.looper.post(j);
+  L.keyframes++;
   return ILSM_OK;
 }
 
@@ -392,34 +412,35 @@ static int loop_post(SlamH& s, long long frame, SlamH::FeSlot* o, const float4* 
 // cannot be handed over is queued as a failed answer behind every keyframe before it.
 static void loop_offer(SlamH& s, long long frame, SlamH::FeSlot* o, const float4* cloud, int n, const double q[4], const double t[3]) {
   if (!s.loop) return;
-  if (s.kf_have && !keyframe_due(s.kf_q, s.kf_t, q, t, s.lopts.keyframe_dist, s.lopts.keyframe_angle_rad)) return;
-  s.kf_have = true;
-  for (int i = 0; i < 4; ++i) s.kf_q[i] = q[i];
-  for (int i = 0; i < 3; ++i) s.kf_t[i] = t[i];
+  SlamH::LoopStage& L = *s.loop;
+  if (L.kf_have && !keyframe_due(L.kf_q, L.kf_t, q, t, L.opts.keyframe_dist, L.opts.keyframe_angle_rad)) return;
+  L.kf_have = true;
+  for (int i = 0; i < 4; ++i) L.kf_q[i] = q[i];
+  for (int i = 0; i < 3; ++i) L.kf_t[i] = t[i];
   SlamH::LoopAnswer a;
-  if (!(a.rc = loop_post(s, frame, o, cloud, n, q, t))) return;
+  if (!(a.rc = loop_post(*s.ctx, L, frame, o, cloud, n, q, t))) return;
   a.err = ilsm_last_error();
   a.ev.frame = frame;
   for (int i = 0; i < 4; ++i) a.ev.q_xyzw[i] = q[i];
   for (int i = 0; i < 3; ++i) a.ev.t[i] = t[i];
-  while (s.looper.in_flight() > 0) take_loop_result(s);
-  s.answered.push_back(std::move(a));
+  while (L.looper.in_flight() > 0) take_loop_result(L);
+  L.answered.push_back(std::move(a));
 }
 
 // one keyframe on the loop stage: ilsm_loop_add_keyframe_dev on ctx3, after the copy into its buffer
-static int loop_job(SlamH& s, const SlamH::LoopJob& j, SlamH::LoopDone& r) {
+static int loop_job(SlamH::LoopStage& L, const SlamH::LoopJob& j, SlamH::LoopDone& r) {
   const auto t0 = std::chrono::steady_clock::now();
   r.ev.frame = j.frame;
   for (int i = 0; i < 4; ++i) r.ev.q_xyzw[i] = j.q[i];
   for (int i = 0; i < 3; ++i) r.ev.t[i] = j.t[i];
-  const SlamH::LoopBuf& b = s.lbuf[j.buf];
+  const SlamH::LoopBuf& b = L.bufs[j.buf];
   {
-    Ctx& l = s.ctx3->c;
+    Ctx& l = L.ctx3->c;
     std::lock_guard<std::mutex> lk(l.mu);
     const cudaError_t e = cudaStreamWaitEvent(l.stream, b.ev, 0);
     if (e != cudaSuccess) return fail_cuda(e, "cudaStreamWaitEvent(loop stage)");
   }
-  const int rc = ilsm_loop_add_keyframe_dev(s.loop, reinterpret_cast<const float*>(b.cloud.p), j.n, 16, j.q, j.t, &r.ev.result);
+  const int rc = ilsm_loop_add_keyframe_dev(L.loop.get(), reinterpret_cast<const float*>(b.cloud.p), j.n, 16, j.q, j.t, &r.ev.result);
   r.seconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
   return rc;
 }
@@ -460,136 +481,86 @@ struct ilsm_slam {
   SlamH s;
 };
 
-extern "C" {
-
-// the slots and stack sets (SlamH::fslot, SlamH::stk) at typical 16-ring sizes up front: a growing buffer costs a
-// device-wide synchronisation
-static int reserve_frame_buffers(SlamH& s) {
+// the mapping stage on its own context and host thread (pipelined and staged handles)
+static int slam_create_mapping_stage(SlamH& s, float line_res, float plane_res, int cube_capacity) {
   int rc;
-  for (SlamH::FeSlot& o : s.fslot) {
-    if (cudaEventCreateWithFlags(&o.ev, cudaEventDisableTiming) != cudaSuccess)
-      return fail(ILSM_ERR_CUDA, "slam_create: event creation failed");
-    if ((rc = o.sharp.reserve(1024)) || (rc = o.flat.reserve(4096)) || (rc = o.lsharp.reserve(8192)) || (rc = o.lflat.reserve(32768)))
-      return rc;
-  }
-  for (SlamH::StackSet& set : s.stk) {
-    if (cudaEventCreateWithFlags(&set.ev_ready, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreateWithFlags(&set.ev_free, cudaEventDisableTiming) != cudaSuccess)
-      return fail(ILSM_ERR_CUDA, "slam_create: event creation failed");
-    if ((rc = set.c.reserve(8192)) || (rc = set.s.reserve(32768)) || (rc = set.n.reserve(4))) return rc;
-  }
+  if ((rc = create_into(s.ctx2, ilsm_create, s.ctx->device)) ||
+      (rc = create_into(s.cube, ilsm_cubemap_create, s.ctx2.get(), line_res, plane_res, cube_capacity)))
+    return rc;
+  s.mapping.start([&s] { cudaSetDevice(s.ctx2->c.device); },
+                  [&s](const SlamH::MapJob& j, SlamH::MapResult& r) { return mapping_job(s, j, r); });
   return ILSM_OK;
 }
 
-// undo a failed ilsm_slam_enable_loop: the handle stays as it was
-static int loop_stage_abort(SlamH& s, int rc) {
-  if (s.loop) ilsm_loop_destroy(s.loop);
-  {
-    std::lock_guard<std::mutex> lk(s.ctx->mu);
-    cudaSetDevice(s.ctx->device);
-    for (SlamH::FeSlot& o : s.fslot) {
-      if (o.ev_read) cudaEventDestroy(o.ev_read);
-      o.ev_read = nullptr;
-    }
-    for (int i = 0; s.lbuf && i < s.lopts.max_pending; ++i)
-      if (s.lbuf[i].ev) cudaEventDestroy(s.lbuf[i].ev);
-    s.lbuf.reset();
-  }
-  if (s.ctx3) ilsm_destroy(s.ctx3);
-  s.loop = nullptr, s.ctx3 = nullptr;
-  return rc;
-}
-
-static int slam_create_common(ilsm_ctx* ctx, float min_range, ilsm_slam** out, ilsm_slam** h_out) {
+// The one creation path of the four ilsm_slam_create* entry points: the parts every handle has, then `mode(s)`, the
+// mode's own.  The handle is held here until it is complete, so that it releases itself on any failure.
+template <typename Mode>
+static int slam_create(ilsm_ctx* ctx, float min_range, ilsm_slam** out, Mode mode) {
   if (!ctx || !out) return fail(ILSM_ERR_INVALID_ARG, "slam_create: null argument");
-  ilsm_slam* h = new (std::nothrow) ilsm_slam();
+  std::unique_ptr<ilsm_slam> h(new (std::nothrow) ilsm_slam());
   if (!h) return fail(ILSM_ERR_OUT_OF_MEMORY, "host allocation failed");
-  h->s.ctx = &ctx->c;
-  h->s.min_range = min_range > 0.f ? min_range : 0.3f;
+  SlamH& s = h->s;
+  s.ctx = &ctx->c;
+  s.min_range = min_range > 0.f ? min_range : 0.3f;
   int rc;
   {
     CtxGuard g(ctx->c);
-    if (!(rc = g.rc) && !(rc = h->s.last_corner.init(&ctx->c))) rc = h->s.last_surf.init(&ctx->c);
-    if (!rc && !(rc = h->s.last_corner.reserve_points(16384))) rc = h->s.last_surf.reserve_points(65536);
-    if (!rc) rc = reserve_frame_buffers(h->s);
+    if ((rc = g.rc) || (rc = s.last_corner.init(&ctx->c)) || (rc = s.last_surf.init(&ctx->c)) ||
+        (rc = s.last_corner.reserve_points(16384)) || (rc = s.last_surf.reserve_points(65536)))
+      return rc;
+    // the slots and stack sets at typical 16-ring sizes up front: a growing buffer costs a device-wide synchronisation
+    for (SlamH::FeSlot& o : s.fslot)
+      if ((rc = o.ev.create()) || (rc = o.ev_read.create()) || (rc = o.sharp.reserve(1024)) || (rc = o.flat.reserve(4096)) ||
+          (rc = o.lsharp.reserve(8192)) || (rc = o.lflat.reserve(32768)))
+        return rc;
+    for (SlamH::StackSet& set : s.stk)
+      if ((rc = set.ev_ready.create()) || (rc = set.ev_free.create()) || (rc = set.c.reserve(8192)) || (rc = set.s.reserve(32768)) ||
+          (rc = set.n.reserve(4)))
+        return rc;
   }
-  if (rc) {
-    ilsm_slam_destroy(h);
-    return rc;
-  }
-  *h_out = h;
+  if ((rc = mode(s))) return rc;  // after the guard: the mode's creates, and a failed handle's release, take the lock
+  *out = h.release();
   return ILSM_OK;
 }
 
-// the mapping stage on its own context and host thread (pipelined and staged handles)
-static int slam_create_mapping_stage(ilsm_slam* h, float line_res, float plane_res, int cube_capacity) {
-  int rc;
-  if ((rc = ilsm_create(h->s.ctx->device, &h->s.ctx2)) ||
-      (rc = ilsm_cubemap_create(h->s.ctx2, line_res, plane_res, cube_capacity, &h->s.cube)))
-    return rc;
-  SlamH* s = &h->s;
-  s->mapping.start([s] { cudaSetDevice(s->ctx2->c.device); },
-                   [s](const SlamH::MapJob& j, SlamH::MapResult& r) { return mapping_job(*s, j, r); });
-  return ILSM_OK;
-}
+extern "C" {
 
 ILSM_API int ilsm_slam_create(ilsm_ctx* ctx, float line_res, float plane_res, float min_range, int cube_capacity,
                               ilsm_slam** out) {
-  ilsm_slam* h = nullptr;
-  int rc = slam_create_common(ctx, min_range, out, &h);
-  if (rc) return rc;
-  if ((rc = ilsm_cubemap_create(ctx, line_res, plane_res, cube_capacity, &h->s.cube))) {
-    ilsm_slam_destroy(h);
-    return rc;
-  }
-  *out = h;
-  return ILSM_OK;
+  return slam_create(ctx, min_range, out, [&](SlamH& s) {
+    return create_into(s.cube, ilsm_cubemap_create, ctx, line_res, plane_res, cube_capacity);
+  });
 }
 
 ILSM_API int ilsm_slam_create_mapopt(ilsm_ctx* ctx, float voxel_leaf, float downsample_size, float min_range, ilsm_slam** out) {
-  ilsm_slam* h = nullptr;
-  int rc = slam_create_common(ctx, min_range, out, &h);
-  if (rc) return rc;
-  if ((rc = ilsm_mapopt_create(ctx, voxel_leaf, downsample_size, &h->s.mapopt))) {
-    ilsm_slam_destroy(h);
-    return rc;
-  }
-  *out = h;
-  return ILSM_OK;
+  return slam_create(ctx, min_range, out, [&](SlamH& s) {
+    return create_into(s.mapopt, ilsm_mapopt_create, ctx, voxel_leaf, downsample_size);
+  });
 }
 
 ILSM_API int ilsm_slam_create_async(ilsm_ctx* ctx, float line_res, float plane_res, float min_range, int cube_capacity,
                                     ilsm_slam** out) {
-  ilsm_slam* h = nullptr;
-  int rc = slam_create_common(ctx, min_range, out, &h);
-  if (rc) return rc;
-  h->s.async = true;
-  if ((rc = slam_create_mapping_stage(h, line_res, plane_res, cube_capacity))) {
-    ilsm_slam_destroy(h);
-    return rc;
-  }
-  *out = h;
-  return ILSM_OK;
+  return slam_create(ctx, min_range, out, [&](SlamH& s) {
+    s.async = true;
+    return slam_create_mapping_stage(s, line_res, plane_res, cube_capacity);
+  });
 }
 
 ILSM_API int ilsm_slam_create_staged(ilsm_ctx* ctx, float line_res, float plane_res, float min_range, int cube_capacity,
                                      ilsm_slam** out) {
-  ilsm_slam* h = nullptr;
-  int rc = slam_create_common(ctx, min_range, out, &h);
-  if (rc) return rc;
-  h->s.staged = true;
-  h->s.last_corner.in_line = h->s.last_surf.in_line = true;  // nothing follows the tree builds on this stage's stream
-  if ((rc = ilsm_create(ctx->c.device, &h->s.ctx0)) || (rc = slam_create_mapping_stage(h, line_res, plane_res, cube_capacity))) {
-    ilsm_slam_destroy(h);
-    return rc;
-  }
-  SlamH* s = &h->s;
-  s->frontend.start([s] { cudaSetDevice(s->ctx0->c.device); },
-                    [s](const SlamH::FeJob& j, SlamH::FeResult& r) { return frontend_job(*s, j, r); });
-  *out = h;
-  return ILSM_OK;
+  return slam_create(ctx, min_range, out, [&](SlamH& s) -> int {
+    s.staged = true;
+    s.last_corner.in_line = s.last_surf.in_line = true;  // nothing follows the tree builds on this stage's stream
+    int rc;
+    if ((rc = create_into(s.ctx0, ilsm_create, ctx->c.device)) || (rc = slam_create_mapping_stage(s, line_res, plane_res, cube_capacity)))
+      return rc;
+    s.frontend.start([&s] { cudaSetDevice(s.ctx0->c.device); },
+                     [&s](const SlamH::FeJob& j, SlamH::FeResult& r) { return frontend_job(s, j, r); });
+    return ILSM_OK;
+  });
 }
 
+// Drains the stages in order, each before anything it reads goes away; then the handle releases what it owns.
 ILSM_API void ilsm_slam_destroy(ilsm_slam* slam) {
   if (!slam) return;
   SlamH& s = slam->s;
@@ -601,46 +572,29 @@ ILSM_API void ilsm_slam_destroy(ilsm_slam* slam) {
             us * s.phase_s[kMapTailWait], us * s.phase_s[kMapLaunch], us * s.phase_s[kMapWait], us * s.phase_s[kFeStageLaunch],
             us * s.phase_s[kFeStageWait], us * s.phase_s[kFeStageGather]);
   if (s.ctx0) {
-    std::lock_guard<std::mutex> lk0(s.ctx0->c.mu);
-    cudaSetDevice(s.ctx0->c.device);
+    CtxGuard g(s.ctx0->c);
     cudaStreamSynchronize(s.ctx0->c.stream);
   }
   s.mapping.stop();
   if (s.ctx2) {  // let the mapping stage drain before anything it reads goes away
-    std::lock_guard<std::mutex> lk2(s.ctx2->c.mu);
-    cudaSetDevice(s.ctx2->c.device);
+    CtxGuard g(s.ctx2->c);
     cudaStreamSynchronize(s.ctx2->c.stream);
     cudaStreamSynchronize(s.ctx2->c.aux);
   }
-  if (s.loop && getenv("ILSM_STAGE_TRACE")) {
-    const long long taken = s.keyframes - s.looper.in_flight();  // the answers the caller collected, with their stage times
-    fprintf(stderr, "[ilsm stage trace] loop: keyframes %lld  collected %lld  stage %.1f us per collected keyframe\n", s.keyframes,
-            taken, 1e6 * s.loop_s / (taken ? taken : 1));
+  if (s.loop) {
+    SlamH::LoopStage& L = *s.loop;
+    if (getenv("ILSM_STAGE_TRACE")) {
+      const long long taken = L.keyframes - L.looper.in_flight();  // the answers the caller collected, with their stage times
+      fprintf(stderr, "[ilsm stage trace] loop: keyframes %lld  collected %lld  stage %.1f us per collected keyframe\n", L.keyframes,
+              taken, 1e6 * L.loop_s / (taken ? taken : 1));
+    }
+    L.looper.stop();  // every posted keyframe is answered; the loop handle's destroy synchronises its stream
   }
-  s.looper.stop();  // every posted keyframe is answered; the loop handle's destroy synchronises its stream
-  if (s.loop) ilsm_loop_destroy(s.loop);
   {
-    std::lock_guard<std::mutex> lk(s.ctx->mu);
-    cudaSetDevice(s.ctx->device);
+    CtxGuard g(*s.ctx);
     cudaStreamSynchronize(s.ctx->stream);
-    for (SlamH::FeSlot& o : s.fslot) {
-      if (o.ev) cudaEventDestroy(o.ev);
-      if (o.ev_read) cudaEventDestroy(o.ev_read);
-    }
-    for (int i = 0; s.lbuf && i < s.lopts.max_pending; ++i)
-      if (s.lbuf[i].ev) cudaEventDestroy(s.lbuf[i].ev);
-    for (SlamH::StackSet& set : s.stk) {
-      if (set.ev_ready) cudaEventDestroy(set.ev_ready);
-      if (set.ev_free) cudaEventDestroy(set.ev_free);
-    }
   }
-  if (s.cube) ilsm_cubemap_destroy(s.cube);
-  if (s.mapopt) ilsm_mapopt_destroy(s.mapopt);
-  if (s.ctx2) ilsm_destroy(s.ctx2);
-  if (s.ctx0) ilsm_destroy(s.ctx0);
-  if (s.ctx3) ilsm_destroy(s.ctx3);
-  cudaSetDevice(s.ctx->device);
-  delete slam;  // frees the slots, stack sets and last-frame maps: no stage reads them any more
+  delete slam;  // outside the context's lock (ilsm_mapopt_destroy takes it), with the handle's device current
 }
 
 ILSM_API void ilsm_slam_loop_opts_default(ilsm_slam_loop_opts* o) {
@@ -672,28 +626,29 @@ ILSM_API int ilsm_slam_enable_loop(ilsm_slam* slam, const ilsm_slam_loop_opts* o
   SlamH& s = slam->s;
   if (s.loop) return fail(ILSM_ERR_STATE, "slam_enable_loop: loop closure is already on");
   if (s.frames > 0 || s.pushed > 0) return fail(ILSM_ERR_STATE, "slam_enable_loop: call it before the first frame");
-  if ((rc = ilsm_create(s.ctx->device, &s.ctx3)) || (rc = ilsm_loop_create(s.ctx3, &o.loop, &s.loop))) return loop_stage_abort(s, rc);
-  s.lopts = o;
+  // built complete before it is installed: on a failure it releases itself and the handle stays as it was
+  std::unique_ptr<SlamH::LoopStage> L(new (std::nothrow) SlamH::LoopStage());
+  if (!L) return fail(ILSM_ERR_OUT_OF_MEMORY, "host allocation failed");
+  L->opts = o;
+  if ((rc = create_into(L->ctx3, ilsm_create, s.ctx->device)) || (rc = create_into(L->loop, ilsm_loop_create, L->ctx3.get(), &o.loop)))
+    return rc;
   {
     CtxGuard g(*s.ctx);
-    if ((rc = g.rc)) return loop_stage_abort(s, rc);
-    s.lbuf.reset(new (std::nothrow) SlamH::LoopBuf[o.max_pending]);
-    if (!s.lbuf) return loop_stage_abort(s, fail(ILSM_ERR_OUT_OF_MEMORY, "host allocation failed"));
-    // the frame's size up front: a growing buffer costs a device-wide synchronisation (reserve_frame_buffers)
-    for (int i = 0; i < o.max_pending; ++i) {
-      if (cudaEventCreateWithFlags(&s.lbuf[i].ev, cudaEventDisableTiming) != cudaSuccess)
-        return loop_stage_abort(s, fail(ILSM_ERR_CUDA, "slam_enable_loop: event creation failed"));
-      if ((rc = s.lbuf[i].cloud.reserve(kFramePoints + 4))) return loop_stage_abort(s, rc);
+    if ((rc = g.rc)) return rc;
+    try {
+      L->bufs.resize(o.max_pending);
+    } catch (const std::bad_alloc&) {
+      return fail(ILSM_ERR_OUT_OF_MEMORY, "host allocation failed");
     }
-    for (SlamH::FeSlot& sl : s.fslot) {
-      if (cudaEventCreateWithFlags(&sl.ev_read, cudaEventDisableTiming) != cudaSuccess)
-        return loop_stage_abort(s, fail(ILSM_ERR_CUDA, "slam_enable_loop: event creation failed"));
-      if (s.ctx2 && (rc = sl.cloud.reserve(kFramePoints + 4))) return loop_stage_abort(s, rc);
-    }
+    // the frame's size up front: a growing buffer costs a device-wide synchronisation (slam_create)
+    for (SlamH::LoopBuf& b : L->bufs)
+      if ((rc = b.ev.create()) || (rc = b.cloud.reserve(kFramePoints + 4))) return rc;
+    for (SlamH::FeSlot& sl : s.fslot)
+      if (s.ctx2 && (rc = sl.cloud.reserve(kFramePoints + 4))) return rc;
   }
-  SlamH* sp = &s;
-  s.looper.start([sp] { cudaSetDevice(sp->ctx3->c.device); },
-                 [sp](const SlamH::LoopJob& j, SlamH::LoopDone& r) { return loop_job(*sp, j, r); });
+  L->looper.start([lp = L.get()] { cudaSetDevice(lp->ctx3->c.device); },
+                  [lp = L.get()](const SlamH::LoopJob& j, SlamH::LoopDone& r) { return loop_job(*lp, j, r); });
+  s.loop = std::move(L);
   return ILSM_OK;
 }
 
@@ -701,27 +656,27 @@ ILSM_API int ilsm_slam_loop_results(ilsm_slam* slam, int wait, ilsm_slam_loop_ev
   if (!slam || !n_out || (capacity > 0 && !out)) return fail(ILSM_ERR_INVALID_ARG, "slam_loop_results: null argument");
   if (capacity < 0) return fail(ILSM_ERR_INVALID_ARG, "slam_loop_results: capacity < 0");
   *n_out = 0;
-  SlamH& s = slam->s;
-  if (!s.loop) return fail(ILSM_ERR_STATE, "slam_loop_results: loop closure is not on (ilsm_slam_enable_loop)");
+  if (!slam->s.loop) return fail(ILSM_ERR_STATE, "slam_loop_results: loop closure is not on (ilsm_slam_enable_loop)");
+  SlamH::LoopStage& L = *slam->s.loop;
   // no context lock: the queue and the stage's in-flight count belong to the thread that hands in the frames, and a drain
   // must not hold up other users of the caller's context
-  while (s.looper.in_flight() > 0 && (wait || s.looper.ready())) take_loop_result(s);
+  while (L.looper.in_flight() > 0 && (wait || L.looper.ready())) take_loop_result(L);
   int k = 0;
-  for (; k < capacity && !s.answered.empty() && !s.answered.front().rc; ++k) {
-    out[k] = s.answered.front().ev;
-    s.answered.pop_front();
+  for (; k < capacity && !L.answered.empty() && !L.answered.front().rc; ++k) {
+    out[k] = L.answered.front().ev;
+    L.answered.pop_front();
   }
   *n_out = k;
-  if (k == 0 && capacity > 0 && !s.answered.empty()) {  // a failed keyframe is next in order: report it
-    const SlamH::LoopAnswer a = std::move(s.answered.front());
-    s.answered.pop_front();
+  if (k == 0 && capacity > 0 && !L.answered.empty()) {  // a failed keyframe is next in order: report it
+    const SlamH::LoopAnswer a = std::move(L.answered.front());
+    L.answered.pop_front();
     return fail(a.rc, "slam_loop_results: keyframe of frame %lld: %s", (long long)a.ev.frame, a.err.c_str());
   }
   return ILSM_OK;
 }
 
-ILSM_API ilsm_cubemap* ilsm_slam_cubemap(ilsm_slam* slam) { return slam ? slam->s.cube : nullptr; }
-ILSM_API ilsm_mapopt* ilsm_slam_mapopt(ilsm_slam* slam) { return slam ? slam->s.mapopt : nullptr; }
+ILSM_API ilsm_cubemap* ilsm_slam_cubemap(ilsm_slam* slam) { return slam ? slam->s.cube.get() : nullptr; }
+ILSM_API ilsm_mapopt* ilsm_slam_mapopt(ilsm_slam* slam) { return slam ? slam->s.mapopt.get() : nullptr; }
 
 }  // extern "C"
 namespace ilsm {
@@ -824,7 +779,7 @@ static int slam_frame_impl(ilsm_slam* slam, const float* xyzi, int n, int stride
     if (!rc) rc = cubemap_frame_collect(*cmp, q_map, t_map, stats ? &stats->mapping : nullptr, stats ? &stats->cubemap : nullptr);
   } else {    // mapOptimization: ground extraction from the frame already on the device + the less-flat cloud
     ilsm_mapopt_stats ms;
-    rc = mapopt_frame_core(s.mapopt, c.fe.raw.p, n, pc2 ? 16 : stride_bytes, reinterpret_cast<const float*>(o.lf), cnt[4], 16,
+    rc = mapopt_frame_core(s.mapopt.get(), c.fe.raw.p, n, pc2 ? 16 : stride_bytes, reinterpret_cast<const float*>(o.lf), cnt[4], 16,
                            false, q_odom, t_odom, q_map, t_map, nullptr, &ms);
     if (!rc && stats) {
       stats->mapping.passes = ms.ran_optimization;
